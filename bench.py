@@ -8,6 +8,7 @@ resident in HBM; `e2e` = the same metric through the reference-facing call
 ``multigrid_v_cycle(H, x0, b)`` (amg1d_vcycle) with pinned HOST vectors, copies inside the timing.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload T|C2|C3|C4|C5|P8|S] [--impl reference]
+                  [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -20,6 +21,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # no __pycache__ in the tree: the benchmark may run from a read-only checkout
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -129,6 +131,23 @@ def measured_peak():
     if os.path.exists(p):
         return float(json.load(open(p))["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_MAX_ENTRIES = 2 ** 21      # 16 MB of x values + 16 MB of their indices
+
+
+def dump_outputs(out_dir, dev, res_norm):
+    """What the last timed step left for its caller, as DIR/<name>.npy (float64): x, the iterate after the last
+    V-cycle (this rank's slab; longer than DUMP_MAX_ENTRIES, a fixed seeded sample of it, positions in x_index),
+    and residual_norm, the ||b - A x|| of that cycle's convergence check."""
+    x = dev.dev_get_solution()
+    idx = np.arange(len(x))
+    if len(x) > DUMP_MAX_ENTRIES:
+        idx = np.sort(np.random.default_rng(0).choice(len(x), DUMP_MAX_ENTRIES, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "x.npy"), x[idx])
+    np.save(os.path.join(out_dir, "x_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "residual_norm.npy"), np.array([res_norm]))
 
 
 # ---- CPU reference arm: the oracle's restatement of multigrid_v_cycle on the host cores ------------
@@ -342,10 +361,11 @@ class Ctx:
         return float(t.item())
 
 
-def measure(ctx, args, workload, ranks, full):
+def measure(ctx, args, workload, ranks, full, dump=None):
     """One workload on `ranks` GPUs (ranks == ctx.world: slab-sharded over every rank; ranks == 1: a single-GPU
     handle - the caller runs it on rank 0 only).  full = True: the whole JSON line (roofline, e2e, ldiv, PCG,
-    pattern modes, CPU baseline); False: throughput + time-to-1e-10 only (the secondary objects)."""
+    pattern modes, CPU baseline); False: throughput + time-to-1e-10 only (the secondary objects).  dump: a
+    directory for rank 0 to write the outputs of the last timed step to (dump_outputs)."""
     import ctypes as C
     torch, capi, lib = ctx.torch, ctx.capi, ctx.lib
     world = ranks
@@ -394,6 +414,8 @@ def measure(ctx, args, workload, ranks, full):
     launches = dev.info("kernel_launches") - launches0
     value = upd / (ms_step * 1e-3)
     res_after = dev.dev_residual_norm()
+    if dump and rank == 0:
+        dump_outputs(dump, dev, res_after)
 
     # ---- host vectors (pinned) with the workload's right-hand side -----------------------------------
     bufs = []
@@ -737,7 +759,7 @@ def run_gpu(args):
     ctx = Ctx()
     world = ctx.world
     workload = args.workload or default_workload(world)
-    line = measure(ctx, args, workload, world, full=not args.light)
+    line = measure(ctx, args, workload, world, full=not args.light, dump=args.dump_outputs)
     if not args.workload and not args.no_extra and not args.light:
         # The default run also carries BASELINE's other multi-GPU configuration and the bases its scaling is
         # judged against, measured in this very process group (rank 0 alone for the single-GPU bases).
@@ -793,7 +815,13 @@ def main():
                     help="amg1d_set_option before the first level is set (e.g. --pre-opt shard_min=65536)")
     ap.add_argument("--opt", action="append", default=[], metavar="KEY=VALUE",
                     help="amg1d_set_option after the upload (A/B experiments, e.g. --opt pdl=0)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (GPU arm; inputs are seeded)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":

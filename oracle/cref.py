@@ -3,6 +3,7 @@ src/solvers.jl:19-50.  Feeds it an oracle ``MeshHierarchy`` (scipy operators, LU
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 import scipy.sparse as sp
@@ -15,9 +16,17 @@ _pd, _pi = C.POINTER(C.c_double), C.POINTER(C.c_int64)
 
 
 def load():
-    if not os.path.exists(_LIB) or os.path.getmtime(_LIB) < os.path.getmtime(os.path.join(_HERE, "vcycle_ref.c")):
+    if os.path.exists(_LIB) and os.path.getmtime(_LIB) >= os.path.getmtime(os.path.join(_HERE, "vcycle_ref.c")):
+        lib = C.CDLL(_LIB)
+    elif os.access(_HERE, os.W_OK):
         subprocess.check_call(["make", "-s", "-C", _HERE])
-    lib = C.CDLL(_LIB)
+        lib = C.CDLL(_LIB)
+    else:
+        # read-only tree: the same Makefile target, built in a temporary directory (the loaded library
+        # stays mapped after the directory is removed)
+        with tempfile.TemporaryDirectory(prefix="vcycle_ref_") as tmp:
+            subprocess.check_call(["make", "-s", "-C", tmp, "-f", os.path.join(_HERE, "Makefile"), f"VPATH={_HERE}"])
+            lib = C.CDLL(os.path.join(tmp, "libvcycle_ref.so"))
     lib.ref_create.restype = C.c_void_p
     lib.ref_create.argtypes = [C.c_int]
     lib.ref_set_level.argtypes = [C.c_void_p, C.c_int, C.c_int64, _pi, _pi, _pd, C.c_int, C.c_int64, _pi, _pd, _pd]
