@@ -13,6 +13,7 @@ LIB_PATH = os.environ.get("AMG1D_LIB") or os.path.join(_HERE, "libamg1d.so")   #
 
 OK, ERR_ARG, ERR_CUDA, ERR_NCCL, ERR_NOMEM, ERR_STATE, ERR_UNSUPPORTED = range(7)
 VEC_X, VEC_B, VEC_R = 0, 1, 2
+MAX_COLS = 8                     # AMG1D_MAX_COLS: right-hand sides of one multi-column set
 
 _pd = C.POINTER(C.c_double)
 _pi64 = C.POINTER(C.c_int64)
@@ -69,6 +70,13 @@ PROTOTYPES = {
     "amg1d_dev_residual_norm": (C.c_int, [_h, _pd]),
     "amg1d_dev_rhs_norm": (C.c_int, [_h, _pd]),
     "amg1d_dev_get_solution": (C.c_int, [_h, _pd]),
+    "amg1d_dev_set_problems": (C.c_int, [_h, C.c_int, _pd, _pd]),
+    "amg1d_dev_fill_rhs_random_multi": (C.c_int, [_h, C.c_int, C.c_uint64]),
+    "amg1d_dev_vcycle_multi": (C.c_int, [_h, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int]),
+    "amg1d_dev_residual_norms": (C.c_int, [_h, _pd]),
+    "amg1d_dev_solve_multi": (C.c_int, [_h, C.c_int, C.c_double, C.c_int, C.c_int, C.c_double, C.POINTER(C.c_int),
+                                        _pd]),
+    "amg1d_dev_get_solutions": (C.c_int, [_h, _pd]),
     "amg1d_synchronize": (C.c_int, [_h]),
     "amg1d_stream": (C.c_void_p, [_h]),
     "amg1d_dev_ptr": (C.c_void_p, [_h, C.c_int, C.c_int]),

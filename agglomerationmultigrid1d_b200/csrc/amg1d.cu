@@ -21,6 +21,7 @@
 #include "../../include/amg1d.h"
 #include "kernels_generic.cuh"
 #include "kernels_fused.cuh"
+#include "kernels_multi.cuh"
 #include "kernels_rows.cuh"
 #include "direct_bcr.cuh"
 #include "device_setup.cuh"
@@ -29,6 +30,8 @@
 #define AMG1D_VERSION 100
 #define PAD_FRONT 64  // doubles in front of element 0 (ghost elements live at the end of them)
 #define PAD_BACK 64
+#define MULTI_SLOTS 4  // device scalars per column of the multi-column set (slot 0: ||b - A x||, 2: ||b||)
+static_assert(MULTI_MAX_COLS == AMG1D_MAX_COLS, "kernels_multi.cuh and amg1d.h disagree on the column limit");
 
 namespace {
 
@@ -161,6 +164,8 @@ struct amg1d {
     int tail_start = -1;
     TailLevel* d_tail = nullptr;
     TailPlan tail_plan_ = {};
+    std::vector<TailLevel> tail_host;   // host copy of d_tail (the multi-column cycle patches in its columns' vectors)
+    uint64_t tail_gen = 0;              // bumped by every build_tail
     // graph cache: a few instantiated V-cycle graphs keyed by (nPre, nPost, alpha, norm, zero guess)
     struct GraphEntry {
         cudaGraphExec_t exec = nullptr;
@@ -217,6 +222,22 @@ struct amg1d {
         struct Nb { int64_t off[3] = {0, 0, 0}; int64_t n = 0; };   // byte offsets of x[0].p, x[1].p, b.p; owned n
         std::vector<Nb> nb[2];                       // per level, for the left / right neighbour
     } p2p;
+    // multi-column resident problems (amg1d_dev_set_problems ...): per column the three vectors of every level, kept
+    // apart from the single-column resident problem in L[l].x / L[l].b
+    struct Multi {
+        struct ColLevel { DVec x[2], b; int cur = 0; };
+        std::vector<std::vector<ColLevel>> col;    // [column][level], grown on demand, never shrunk
+        std::vector<double*> partial;              // per column: ||b - A x||^2 partial sums (partial_cap + 256)
+        int k = 0;                                 // columns of the current set (0: none)
+        double* d_scal = nullptr;                  // MULTI_MAX_COLS x MULTI_SLOTS device scalars (slots as d_scal)
+        double* h_scal = nullptr;                  // pinned host copy
+        TailLevel* d_tail = nullptr;               // MULTI_MAX_COLS x TAIL_MAXL descriptors of the single-CTA tail
+        uint64_t tail_synced = ~0ull;              // tail_gen that d_tail was filled for
+        bool norm_valid = false;                   // d_scal slot 0 of every column holds ||b - A x|| of its iterate
+        int64_t launches_per_cycle = 0;
+        struct Graph { GraphEntry g; unsigned mask = 0; };   // keyed as graphs[] plus the active-column set
+        Graph graphs[4];
+    } multi;
 };
 
 namespace {
@@ -1156,7 +1177,12 @@ void invalidate_graph(amg1d* h) {
         if (g.exec) cudaGraphExecDestroy(g.exec);
         g = amg1d::GraphEntry();
     }
+    for (auto& g : h->multi.graphs) {
+        if (g.g.exec) cudaGraphExecDestroy(g.g.exec);
+        g = amg1d::Multi::Graph();
+    }
     h->norm_valid = false;
+    h->multi.norm_valid = false;
 }
 
 int p2p_check(amg1d* h) {                     // after a stream synchronisation: did a peer-memory wait time out?
@@ -1303,6 +1329,8 @@ int factor_coarsest(amg1d* h) {
 // coarsest level alone stays with g_coarse_solve.
 int build_tail(amg1d* h) {
     h->tail_start = -1;
+    h->tail_host.clear();
+    h->tail_gen++;
     if (h->d_tail) { cudaFree(h->d_tail); h->d_tail = nullptr; }
     const int nl = h->n_levels;
     if (nl < 3 || h->opt_coarse_cta < 1 || !h->L[nl - 1].present || h->coarse_bcr.ready()) return AMG1D_OK;
@@ -1353,6 +1381,7 @@ int build_tail(amg1d* h) {
     if (e != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "f_tail configuration failed: %s", cudaGetErrorString(e));
     RET(dev_alloc(h, (void**)&h->d_tail, (int64_t)(tl.size() * sizeof(TailLevel))));
     CK(cudaMemcpy(h->d_tail, tl.data(), tl.size() * sizeof(TailLevel), cudaMemcpyHostToDevice));
+    h->tail_host = tl;
     h->tail_start = ts;
     return AMG1D_OK;
 }
@@ -1369,6 +1398,303 @@ int check_dev_problem(amg1d* h) {
     if (!h->dev_problem)
         return fail(h, AMG1D_ERR_STATE, "the device-resident problem was overwritten by a per-level host operation "
                     "(amg1d_residual / amg1d_smoother_solve on level 0, amg1d_pcg); call amg1d_dev_set_problem again");
+    return AMG1D_OK;
+}
+
+// ---- multi-column resident problems (amg1d_dev_set_problems ...) ----------------------------------------------------
+// Column c of the set has its own x[0], x[1], b (and buffer parity) on every level.  Levels whose legs have a fused
+// multi-column kernel (kernels_multi.cuh) run one launch for all active columns; every other operation of the cycle -
+// the row-per-thread and generic tiers, the single-CTA tail, the coarse solve - runs its single-column code once per
+// column with that column's vectors swapped into the level (ColumnBind), so per column it is exactly the single-column
+// cycle.
+
+// Swaps column c's vectors, buffer parities, scalar slots and reduction scratch with the handle's own for as long as it
+// lives (the swap is its own inverse).
+struct ColumnBind {
+    amg1d* h;
+    int c;
+    double* scal;
+    double* part;
+    ColumnBind(amg1d* h_, int c_)
+        : h(h_), c(c_), scal(h_->multi.d_scal + c_ * MULTI_SLOTS), part(h_->multi.partial[(size_t)c_]) { swap(); }
+    ~ColumnBind() { swap(); }
+    void swap() {
+        auto& cl = h->multi.col[(size_t)c];
+        for (int l = 0; l < h->n_levels; ++l) {
+            Level& lv = h->L[l];
+            std::swap(lv.x[0], cl[(size_t)l].x[0]);
+            std::swap(lv.x[1], cl[(size_t)l].x[1]);
+            std::swap(lv.b, cl[(size_t)l].b);
+            std::swap(lv.cur, cl[(size_t)l].cur);
+        }
+        std::swap(h->d_scal, scal);
+        std::swap(h->partial, part);
+    }
+};
+
+int64_t vec_bytes(const DVec& v) { return (PAD_FRONT + v.len + PAD_BACK) * 8; }
+
+void multi_free_column(amg1d* h, std::vector<amg1d::Multi::ColLevel>& cl, double* partial) {
+    for (auto& v : cl)
+        for (DVec* d : {&v.x[0], &v.x[1], &v.b})
+            if (d->raw) { h->device_bytes -= vec_bytes(*d); vec_free(*d); }
+    if (partial) { cudaFree(partial); h->device_bytes -= (h->partial_cap + 256) * 8; }
+}
+
+// storage for k columns: the set only grows; a failed allocation releases what it took and leaves the rest as it was
+int multi_alloc(amg1d* h, int k) {
+    amg1d::Multi& M = h->multi;
+    if (!M.d_scal) RET(dev_alloc(h, (void**)&M.d_scal, MULTI_MAX_COLS * MULTI_SLOTS * 8));
+    if (!M.h_scal) CK(cudaMallocHost(&M.h_scal, MULTI_MAX_COLS * MULTI_SLOTS * 8));
+    if (!M.d_tail) RET(dev_alloc(h, (void**)&M.d_tail, (int64_t)(MULTI_MAX_COLS * TAIL_MAXL * sizeof(TailLevel))));
+    while ((int)M.col.size() < k) {
+        std::vector<amg1d::Multi::ColLevel> cl((size_t)h->n_levels);
+        double* part = nullptr;
+        int rc = AMG1D_OK;
+        for (int l = 0; l < h->n_levels && rc == AMG1D_OK; ++l) {
+            const Level& lv = h->L[l];
+            rc = vec_alloc(h, cl[(size_t)l].x[0], lv.n, lv.m);
+            if (rc == AMG1D_OK) rc = vec_alloc(h, cl[(size_t)l].x[1], lv.n, lv.m);
+            if (rc == AMG1D_OK) rc = vec_alloc(h, cl[(size_t)l].b, lv.n, lv.m);
+        }
+        if (rc == AMG1D_OK) rc = dev_alloc(h, (void**)&part, (h->partial_cap + 256) * 8);
+        if (rc != AMG1D_OK) {
+            multi_free_column(h, cl, part);
+            cudaGetLastError();                  // an out-of-memory status must not surface at the next launch check
+            return fail(h, rc, "column %d of the multi-column set: %s", (int)M.col.size(), h->err.c_str());
+        }
+        M.col.push_back(std::move(cl));
+        M.partial.push_back(part);
+        M.tail_synced = ~0ull;
+    }
+    return AMG1D_OK;
+}
+
+// descriptors of the single-CTA tail for every column: the handle's own with the columns' vectors (before capture)
+int multi_sync_tail(amg1d* h) {
+    amg1d::Multi& M = h->multi;
+    if (h->tail_start <= 0 || M.tail_synced == h->tail_gen) return AMG1D_OK;
+    const int ts = h->tail_start;
+    std::vector<TailLevel> all((size_t)MULTI_MAX_COLS * TAIL_MAXL);
+    for (size_t c = 0; c < M.col.size(); ++c)
+        for (size_t i = 0; i < h->tail_host.size(); ++i) {
+            TailLevel d = h->tail_host[i];
+            d.x = M.col[c][(size_t)ts + i].x[0].p;
+            d.b = M.col[c][(size_t)ts + i].b.p;
+            all[c * TAIL_MAXL + i] = d;
+        }
+    CK(cudaMemcpyAsync(M.d_tail, all.data(), all.size() * sizeof(TailLevel), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    M.tail_synced = h->tail_gen;
+    return AMG1D_OK;
+}
+
+// the fused multi-column kernels serve level l (the test of leg_down / leg_up plus a kernel for the combination)
+bool multi_leg_level(const amg1d* h, int l) {
+    const Level& lv = h->L[l];
+    const Transfer& t = h->T[l];
+    return h->opt_fused && t.fusable && !lv.smooth_tri && fused_multi_available(lv.md, t.mc);
+}
+
+int prof_unmark(amg1d* h, int level, int leg) {      // drop the opening bracket of a leg that did not launch
+    if (!h->opt_profile) return AMG1D_OK;
+    auto& ev = h->prof[level * 2 + leg].ev;
+    cudaEventDestroy(ev.back());
+    ev.pop_back();
+    return AMG1D_OK;
+}
+
+int leg_down_multi(amg1d* h, int l, const int* act, int na, int nPre, double alpha, bool zero0) {
+    Level& lv = h->L[l];
+    Transfer& t = h->T[l];
+    amg1d::Multi& M = h->multi;
+    const bool zero = l > 0 || zero0;
+    if (multi_leg_level(h, l)) {
+        MultiCols mc = {};
+        int ob[MULTI_MAX_COLS];
+        for (int i = 0; i < na; ++i) {
+            auto& cl = M.col[(size_t)act[i]];
+            auto& v = cl[(size_t)l];
+            if (zero) v.cur = 0;
+            ob[i] = zero ? 0 : 1 - v.cur;
+            mc.b[i] = v.b.p;
+            mc.xin[i] = v.x[v.cur].p;
+            mc.xout[i] = v.x[ob[i]].p;
+            mc.xc[i] = cl[(size_t)l + 1].b.p;
+        }
+        RET(prof_mark(h, l, 0));
+        cudaError_t le = cudaSuccess;
+        const int fr = fused_down_multi(lv.md, t.mc, make_map_closed(t), nPre, zero, lv.mat, make_pat(h, l), mc, na,
+                                        tp0(t), tp1(t), lv.n, alpha, make_slab(h, l), h->stream, h->opt_pdl != 0, &le,
+                                        leg_rec(h, lv, t.mc));
+        if (fr == FUSED_ERR) return fail(h, AMG1D_ERR_CUDA, "f_down_multi launch failed on level %d: %s", l, cudaGetErrorString(le));
+        if (fr == FUSED_OK) {
+            for (int i = 0; i < na; ++i) M.col[(size_t)act[i]][(size_t)l].cur = ob[i];
+            h->launch_counter++;
+            LAUNCH_CHECK();
+            return prof_mark(h, l, 0);
+        }
+        RET(prof_unmark(h, l, 0));
+    }
+    for (int i = 0; i < na; ++i) {
+        ColumnBind cb(h, act[i]);
+        RET(leg_down(h, l, nPre, alpha, zero0));
+    }
+    return AMG1D_OK;
+}
+
+// norm: level 0 of a cycle that leaves ||b - A x|| in slot 0 of every column (done[i]: already there)
+int leg_up_multi(amg1d* h, int l, const int* act, int na, int nPost, double alpha, bool norm, bool* done) {
+    Level& lv = h->L[l];
+    Transfer& t = h->T[l];
+    amg1d::Multi& M = h->multi;
+    if (multi_leg_level(h, l)) {
+        MultiCols mc = {};
+        for (int i = 0; i < na; ++i) {
+            auto& cl = M.col[(size_t)act[i]];
+            auto& v = cl[(size_t)l];
+            auto& vc = cl[(size_t)l + 1];
+            mc.b[i] = v.b.p;
+            mc.xin[i] = v.x[v.cur].p;
+            mc.xout[i] = v.x[1 - v.cur].p;
+            mc.xc[i] = vc.x[vc.cur].p;
+            mc.partial[i] = norm ? M.partial[(size_t)act[i]] : nullptr;
+        }
+        RET(prof_mark(h, l, 1));
+        cudaError_t le = cudaSuccess;
+        int nb = 0;
+        const int fr = fused_up_multi(lv.md, t.mc, make_map_closed(t), nPost, lv.mat, make_pat(h, l), mc, na, tp0(t),
+                                      tp1(t), lv.n, alpha, norm, h->partial_cap, &nb, make_slab(h, l), h->stream,
+                                      h->opt_pdl != 0, &le, leg_rec(h, lv, t.mc));
+        if (fr == FUSED_ERR) return fail(h, AMG1D_ERR_CUDA, "f_up_multi launch failed on level %d: %s", l, cudaGetErrorString(le));
+        if (fr == FUSED_OK) {
+            for (int i = 0; i < na; ++i) { auto& v = M.col[(size_t)act[i]][(size_t)l]; v.cur = 1 - v.cur; }
+            h->launch_counter++;
+            LAUNCH_CHECK();
+            RET(prof_mark(h, l, 1));
+            if (norm)
+                for (int i = 0; i < na; ++i) {
+                    ColumnBind cb(h, act[i]);
+                    RET(op_reduce_partials(h, nb, 0));
+                    done[i] = true;
+                }
+            return AMG1D_OK;
+        }
+        RET(prof_unmark(h, l, 1));
+    }
+    for (int i = 0; i < na; ++i) {
+        ColumnBind cb(h, act[i]);
+        bool pushed = false;
+        RET(leg_up(h, l, nPost, alpha, norm, &done[i], &pushed));
+    }
+    return AMG1D_OK;
+}
+
+// enqueue_vcycle for the active columns act[0..na) of the multi-column set (single GPU)
+int enqueue_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, double alpha, bool want_norm,
+                         bool zero0) {
+    const int nl = h->n_levels;
+    const int ts = h->tail_start > 0 ? h->tail_start : nl;
+    amg1d::Multi& M = h->multi;
+    bool done[MULTI_MAX_COLS] = {};
+    for (int l = 0; l < nl - 1 && l < ts; ++l) RET(leg_down_multi(h, l, act, na, nPre, alpha, zero0));
+    if (ts < nl) {
+        for (int i = 0; i < na; ++i) {
+            for (int l = ts; l < nl; ++l) M.col[(size_t)act[i]][(size_t)l].cur = 0;
+            cudaError_t te = tail_launch(h->L[ts].m, M.d_tail + (size_t)act[i] * TAIL_MAXL, nl - ts, h->coarse_fac,
+                                         nPre, nPost, alpha, h->tail_plan_, h->stream, h->opt_pdl != 0);
+            if (te != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "f_tail launch failed: %s", cudaGetErrorString(te));
+            h->launch_counter++;
+        }
+    } else {
+        for (int i = 0; i < na; ++i) {
+            ColumnBind cb(h, act[i]);
+            Level& lv = h->L[nl - 1];
+            if (nl > 1 || zero0) lv.cur = 0;
+            RET(op_coarse(h, lv.b.p, lv.x[lv.cur].p));
+        }
+    }
+    for (int l = std::min(nl - 2, ts - 1); l >= 0; --l)
+        RET(leg_up_multi(h, l, act, na, nPost, alpha, want_norm && l == 0, done));
+    for (int i = 0; i < na; ++i) {
+        auto& v = M.col[(size_t)act[i]][0];
+        if (v.cur != 0) {
+            CK(cudaMemcpyAsync(v.x[0].p, v.x[1].p, (size_t)v.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
+            v.cur = 0;
+        }
+        if (want_norm && !done[i]) {
+            ColumnBind cb(h, act[i]);
+            RET(op_resnorm(h, 0, 0));
+        }
+    }
+    return AMG1D_OK;
+}
+
+// run_vcycle for the multi-column set: graph replay keyed by the cycle parameters and the active columns
+int run_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, double alpha, bool want_norm, bool zero0) {
+    if (nPre < 0 || nPost < 0) return fail(h, AMG1D_ERR_ARG, "nPre and nPost must be >= 0");
+    amg1d::Multi& M = h->multi;
+    RET(multi_sync_tail(h));
+    if (!h->opt_graph || h->opt_profile) {
+        const int64_t c0 = h->launch_counter;
+        RET(enqueue_vcycle_multi(h, act, na, nPre, nPost, alpha, want_norm, zero0));
+        M.launches_per_cycle = h->launch_counter - c0;
+        return AMG1D_OK;
+    }
+    unsigned mask = 0;
+    for (int i = 0; i < na; ++i) mask |= 1u << act[i];
+    amg1d::Multi::Graph* ge = nullptr;
+    for (auto& g : M.graphs)
+        if (g.g.exec && g.mask == mask && g.g.pre == nPre && g.g.post == nPost && g.g.alpha == alpha &&
+            g.g.norm == (int)want_norm && g.g.zero0 == (int)zero0)
+            ge = &g;
+    if (!ge) {
+        ge = &M.graphs[0];
+        for (auto& g : M.graphs) if (!g.g.exec) { ge = &g; break; } else if (g.g.stamp < ge->g.stamp) ge = &g;
+        if (ge->g.exec) { cudaGraphExecDestroy(ge->g.exec); ge->g.exec = nullptr; }
+        for (int i = 0; i < na; ++i)
+            if (M.col[(size_t)act[i]][0].cur != 0) return fail(h, AMG1D_ERR_STATE, "internal: level-0 buffer parity");
+        cudaGraph_t g = nullptr;
+        const int64_t c0 = h->launch_counter;
+        CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
+        int rc = enqueue_vcycle_multi(h, act, na, nPre, nPost, alpha, want_norm, zero0);
+        cudaError_t ce = cudaStreamEndCapture(h->stream, &g);
+        if (rc != AMG1D_OK) { if (g) cudaGraphDestroy(g); return rc; }
+        if (ce != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(ce));
+        ge->g.launches = h->launch_counter - c0;
+        h->launch_counter = c0;
+        ce = cudaGraphInstantiate(&ge->g.exec, g, 0);
+        cudaGraphDestroy(g);
+        if (ce != cudaSuccess) { ge->g.exec = nullptr; return fail(h, AMG1D_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(ce)); }
+        ge->g.pre = nPre; ge->g.post = nPost; ge->g.alpha = alpha; ge->g.norm = (int)want_norm; ge->g.zero0 = (int)zero0;
+        ge->mask = mask;
+    }
+    ge->g.stamp = ++h->graph_clock;
+    CK(cudaGraphLaunch(ge->g.exec, h->stream));
+    M.launches_per_cycle = ge->g.launches;
+    h->launch_counter += ge->g.launches;
+    return AMG1D_OK;
+}
+
+int check_multi(amg1d* h, bool need_set) {
+    RET(check_ready(h));
+    if (h->nranks > 1)
+        return fail(h, AMG1D_ERR_UNSUPPORTED, "multi-column problems run on a single GPU (this handle has %d ranks)",
+                    h->nranks);
+    if (need_set && h->multi.k == 0)
+        return fail(h, AMG1D_ERR_STATE, "no multi-column problem set (amg1d_dev_set_problems / amg1d_dev_fill_rhs_random_multi)");
+    return AMG1D_OK;
+}
+
+int check_cols(amg1d* h, int k) {
+    if (k < 1 || k > MULTI_MAX_COLS) return fail(h, AMG1D_ERR_ARG, "column count %d outside [1, %d]", k, MULTI_MAX_COLS);
+    return AMG1D_OK;
+}
+
+int read_multi_scalars(amg1d* h) {
+    CK(cudaMemcpyAsync(h->multi.h_scal, h->multi.d_scal, MULTI_MAX_COLS * MULTI_SLOTS * 8, cudaMemcpyDeviceToHost,
+                       h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return AMG1D_OK;
 }
 
@@ -1702,6 +2028,12 @@ int amg1d_destroy(amg1d_t* h) {
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
     for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
+    for (auto& g : h->multi.graphs) if (g.g.exec) cudaGraphExecDestroy(g.g.exec);
+    for (auto& cl : h->multi.col) for (auto& v : cl) { vec_free(v.x[0]); vec_free(v.x[1]); vec_free(v.b); }
+    for (double* p : h->multi.partial) cudaFree(p);
+    if (h->multi.d_scal) cudaFree(h->multi.d_scal);
+    if (h->multi.h_scal) cudaFreeHost(h->multi.h_scal);
+    if (h->multi.d_tail) cudaFree(h->multi.d_tail);
     vec_free(h->cg_x); vec_free(h->cg_p); vec_free(h->cg_ap);
     for (auto& pr : h->prof) for (auto ev : pr.ev) cudaEventDestroy(ev);
     for (auto& lv : h->L) {
@@ -2476,6 +2808,114 @@ int amg1d_dev_get_solution(amg1d_t* h, double* x) {
     return to_host(h, 0, h->L[0].x[h->L[0].cur].p, x);
 }
 
+// ---- multi-column resident problems ----------------------------------------------------------------------------
+int amg1d_dev_set_problems(amg1d_t* h, int k, const double* X0, const double* B) {
+    RET(check_multi(h, false));
+    RET(check_cols(h, k));
+    if (!B) return fail(h, AMG1D_ERR_ARG, "null B");
+    RET(multi_alloc(h, k));
+    amg1d::Multi& M = h->multi;
+    const int64_t nh = h->L[0].n_host;
+    M.k = 0;
+    M.norm_valid = false;
+    for (int c = 0; c < k; ++c) {
+        auto& v = M.col[(size_t)c][0];
+        RET(to_device(h, 0, B + c * nh, v.b.p));
+        v.cur = 0;
+        if (X0) RET(to_device(h, 0, X0 + c * nh, v.x[0].p));
+        else CK(cudaMemsetAsync(v.x[0].p, 0, (size_t)v.x[0].len * 8, h->stream));
+    }
+    M.k = k;
+    return AMG1D_OK;
+}
+
+int amg1d_dev_fill_rhs_random_multi(amg1d_t* h, int k, uint64_t seed) {
+    RET(check_multi(h, false));
+    RET(check_cols(h, k));
+    Level& l0 = h->L[0];
+    if (l0.perm) return fail(h, AMG1D_ERR_UNSUPPORTED, "random rhs only for unpermuted (DG) fine levels");
+    RET(multi_alloc(h, k));
+    amg1d::Multi& M = h->multi;
+    M.norm_valid = false;
+    for (int c = 0; c < k; ++c) {
+        auto& v = M.col[(size_t)c][0];
+        k_fill_random<<<1184, 256, 0, h->stream>>>(v.b.p, v.b.len, seed + (uint64_t)c, l0.start * l0.m);
+        LAUNCH_CHECK();
+        v.cur = 0;
+        CK(cudaMemsetAsync(v.x[0].p, 0, (size_t)v.x[0].len * 8, h->stream));
+    }
+    M.k = k;
+    return AMG1D_OK;
+}
+
+int amg1d_dev_vcycle_multi(amg1d_t* h, int nPre, int nPost, double alpha, int zero_guess, int with_residual_norms) {
+    RET(check_multi(h, true));
+    amg1d::Multi& M = h->multi;
+    int act[MULTI_MAX_COLS];
+    for (int c = 0; c < M.k; ++c) act[c] = c;
+    M.norm_valid = false;
+    RET(run_vcycle_multi(h, act, M.k, nPre, nPost, alpha, with_residual_norms != 0, zero_guess != 0));
+    M.norm_valid = with_residual_norms != 0;
+    return AMG1D_OK;
+}
+
+int amg1d_dev_residual_norms(amg1d_t* h, double* res) {
+    RET(check_multi(h, true));
+    amg1d::Multi& M = h->multi;
+    if (!M.norm_valid)
+        for (int c = 0; c < M.k; ++c) {
+            ColumnBind cb(h, c);
+            RET(op_resnorm(h, 0, 0));
+        }
+    RET(read_multi_scalars(h));
+    if (res)
+        for (int c = 0; c < M.k; ++c) res[c] = M.h_scal[c * MULTI_SLOTS];
+    return AMG1D_OK;
+}
+
+int amg1d_dev_solve_multi(amg1d_t* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters,
+                          double* res) {
+    RET(check_multi(h, true));
+    if (!res || !iters) return fail(h, AMG1D_ERR_ARG, "null argument");
+    if (maxiter < 0) return fail(h, AMG1D_ERR_ARG, "maxiter must be >= 0");
+    amg1d::Multi& M = h->multi;
+    const int k = M.k;
+    for (int c = 0; c < k; ++c) {
+        iters[c] = 0;
+        ColumnBind cb(h, c);
+        RET(op_norm(h, h->L[0].b.p, nullptr, h->L[0].b.len, 2));
+    }
+    M.norm_valid = false;
+    int act[MULTI_MAX_COLS];
+    int na = k;
+    for (int c = 0; c < k; ++c) act[c] = c;
+    for (int i = 0; i < maxiter && na > 0; ++i) {
+        RET(run_vcycle_multi(h, act, na, nPre, nPost, alpha, true, false));
+        RET(read_multi_scalars(h));
+        int keep = 0;
+        for (int j = 0; j < na; ++j) {
+            const int c = act[j];
+            const double r = M.h_scal[c * MULTI_SLOTS];
+            res[(int64_t)c * maxiter + i] = r;
+            iters[c] = i + 1;
+            if (!(r < tol * M.h_scal[c * MULTI_SLOTS + 2])) act[keep++] = c;   // multigrid()'s stop rule, per column
+        }
+        na = keep;
+    }
+    return AMG1D_OK;
+}
+
+int amg1d_dev_get_solutions(amg1d_t* h, double* X) {
+    RET(check_multi(h, true));
+    if (!X) return fail(h, AMG1D_ERR_ARG, "null X");
+    const int64_t nh = h->L[0].n_host;
+    for (int c = 0; c < h->multi.k; ++c) {
+        auto& v = h->multi.col[(size_t)c][0];
+        RET(to_host(h, 0, v.x[v.cur].p, X + c * nh));
+    }
+    return AMG1D_OK;
+}
+
 int amg1d_synchronize(amg1d_t* h) {
     if (!h) return AMG1D_ERR_ARG;
     CK(cudaStreamSynchronize(h->stream));
@@ -3024,6 +3464,14 @@ int64_t amg1d_get_info(amg1d_t* h, const char* key) {
         int64_t s = 0;
         for (int l = 0; l < h->n_levels - 1; ++l) s += h->L[l].n_glob * h->L[l].m;
         return s;
+    }
+    if (!strcmp(key, "multi_columns")) return h->multi.k;
+    if (!strcmp(key, "multi_launches_per_cycle")) return h->multi.launches_per_cycle;
+    if (!strncmp(key, "multi_legs:", 11)) {         // 1: the multi-column cycle reads this level's operator once for all
+        const int l = atoi(key + 11);               //    columns (fused multi-column legs), 0: once per column
+        if (!valid_level(h, l) || !h->finalized || h->nranks > 1 || l + 1 >= h->n_levels) return 0;
+        if (h->tail_start > 0 && l >= h->tail_start) return 0;
+        return multi_leg_level(h, l) ? 1 : 0;
     }
     return -1;
 }

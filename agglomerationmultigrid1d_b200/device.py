@@ -311,6 +311,53 @@ class DeviceHierarchy:
         self._ck(self._lib.amg1d_dev_get_solution(self._h, capi.dptr(x)))
         return x
 
+    # ---- multi-column device-resident set (up to capi.MAX_COLS right-hand sides per V-cycle) ----------------------
+    def _check_cols(self, X):
+        if X.ndim != 2 or X.shape[0] != self.n_dof[0] or not 1 <= X.shape[1] <= capi.MAX_COLS:
+            raise ValueError(f"DimensionMismatch: expected ({self.n_dof[0]}, k) with 1 <= k <= {capi.MAX_COLS}, "
+                             f"got {X.shape}")
+
+    def dev_set_problems(self, X0, B):
+        """Upload k = B.shape[1] right-hand sides (and initial guesses X0, None = 0), each of shape (n_dof, k)."""
+        B = np.asfortranarray(B, dtype=np.float64)
+        self._check_cols(B)
+        if X0 is not None:
+            X0 = np.asfortranarray(X0, dtype=np.float64)
+            if X0.shape != B.shape:
+                raise ValueError(f"DimensionMismatch: X0 {X0.shape} vs B {B.shape}")
+        PD = C.POINTER(C.c_double)
+        self._ck(self._lib.amg1d_dev_set_problems(self._h, B.shape[1], X0.ctypes.data_as(PD) if X0 is not None else None,
+                                                  B.ctypes.data_as(PD)))
+
+    def dev_fill_rhs_random_multi(self, k, seed=0):
+        """Column c gets the right-hand side of dev_fill_rhs_random(seed + c); x = 0."""
+        self._ck(self._lib.amg1d_dev_fill_rhs_random_multi(self._h, int(k), seed))
+
+    def dev_vcycle_multi(self, nPre=3, nPost=3, alpha=2.0 / 3.0, zero_guess=False, with_residual_norms=False):
+        self._ck(self._lib.amg1d_dev_vcycle_multi(self._h, nPre, nPost, alpha, int(bool(zero_guess)),
+                                                  int(bool(with_residual_norms))))
+
+    def dev_residual_norms(self):
+        k = self.info("multi_columns")
+        res = np.zeros(max(k, 1))
+        self._ck(self._lib.amg1d_dev_residual_norms(self._h, capi.dptr(res)))
+        return res[:k].copy()
+
+    def dev_solve_multi(self, maxiter, tol, nPre=3, nPost=3, alpha=2.0 / 3.0):
+        """``multigrid`` on every column of the set; returns (iters, [res per column])."""
+        k = self.info("multi_columns")
+        res = np.zeros(max(maxiter, 1) * max(k, 1))
+        it = (C.c_int * max(k, 1))()
+        self._ck(self._lib.amg1d_dev_solve_multi(self._h, maxiter, tol, nPre, nPost, alpha, it, capi.dptr(res)))
+        iters = [int(it[c]) for c in range(k)]
+        return iters, [res[c * maxiter:c * maxiter + iters[c]].copy() for c in range(k)]
+
+    def dev_get_solutions(self):
+        k = self.info("multi_columns")
+        X = np.zeros((self.n_dof[0], max(k, 1)), order="F")
+        self._ck(self._lib.amg1d_dev_get_solutions(self._h, X.ctypes.data_as(C.POINTER(C.c_double))))
+        return X[:, :k]
+
     def synchronize(self):
         self._ck(self._lib.amg1d_synchronize(self._h))
 

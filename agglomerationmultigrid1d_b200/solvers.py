@@ -5,6 +5,7 @@ libamg1d.so (the GPU).  There is no CPU implementation behind them.
 
     multigrid_v_cycle(H, x0, b; nPre=3, nPost=3, alpha=2/3) -> x            src/solvers.jl:19-50
     ldiv(H, b) -> b overwritten / ldiv(y, H, b) -> y overwritten            src/solvers.jl:63-92
+        (b, y may be n_dof x k matrices: the columns share V-cycles, up to 8 at a time)
     pcg(H, x0, b, maxiter, tol) -> (x, iter, res)      CG with ldiv! as preconditioner (the hook's purpose)
     multigrid(H, x0, b, maxiter, tol) -> (x, iter, res, err)                src/solvers.jl:116-139
     iterative_smoother_solve(A, smoother, x0, b; maxiter, tol, alpha)       src/solvers.jl:189-213
@@ -14,6 +15,7 @@ import numpy as np
 import scipy.sparse as sp
 
 from . import blocks as blk
+from ._capi import MAX_COLS
 from .device import DeviceHierarchy
 from .smoother import AbstractSmoother, AdditiveSchwarzSmoother, schwarz_tridiag_blocks, smoother_inverse
 
@@ -29,7 +31,8 @@ def multigrid_v_cycle(H, x0, b, nPre=3, nPost=3, alpha=2.0 / 3.0):
 
 
 def ldiv(*args):
-    """``ldiv!(H, b)``: b <- one V-cycle from a zero guess; ``ldiv!(y, H, b)``: y <- the same."""
+    """``ldiv!(H, b)``: b <- one V-cycle from a zero guess; ``ldiv!(y, H, b)``: y <- the same.  A 2-D b (n_dof x k,
+    any k) is ``ldiv!(Y, H, B)``: every column as by the 1-D call, up to 8 columns per V-cycle."""
     if len(args) == 2:
         H, b = args
         out = b
@@ -37,7 +40,21 @@ def ldiv(*args):
         out, H, b = args
     else:
         raise TypeError("ldiv(H, b) or ldiv(y, H, b)")
-    out[:] = _device_of(H).ldiv(b)          # zero guess inside the library: no x0 upload, first sweep skips A
+    dev = _device_of(H)
+    if np.ndim(b) == 2:
+        # ldiv!(Y, H, B): the columns in sets of up to 8 through the multi-column cycle, each column bit-identical
+        # to ldiv!(y, H, b) on it alone
+        B = np.asarray(b, dtype=np.float64)
+        if np.shape(out) != B.shape:
+            raise ValueError(f"DimensionMismatch: Y {np.shape(out)} vs B {B.shape}")
+        Y = np.empty(B.shape, order="F")
+        for c0 in range(0, B.shape[1], MAX_COLS):
+            dev.dev_set_problems(None, B[:, c0:c0 + MAX_COLS])
+            dev.dev_vcycle_multi(zero_guess=True)
+            Y[:, c0:c0 + MAX_COLS] = dev.dev_get_solutions()
+        out[:] = Y
+        return None
+    out[:] = dev.ldiv(b)          # zero guess inside the library: no x0 upload, first sweep skips A
     return None
 
 

@@ -259,6 +259,32 @@ int amg1d_dev_vcycle(amg1d_t* h, int nPre, int nPost, double alpha, int with_res
 int amg1d_dev_residual_norm(amg1d_t* h, double* res);              /* ||A x - b||_2, synchronises */
 int amg1d_dev_rhs_norm(amg1d_t* h, double* nb);                    /* ||b||_2, synchronises */
 int amg1d_dev_get_solution(amg1d_t* h, double* x);                 /* device -> host */
+
+/* ---- multi-column device-resident problems ----------------------------------------------------------
+ * ldiv!(Y, H, B) / multigrid_v_cycle / multigrid (src/solvers.jl:19-50, :63-92, :116-139) for k <= AMG1D_MAX_COLS
+ * right-hand sides at once: the reference's ldiv! methods make MeshHierarchy a preconditioner, which block Krylov
+ * methods, time steppers and multi-load problems apply to many vectors.  One V-cycle serves all columns: on levels
+ * with fused legs (amg1d_get_info("multi_legs:<level>") = 1) each leg reads the level's operator once for all columns;
+ * the other levels, the coarse tail and the coarse solve run once per column.  Every column's iterate and residual
+ * norm are bit-identical to the single-column calls on that column.  Single GPU handles only (AMG1D_ERR_UNSUPPORTED
+ * otherwise).  The column set is separate device storage (three vectors per level and column, counted in
+ * "device_bytes", allocated at the first call and grown when k grows): the single-column resident problem of
+ * amg1d_dev_set_problem is neither read nor written by these calls, nor the column set by that one.  X0, B, X are
+ * n_dof_host x k column-major (level 0's host vector length); X0 == NULL: zero initial guesses. */
+#define AMG1D_MAX_COLS 8
+int amg1d_dev_set_problems(amg1d_t* h, int k, const double* X0, const double* B);   /* host -> device */
+/* column c gets exactly the b of amg1d_dev_fill_rhs_random(h, seed + c); x = 0 */
+int amg1d_dev_fill_rhs_random_multi(amg1d_t* h, int k, uint64_t seed);
+/* one V-cycle on every column, asynchronous; zero_guess = 1: the ldiv! form of amg1d_ldiv (x0 = 0, not read, the first
+ * pre-smoothing sweep skips A); with_residual_norms = 1 leaves ||b - A x||_2 of every column on the device */
+int amg1d_dev_vcycle_multi(amg1d_t* h, int nPre, int nPost, double alpha, int zero_guess, int with_residual_norms);
+int amg1d_dev_residual_norms(amg1d_t* h, double* res);             /* k values ||b - A x||_2, synchronises */
+/* multigrid() per column: iters (k ints), res (maxiter x k, column-major).  A column that meets its own stop rule
+ * leaves the set of cycled columns, so its iterate, iters[c] and res history equal amg1d_dev_solve on it alone. */
+int amg1d_dev_solve_multi(amg1d_t* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters,
+                          double* res);
+int amg1d_dev_get_solutions(amg1d_t* h, double* X);                /* device -> host, n_dof_host x k */
+
 int amg1d_synchronize(amg1d_t* h);
 void* amg1d_stream(amg1d_t* h);                                    /* the cudaStream_t in use */
 void* amg1d_dev_ptr(amg1d_t* h, int level, int which);             /* raw device pointer (AMG1D_VEC_*) */
@@ -307,7 +333,12 @@ int64_t amg1d_get_info(amg1d_t* h, const char* key); /* "kernel_launches", "laun
                                                         pipelined legs), "dinv_pivots:<level>" (1 = that
                                                         inversion keeps the partial-pivoting chain),
                                                         "pattern:<level>" (1 = the
-                                                        level has a pattern table), the option keys,
+                                                        level has a pattern table), "multi_columns"
+                                                        (k of the multi-column set, 0: none),
+                                                        "multi_legs:<level>" (1 = the multi-column
+                                                        cycle reads the level's operator once for all
+                                                        columns), "multi_launches_per_cycle",
+                                                        the option keys,
                                                         ... (-1: unknown key) */
 
 /* With option "profile" = 1 every V-cycle runs un-graphed and brackets each level's down leg (leg 0:

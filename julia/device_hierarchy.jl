@@ -201,6 +201,45 @@ end
 dev_solution(D::DeviceHierarchy) = (x = Vector{Float64}(undef, D.nDof[1]);
     amg1d_check(D.handle, ccall((:amg1d_dev_get_solution, libamg1d), Cint, (Ptr{Cvoid}, Ptr{Float64}), D.handle, x)); x)
 
+# ---- up to AMG1D_MAX_COLS right-hand sides per V-cycle (multi-column resident set) -------------------------------
+# UNVERIFIED like the rest of this file (no Julia in this repository's build environment); the Python driver
+# (device.py: dev_set_problems ... dev_get_solutions, solvers.ldiv with a 2-D b) is the tested path.
+const AMG1D_MAX_COLS = 8
+dev_set_problems!(D::DeviceHierarchy, X0::Union{Nothing,AbstractMatrix}, B::AbstractMatrix) =
+    (Bd = Matrix{Float64}(B); Xd = X0 === nothing ? Ptr{Float64}(C_NULL) : Matrix{Float64}(X0);
+     GC.@preserve Bd Xd amg1d_check(D.handle, ccall((:amg1d_dev_set_problems, libamg1d), Cint,
+        (Ptr{Cvoid}, Cint, Ptr{Float64}, Ptr{Float64}), D.handle, size(Bd, 2), Xd, Bd)))
+dev_fill_rhs_random_multi!(D::DeviceHierarchy, k::Integer, seed::Integer) =
+    amg1d_check(D.handle, ccall((:amg1d_dev_fill_rhs_random_multi, libamg1d), Cint, (Ptr{Cvoid}, Cint, UInt64),
+                                D.handle, k, seed))
+dev_vcycle_multi!(D::DeviceHierarchy; nPre::Integer = 3, nPost::Integer = 3, alpha::AbstractFloat = 2.0 / 3.0,
+                  zeroGuess::Bool = false, withResidualNorms::Bool = false) =
+    amg1d_check(D.handle, ccall((:amg1d_dev_vcycle_multi, libamg1d), Cint, (Ptr{Cvoid}, Cint, Cint, Float64, Cint, Cint),
+                                D.handle, nPre, nPost, alpha, zeroGuess ? 1 : 0, withResidualNorms ? 1 : 0))
+dev_residual_norms(D::DeviceHierarchy) = (res = zeros(get_info(D, "multi_columns"));
+    amg1d_check(D.handle, ccall((:amg1d_dev_residual_norms, libamg1d), Cint, (Ptr{Cvoid}, Ptr{Float64}), D.handle, res)); res)
+function multigrid_resident_multi(D::DeviceHierarchy, maxiter::Integer, tol::AbstractFloat)
+    k = get_info(D, "multi_columns"); res = zeros(maxiter, k); it = zeros(Cint, k)
+    amg1d_check(D.handle, ccall((:amg1d_dev_solve_multi, libamg1d), Cint,
+        (Ptr{Cvoid}, Cint, Float64, Cint, Cint, Float64, Ptr{Cint}, Ptr{Float64}),
+        D.handle, maxiter, tol, 3, 3, 2.0 / 3.0, it, res))
+    return Int.(it), [res[1:it[c], c] for c in 1:k]
+end
+dev_solutions(D::DeviceHierarchy) = (X = Matrix{Float64}(undef, D.nDof[1], get_info(D, "multi_columns"));
+    amg1d_check(D.handle, ccall((:amg1d_dev_get_solutions, libamg1d), Cint, (Ptr{Cvoid}, Ptr{Float64}), D.handle, X)); X)
+
+# ldiv!(Y, H, B): every column as ldiv!(y, H, b), up to AMG1D_MAX_COLS columns per V-cycle
+function ldiv!(Y::AbstractMatrix, D::DeviceHierarchy, B::AbstractMatrix)
+    size(Y) == size(B) || throw(DimensionMismatch("Y $(size(Y)) vs B $(size(B))"))
+    for c0 in 1:AMG1D_MAX_COLS:size(B, 2)
+        cols = c0:min(c0 + AMG1D_MAX_COLS - 1, size(B, 2))
+        dev_set_problems!(D, nothing, B[:, cols])
+        dev_vcycle_multi!(D; zeroGuess = true)
+        Y[:, cols] = dev_solutions(D)
+    end
+    return
+end
+
 function apply_smoother(D::DeviceHierarchy, level::Integer, B::AbstractVecOrMat; alpha::Float64 = 1.0)
     Bd = Matrix{Float64}(reshape(Array(B), size(B, 1), :)); Y = similar(Bd)
     amg1d_check(D.handle, ccall((:amg1d_apply_smoother, libamg1d), Cint,
@@ -261,3 +300,4 @@ multigrid(H::MeshHierarchy, x0::AbstractVector, b::AbstractVector, maxiter::Inte
     multigrid(device(H), H, x0, b, maxiter, tol)
 ldiv!(y::AbstractVector, H::MeshHierarchy, b::AbstractVector) = ldiv!(y, device(H), b)
 ldiv!(H::MeshHierarchy, b::AbstractVector) = ldiv!(b, device(H), b)
+ldiv!(Y::AbstractMatrix, H::MeshHierarchy, B::AbstractMatrix) = ldiv!(Y, device(H), B)
