@@ -76,6 +76,8 @@ PROTOTYPES = {
     "amg1d_dev_residual_norms": (C.c_int, [_h, _pd]),
     "amg1d_dev_solve_multi": (C.c_int, [_h, C.c_int, C.c_double, C.c_int, C.c_int, C.c_double, C.POINTER(C.c_int),
                                         _pd]),
+    "amg1d_dev_pcg_multi": (C.c_int, [_h, C.c_int, C.c_double, C.c_int, C.c_int, C.c_double, C.POINTER(C.c_int),
+                                      _pd]),
     "amg1d_dev_get_solutions": (C.c_int, [_h, _pd]),
     "amg1d_synchronize": (C.c_int, [_h]),
     "amg1d_stream": (C.c_void_p, [_h]),

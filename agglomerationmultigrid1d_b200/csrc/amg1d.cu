@@ -30,7 +30,8 @@
 #define AMG1D_VERSION 100
 #define PAD_FRONT 64  // doubles in front of element 0 (ghost elements live at the end of them)
 #define PAD_BACK 64
-#define MULTI_SLOTS 4  // device scalars per column of the multi-column set (slot 0: ||b - A x||, 2: ||b||)
+#define MULTI_SLOTS 8  // device scalars per column of the multi-column set (slot 0: ||b - A x||, 2: ||b||; the CG_*
+                       // slots of amg1d_dev_pcg_multi up to CG_RZ_NEW = 7)
 static_assert(MULTI_MAX_COLS == AMG1D_MAX_COLS, "kernels_multi.cuh and amg1d.h disagree on the column limit");
 
 namespace {
@@ -234,7 +235,11 @@ struct amg1d {
         TailLevel* d_tail = nullptr;               // MULTI_MAX_COLS x TAIL_MAXL descriptors of the single-CTA tail
         uint64_t tail_synced = ~0ull;              // tail_gen that d_tail was filled for
         bool norm_valid = false;                   // d_scal slot 0 of every column holds ||b - A x|| of its iterate
+        bool rhs_consumed = false;                 // amg1d_dev_pcg_multi turned the right-hand sides into CG residuals
         int64_t launches_per_cycle = 0;
+        struct CgCol { DVec x, p, ap; };           // per column: CG solution, search direction, A p on level 0
+        std::vector<CgCol> cg;                     // grown by amg1d_dev_pcg_multi only
+        int64_t pcg_launches = 0;                  // launches of the last PCG iteration outside the V-cycle
         struct Graph { GraphEntry g; unsigned mask = 0; };   // keyed as graphs[] plus the active-column set
         Graph graphs[4];
     } multi;
@@ -1676,13 +1681,17 @@ int run_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, doub
     return AMG1D_OK;
 }
 
-int check_multi(amg1d* h, bool need_set) {
+// need_rhs: the call reads the set's right-hand sides, which amg1d_dev_pcg_multi consumes
+int check_multi(amg1d* h, bool need_set, bool need_rhs = true) {
     RET(check_ready(h));
     if (h->nranks > 1)
         return fail(h, AMG1D_ERR_UNSUPPORTED, "multi-column problems run on a single GPU (this handle has %d ranks)",
                     h->nranks);
     if (need_set && h->multi.k == 0)
         return fail(h, AMG1D_ERR_STATE, "no multi-column problem set (amg1d_dev_set_problems / amg1d_dev_fill_rhs_random_multi)");
+    if (need_set && need_rhs && h->multi.rhs_consumed)
+        return fail(h, AMG1D_ERR_STATE, "the multi-column right-hand sides became CG residuals in amg1d_dev_pcg_multi; "
+                    "install a set again (amg1d_dev_set_problems / amg1d_dev_fill_rhs_random_multi)");
     return AMG1D_OK;
 }
 
@@ -2031,6 +2040,7 @@ int amg1d_destroy(amg1d_t* h) {
     for (auto& g : h->multi.graphs) if (g.g.exec) cudaGraphExecDestroy(g.g.exec);
     for (auto& cl : h->multi.col) for (auto& v : cl) { vec_free(v.x[0]); vec_free(v.x[1]); vec_free(v.b); }
     for (double* p : h->multi.partial) cudaFree(p);
+    for (auto& g : h->multi.cg) { vec_free(g.x); vec_free(g.p); vec_free(g.ap); }
     if (h->multi.d_scal) cudaFree(h->multi.d_scal);
     if (h->multi.h_scal) cudaFreeHost(h->multi.h_scal);
     if (h->multi.d_tail) cudaFree(h->multi.d_tail);
@@ -2826,6 +2836,7 @@ int amg1d_dev_set_problems(amg1d_t* h, int k, const double* X0, const double* B)
         else CK(cudaMemsetAsync(v.x[0].p, 0, (size_t)v.x[0].len * 8, h->stream));
     }
     M.k = k;
+    M.rhs_consumed = false;
     return AMG1D_OK;
 }
 
@@ -2845,6 +2856,7 @@ int amg1d_dev_fill_rhs_random_multi(amg1d_t* h, int k, uint64_t seed) {
         CK(cudaMemsetAsync(v.x[0].p, 0, (size_t)v.x[0].len * 8, h->stream));
     }
     M.k = k;
+    M.rhs_consumed = false;
     return AMG1D_OK;
 }
 
@@ -2906,7 +2918,7 @@ int amg1d_dev_solve_multi(amg1d_t* h, int maxiter, double tol, int nPre, int nPo
 }
 
 int amg1d_dev_get_solutions(amg1d_t* h, double* X) {
-    RET(check_multi(h, true));
+    RET(check_multi(h, true, false));
     if (!X) return fail(h, AMG1D_ERR_ARG, "null X");
     const int64_t nh = h->L[0].n_host;
     for (int c = 0; c < h->multi.k; ++c) {
@@ -3149,6 +3161,175 @@ int pcg_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double alpha
                     "or the V-cycle preconditioner is not symmetric positive definite)", it);
     return AMG1D_OK;
 }
+
+// ---- pcg_run on every column of the multi-column set (amg1d_dev_pcg_multi) --------------------------------------
+// Column c's level-0 CG vectors; allocated at the first call and grown with k, a failed allocation releases what it took.
+int pcg_multi_alloc(amg1d* h, int k) {
+    amg1d::Multi& M = h->multi;
+    const Level& l0 = h->L[0];
+    while ((int)M.cg.size() < k) {
+        amg1d::Multi::CgCol g;
+        int rc = vec_alloc(h, g.x, l0.n, l0.m);
+        if (rc == AMG1D_OK) rc = vec_alloc(h, g.p, l0.n, l0.m);
+        if (rc == AMG1D_OK) rc = vec_alloc(h, g.ap, l0.n, l0.m);
+        if (rc != AMG1D_OK) {
+            for (DVec* d : {&g.x, &g.p, &g.ap})
+                if (d->raw) { h->device_bytes -= vec_bytes(*d); vec_free(*d); }
+            cudaGetLastError();                  // an out-of-memory status must not surface at the next launch check
+            return fail(h, rc, "CG vectors of column %d of the multi-column set: %s", (int)M.cg.size(), h->err.c_str());
+        }
+        M.cg.push_back(g);
+    }
+    return AMG1D_OK;
+}
+
+// The vectors, reduction scratch and scalar windows of the active columns act[0..na), entry i for column act[i].
+struct CgMultiVecs {
+    ColVecs X, R, P, AP, Z, part, scal;
+    CgMultiVecs(amg1d* h, const int* act, int na) : X(), R(), P(), AP(), Z(), part(), scal() {
+        amg1d::Multi& M = h->multi;
+        for (int i = 0; i < na; ++i) {
+            const int c = act[i];
+            auto& v = M.col[(size_t)c][0];
+            X.v[i] = M.cg[(size_t)c].x.p;
+            P.v[i] = M.cg[(size_t)c].p.p;
+            AP.v[i] = M.cg[(size_t)c].ap.p;
+            R.v[i] = v.b.p;                      // the residual lives in the column's level-0 rhs buffer, as in pcg_run
+            Z.v[i] = v.x[v.cur].p;               // the preconditioned residual: the column's level-0 iterate
+            part.v[i] = M.partial[(size_t)c];
+            scal.v[i] = M.d_scal + c * MULTI_SLOTS;
+        }
+    }
+};
+
+// op_sum_partials (take_sqrt 0) / op_reduce_partials (take_sqrt 1) of every active column in one launch per stage
+int reduce_partials_multi(amg1d* h, const CgMultiVecs& v, int na, int64_t np, int slot, int take_sqrt) {
+    ColVecs src = v.part;
+    if (np > 8192) {
+        ColVecs st2 = {};
+        for (int i = 0; i < na; ++i) st2.v[i] = v.part.v[i] + h->partial_cap;
+        k_sum_partial_multi<<<dim3(256, na), AMG1D_RED_THREADS, 0, h->stream>>>(v.part, np, st2);
+        h->launch_counter++;
+        src = st2;
+        np = 256;
+    }
+    k_reduce_final_multi<<<dim3(1, na), AMG1D_RED_THREADS, 0, h->stream>>>(src, (int)np, v.scal, slot, take_sqrt);
+    h->launch_counter++;
+    LAUNCH_CHECK();
+    return AMG1D_OK;
+}
+
+// op_matvec_dot(h, 0, x_c, y_c, slot) for every active column: one launch that reads level 0's operator once where
+// op_matvec_dot would take the fused kernel (the same predicate, hence the same partial sums), its own code per
+// column (ColumnBind) elsewhere
+int matvec_dot_multi(amg1d* h, const int* act, int na, const CgMultiVecs& v, const ColVecs& x, const ColVecs& y,
+                     int slot) {
+    Level& l0 = h->L[0];
+    MatvecCols mc = {};
+    for (int i = 0; i < na; ++i) {
+        mc.x[i] = x.v[i];
+        mc.y[i] = y.v[i];
+        mc.partial[i] = slot >= 0 ? v.part.v[i] : nullptr;
+    }
+    int nb = 0;
+    if (h->opt_fused && fused_matvec_dot_multi(l0.md, l0.mat, mc, na, l0.n, h->partial_cap, &nb, h->stream)) {
+        h->launch_counter++;
+        LAUNCH_CHECK();
+        return slot >= 0 ? reduce_partials_multi(h, v, na, nb, slot, 0) : AMG1D_OK;
+    }
+    for (int i = 0; i < na; ++i) {
+        ColumnBind cb(h, act[i]);
+        RET(op_matvec_dot(h, 0, x.v[i], y.v[i], slot));
+    }
+    return AMG1D_OK;
+}
+
+// pcg_run step for step on every column of the set, the columns that are still iterating batched into each launch.
+// The initial guess is the column's resident iterate, the solution becomes it; the right-hand side becomes the residual.
+int pcg_multi_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters, double* res) {
+    Level& l0 = h->L[0];
+    amg1d::Multi& M = h->multi;
+    const int k = M.k;
+    const int64_t N = l0.n * l0.m;
+    const size_t bytes = (size_t)l0.x[0].len * 8;
+    RET(pcg_multi_alloc(h, k));
+    int act[MULTI_MAX_COLS];
+    int na = k;
+    for (int c = 0; c < k; ++c) {
+        act[c] = c;
+        iters[c] = 0;
+        auto& v = M.col[(size_t)c][0];
+        CK(cudaMemcpyAsync(M.cg[(size_t)c].x.p, v.x[v.cur].p, bytes, cudaMemcpyDeviceToDevice, h->stream));
+    }
+    M.norm_valid = false;
+    M.rhs_consumed = true;
+    const int nbv = (int)std::max<int64_t>(1, std::min<int64_t>(AMG1D_RED_BLOCKS, (N + AMG1D_RED_THREADS - 1) / AMG1D_RED_THREADS));
+    const dim3 gv(nbv, na), gs(1, na);
+    {
+        const CgMultiVecs v(h, act, na);
+        k_sqdiff_partial_multi<<<gv, AMG1D_RED_THREADS, 0, h->stream>>>(v.R, N, v.part);           // ||b||
+        k_reduce_final_multi<<<gs, AMG1D_RED_THREADS, 0, h->stream>>>(v.part, nbv, v.scal, CG_NB, 1);
+        h->launch_counter += 2;
+        LAUNCH_CHECK();
+        RET(matvec_dot_multi(h, act, na, v, v.X, v.AP, -1));                                       // r = b - A x0
+        k_axpy_multi<<<gv, AMG1D_RED_THREADS, 0, h->stream>>>(v.R, v.AP, N, -1.0);
+        k_sqdiff_partial_multi<<<gv, AMG1D_RED_THREADS, 0, h->stream>>>(v.R, N, v.part);
+        k_reduce_final_multi<<<gs, AMG1D_RED_THREADS, 0, h->stream>>>(v.part, nbv, v.scal, CG_RES, 1);
+        h->launch_counter += 3;
+        LAUNCH_CHECK();
+    }
+    RET(read_multi_scalars(h));
+    na = 0;
+    for (int c = 0; c < k; ++c) {
+        const double* s = M.h_scal + c * MULTI_SLOTS;
+        if (!std::isfinite(s[CG_RES]) || !std::isfinite(s[CG_NB]))
+            return fail(h, AMG1D_ERR_ARG, "amg1d_dev_pcg_multi: non-finite right-hand side or initial guess in column %d", c);
+        if (!(s[CG_NB] == 0.0 || s[CG_RES] <= tol * s[CG_NB])) act[na++] = c;   // pcg_run's initial-residual test
+    }
+    for (int i = 0; i < maxiter && na > 0; ++i) {
+        // z = M^-1 r: one multi-column V-cycle from a zero guess with right-hand sides r (already in place)
+        RET(run_vcycle_multi(h, act, na, nPre, nPost, alpha, false, true));
+        const int64_t c0 = h->launch_counter;
+        const CgMultiVecs v(h, act, na);
+        const dim3 g(nbv, na);
+        k_dot_partial_multi<<<g, AMG1D_RED_THREADS, 0, h->stream>>>(v.R, v.Z, N, v.part);
+        h->launch_counter++;
+        LAUNCH_CHECK();
+        RET(reduce_partials_multi(h, v, na, nbv, i == 0 ? CG_RZ : CG_RZ_NEW, 0));
+        if (i > 0) { k_cg_beta_multi<<<1, na, 0, h->stream>>>(v.scal); h->launch_counter++; }
+        k_cg_direction_multi<<<g, AMG1D_RED_THREADS, 0, h->stream>>>(v.P, v.Z, N, v.scal, i == 0 ? 1 : 0);
+        h->launch_counter++;
+        LAUNCH_CHECK();
+        RET(matvec_dot_multi(h, act, na, v, v.P, v.AP, CG_PAP));
+        k_cg_alpha_multi<<<1, na, 0, h->stream>>>(v.scal);
+        k_cg_update_multi<<<g, AMG1D_RED_THREADS, 0, h->stream>>>(v.X, v.R, v.P, v.AP, N, v.scal, v.part);
+        h->launch_counter += 2;
+        LAUNCH_CHECK();
+        RET(reduce_partials_multi(h, v, na, nbv, CG_RES, 1));                                  // ||r||_2
+        M.pcg_launches = h->launch_counter - c0;
+        RET(read_multi_scalars(h));
+        int keep = 0;
+        for (int j = 0; j < na; ++j) {
+            const int c = act[j];
+            const double r = M.h_scal[c * MULTI_SLOTS + CG_RES];
+            res[(int64_t)c * maxiter + i] = r;
+            iters[c] = i + 1;
+            if (r >= tol * M.h_scal[c * MULTI_SLOTS + CG_NB]) act[keep++] = c;                   // also stops on NaN
+        }
+        na = keep;
+    }
+    for (int c = 0; c < k; ++c) {                                  // the solutions become the resident iterates
+        auto& v = M.col[(size_t)c][0];
+        v.cur = 0;
+        CK(cudaMemcpyAsync(v.x[0].p, M.cg[(size_t)c].x.p, bytes, cudaMemcpyDeviceToDevice, h->stream));
+    }
+    for (int c = 0; c < k; ++c)
+        if (iters[c] > 0 && !std::isfinite(res[(int64_t)c * maxiter + iters[c] - 1]))
+            return fail(h, AMG1D_ERR_ARG, "amg1d_dev_pcg_multi: breakdown in column %d at iteration %d (non-finite "
+                        "residual: the operator or the V-cycle preconditioner is not symmetric positive definite)",
+                        c, iters[c]);
+    return AMG1D_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -3176,6 +3357,14 @@ int amg1d_dev_pcg(amg1d_t* h, int maxiter, double tol, int nPre, int nPost, doub
     l0.cur = 0;                                                  // the solution becomes the resident iterate
     CK(cudaMemcpyAsync(l0.x[0].p, h->cg_x.p, (size_t)l0.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
     return AMG1D_OK;
+}
+
+int amg1d_dev_pcg_multi(amg1d_t* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters,
+                        double* res) {
+    RET(check_multi(h, true));
+    if (!res || !iters) return fail(h, AMG1D_ERR_ARG, "null argument");
+    if (maxiter < 0) return fail(h, AMG1D_ERR_ARG, "maxiter must be >= 0");
+    return pcg_multi_run(h, maxiter, tol, nPre, nPost, alpha, iters, res);
 }
 
 int amg1d_apply_smoother(amg1d_t* h, int level, double* Y, const double* B, int64_t n_rhs,
@@ -3467,6 +3656,7 @@ int64_t amg1d_get_info(amg1d_t* h, const char* key) {
     }
     if (!strcmp(key, "multi_columns")) return h->multi.k;
     if (!strcmp(key, "multi_launches_per_cycle")) return h->multi.launches_per_cycle;
+    if (!strcmp(key, "multi_pcg_launches_per_iteration")) return h->multi.pcg_launches;
     if (!strncmp(key, "multi_legs:", 11)) {         // 1: the multi-column cycle reads this level's operator once for all
         const int l = atoi(key + 11);               //    columns (fused multi-column legs), 0: once per column
         if (!valid_level(h, l) || !h->finalized || h->nranks > 1 || l + 1 >= h->n_levels) return 0;

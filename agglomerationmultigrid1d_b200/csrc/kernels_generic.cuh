@@ -264,89 +264,182 @@ __device__ __forceinline__ double block_sum(double v) {
     return t;  // valid in thread 0
 }
 
-// partial[b] = sum over a grid-stride slice of (a[i] - c[i])^2   (c may be null)
-__global__ void k_sqdiff_partial(const double* __restrict__ a, const double* __restrict__ c,
-                                 int64_t n, double* __restrict__ partial) {
+// The per-element statements of the reductions and CG vector updates below, over this block's grid-stride slice
+// (block blockIdx.x of gridDim.x).  The single-column kernels and their multi-column forms (column = blockIdx.y, the
+// same gridDim.x per column) both call them, so each column's partial sums are those of the single-column kernel.
+#define GRID_SLICE(i, n) \
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < (n); i += (int64_t)gridDim.x * blockDim.x)
+
+__device__ __forceinline__ double sqdiff_slice(const double* __restrict__ a, const double* __restrict__ c, int64_t n) {
     double s = 0.0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
-         i += (int64_t)gridDim.x * blockDim.x) {
+    GRID_SLICE(i, n) {
         const double d = c ? a[i] - c[i] : a[i];
         s = fma(d, d, s);
     }
-    s = block_sum(s);
+    return s;
+}
+
+__device__ __forceinline__ double dot_slice(const double* __restrict__ a, const double* __restrict__ c, int64_t n) {
+    double s = 0.0;
+    GRID_SLICE(i, n) s = fma(a[i], c[i], s);
+    return s;
+}
+
+__device__ __forceinline__ double sum_slice(const double* __restrict__ partial, int64_t np) {
+    double s = 0.0;
+    GRID_SLICE(i, np) s += partial[i];
+    return s;
+}
+
+// one block: the final stage, in a fixed order (thread t sums entries t, t + blockDim.x, ...)
+__device__ __forceinline__ double reduce_final_sum(const double* __restrict__ partial, int np) {
+    double s = 0.0;
+    for (int i = threadIdx.x; i < np; i += blockDim.x) s += partial[i];
+    return block_sum(s);
+}
+
+// partial[b] = sum over a grid-stride slice of (a[i] - c[i])^2   (c may be null)
+__global__ void k_sqdiff_partial(const double* __restrict__ a, const double* __restrict__ c,
+                                 int64_t n, double* __restrict__ partial) {
+    const double s = block_sum(sqdiff_slice(a, c, n));
     if (threadIdx.x == 0) partial[blockIdx.x] = s;
 }
 
 // partial[b] = sum over a grid-stride slice of a[i] * c[i]
 __global__ void k_dot_partial(const double* __restrict__ a, const double* __restrict__ c, int64_t n,
                               double* __restrict__ partial) {
-    double s = 0.0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
-         i += (int64_t)gridDim.x * blockDim.x)
-        s = fma(a[i], c[i], s);
-    s = block_sum(s);
+    const double s = block_sum(dot_slice(a, c, n));
     if (threadIdx.x == 0) partial[blockIdx.x] = s;
 }
 
 // ---- conjugate gradients (amg1d_pcg): scalars live in the device scalar array ------------------------
 enum { CG_RES = 0, CG_NB = 2, CG_RZ = 3, CG_PAP = 4, CG_ALPHA = 5, CG_BETA = 6, CG_RZ_NEW = 7 };
 
-// y += a x
-__global__ void k_axpy(double* __restrict__ y, const double* __restrict__ x, int64_t n, double a) {
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
-         i += (int64_t)gridDim.x * blockDim.x)
-        y[i] = fma(a, x[i], y[i]);
+__device__ __forceinline__ void axpy_slice(double* __restrict__ y, const double* __restrict__ x, int64_t n, double a) {
+    GRID_SLICE(i, n) y[i] = fma(a, x[i], y[i]);
 }
 
 // alpha = rz / pAp
 // (a zero denominator - b = 0, or an exact x0 - gives a zero step instead of 0/0 = NaN)
-__global__ void k_cg_alpha(double* s) { s[CG_ALPHA] = s[CG_PAP] != 0.0 ? s[CG_RZ] / s[CG_PAP] : 0.0; }
+__device__ __forceinline__ void cg_alpha(double* s) { s[CG_ALPHA] = s[CG_PAP] != 0.0 ? s[CG_RZ] / s[CG_PAP] : 0.0; }
 // beta = rz_new / rz; rz = rz_new
-__global__ void k_cg_beta(double* s) { s[CG_BETA] = s[CG_RZ] != 0.0 ? s[CG_RZ_NEW] / s[CG_RZ] : 0.0; s[CG_RZ] = s[CG_RZ_NEW]; }
+__device__ __forceinline__ void cg_beta(double* s) {
+    s[CG_BETA] = s[CG_RZ] != 0.0 ? s[CG_RZ_NEW] / s[CG_RZ] : 0.0;
+    s[CG_RZ] = s[CG_RZ_NEW];
+}
 
-// x += alpha p;  r -= alpha Ap;  partial[b] = sum r[i]^2 over the block's slice
-__global__ void k_cg_update(double* __restrict__ x, double* __restrict__ r, const double* __restrict__ p,
-                            const double* __restrict__ Ap, int64_t n, const double* __restrict__ s,
-                            double* __restrict__ partial) {
-    const double alpha = s[CG_ALPHA];
+// x += alpha p;  r -= alpha Ap;  returns the slice's sum of r[i]^2
+__device__ __forceinline__ double cg_update_slice(double* __restrict__ x, double* __restrict__ r,
+                                                  const double* __restrict__ p, const double* __restrict__ Ap,
+                                                  int64_t n, double alpha) {
     double acc = 0.0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
-         i += (int64_t)gridDim.x * blockDim.x) {
+    GRID_SLICE(i, n) {
         x[i] = fma(alpha, p[i], x[i]);
         const double ri = fma(-alpha, Ap[i], r[i]);
         r[i] = ri;
         acc = fma(ri, ri, acc);
     }
-    acc = block_sum(acc);
+    return acc;
+}
+
+// p = z + beta p   (first: p = z)
+__device__ __forceinline__ void cg_direction_slice(double* __restrict__ p, const double* __restrict__ z, int64_t n,
+                                                   double beta, int first) {
+    GRID_SLICE(i, n) p[i] = first ? z[i] : fma(beta, p[i], z[i]);
+}
+
+// y += a x
+__global__ void k_axpy(double* __restrict__ y, const double* __restrict__ x, int64_t n, double a) {
+    axpy_slice(y, x, n, a);
+}
+
+__global__ void k_cg_alpha(double* s) { cg_alpha(s); }
+__global__ void k_cg_beta(double* s) { cg_beta(s); }
+
+// x += alpha p;  r -= alpha Ap;  partial[b] = sum r[i]^2 over the block's slice
+__global__ void k_cg_update(double* __restrict__ x, double* __restrict__ r, const double* __restrict__ p,
+                            const double* __restrict__ Ap, int64_t n, const double* __restrict__ s,
+                            double* __restrict__ partial) {
+    const double acc = block_sum(cg_update_slice(x, r, p, Ap, n, s[CG_ALPHA]));
     if (threadIdx.x == 0) partial[blockIdx.x] = acc;
 }
 
 // p = z + beta p   (first = 1: p = z)
 __global__ void k_cg_direction(double* __restrict__ p, const double* __restrict__ z, int64_t n,
                                const double* __restrict__ s, int first) {
-    const double beta = first ? 0.0 : s[CG_BETA];
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
-         i += (int64_t)gridDim.x * blockDim.x)
-        p[i] = first ? z[i] : fma(beta, p[i], z[i]);
+    cg_direction_slice(p, z, n, first ? 0.0 : s[CG_BETA], first);
 }
 
 // second-stage partial sums for long partial arrays: out[b] = sum of a fixed grid-stride slice
 __global__ void k_sum_partial(const double* __restrict__ partial, int64_t np, double* __restrict__ out) {
-    double s = 0.0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < np;
-         i += (int64_t)gridDim.x * blockDim.x)
-        s += partial[i];
-    s = block_sum(s);
+    const double s = block_sum(sum_slice(partial, np));
     if (threadIdx.x == 0) out[blockIdx.x] = s;
 }
 
 // out[slot] = sqrt(sum partial[0..np))
 __global__ void k_reduce_final(const double* __restrict__ partial, int np, double* __restrict__ out,
                                int slot, int take_sqrt) {
-    double s = 0.0;
-    for (int i = threadIdx.x; i < np; i += blockDim.x) s += partial[i];
-    s = block_sum(s);
+    const double s = reduce_final_sum(partial, np);
     if (threadIdx.x == 0) out[slot] = take_sqrt ? sqrt(s) : s;
+}
+
+// ---- the same for up to MULTI_MAX_COLS columns in one launch (amg1d_dev_pcg_multi) --------------------
+// Column i of a launch is blockIdx.y (the scalar kernels: threadIdx.x); every ColVecs entry i is that column's
+// vector, partial array or scalar window.  Per column the grid, the slices and the partial layout are those of the
+// single-column kernel, so the column's results are bit-identical to it.
+#define MULTI_MAX_COLS 8
+
+struct ColVecs {
+    double* v[MULTI_MAX_COLS];
+};
+
+__global__ void k_sqdiff_partial_multi(const __grid_constant__ ColVecs a, int64_t n, const __grid_constant__ ColVecs partial) {
+    const int c = blockIdx.y;
+    const double s = block_sum(sqdiff_slice(a.v[c], nullptr, n));
+    if (threadIdx.x == 0) partial.v[c][blockIdx.x] = s;
+}
+
+__global__ void k_dot_partial_multi(const __grid_constant__ ColVecs a, const __grid_constant__ ColVecs b, int64_t n,
+                                    const __grid_constant__ ColVecs partial) {
+    const int c = blockIdx.y;
+    const double s = block_sum(dot_slice(a.v[c], b.v[c], n));
+    if (threadIdx.x == 0) partial.v[c][blockIdx.x] = s;
+}
+
+__global__ void k_axpy_multi(const __grid_constant__ ColVecs y, const __grid_constant__ ColVecs x, int64_t n, double a) {
+    axpy_slice(y.v[blockIdx.y], x.v[blockIdx.y], n, a);
+}
+
+__global__ void k_cg_alpha_multi(const __grid_constant__ ColVecs s) { cg_alpha(s.v[threadIdx.x]); }
+__global__ void k_cg_beta_multi(const __grid_constant__ ColVecs s) { cg_beta(s.v[threadIdx.x]); }
+
+__global__ void k_cg_update_multi(const __grid_constant__ ColVecs x, const __grid_constant__ ColVecs r,
+                                  const __grid_constant__ ColVecs p, const __grid_constant__ ColVecs Ap, int64_t n,
+                                  const __grid_constant__ ColVecs s, const __grid_constant__ ColVecs partial) {
+    const int c = blockIdx.y;
+    const double acc = block_sum(cg_update_slice(x.v[c], r.v[c], p.v[c], Ap.v[c], n, s.v[c][CG_ALPHA]));
+    if (threadIdx.x == 0) partial.v[c][blockIdx.x] = acc;
+}
+
+__global__ void k_cg_direction_multi(const __grid_constant__ ColVecs p, const __grid_constant__ ColVecs z, int64_t n,
+                                     const __grid_constant__ ColVecs s, int first) {
+    const int c = blockIdx.y;
+    cg_direction_slice(p.v[c], z.v[c], n, first ? 0.0 : s.v[c][CG_BETA], first);
+}
+
+__global__ void k_sum_partial_multi(const __grid_constant__ ColVecs partial, int64_t np,
+                                    const __grid_constant__ ColVecs out) {
+    const int c = blockIdx.y;
+    const double s = block_sum(sum_slice(partial.v[c], np));
+    if (threadIdx.x == 0) out.v[c][blockIdx.x] = s;
+}
+
+// out.v[i][slot] = sum (or its square root) of partial.v[i][0..np)
+__global__ void k_reduce_final_multi(const __grid_constant__ ColVecs partial, int np, const __grid_constant__ ColVecs out,
+                                     int slot, int take_sqrt) {
+    const int c = blockIdx.y;
+    const double s = reduce_final_sum(partial.v[c], np);
+    if (threadIdx.x == 0) out.v[c][slot] = take_sqrt ? sqrt(s) : s;
 }
 
 // ---- set-up helpers -----------------------------------------------------------------------------

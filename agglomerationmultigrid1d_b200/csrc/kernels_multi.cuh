@@ -8,6 +8,8 @@
 //                                   f_up (down_leg / up_leg, kernels_fused.cuh) once per column
 //  f_down_multi_dv / f_up_multi_dv  the same with the inverse kept in registers (load_blocks_dv): the form of the levels
 //                                   whose single-column legs are f_*_dv or the pipelined f_*_pp
+//  f_matvec_dot_multi               y_c = A x_c and the per-block partial sums of x_c . y_c of every column (the A p,
+//                                   p . A p step of amg1d_dev_pcg_multi): f_matvec_dot with the operator read once
 //
 // Per column the arithmetic, its order and the window partition (fused_window) are those of the single-column leg, so
 // every column's iterate, coarse right-hand side and per-window ||b - A x||^2 partial sums are bit-identical to a
@@ -18,11 +20,10 @@
 // coarse block size MC, ratio R; rec: the inverse is not read):
 //   f_down_multi   8 (Kop / k + 3 M + MC / R)     against 8 (Kop + 3 M + MC / R) for f_down
 //   f_up_multi     8 (Kop / k + 3 M + MC / R)     against 8 (Kop + 3 M + MC / R) for f_up
-// (T level 0: Kop = 24, M = 4: 38 -> 24 / k + 14 doubles per element and column.)
+//   f_matvec_dot_multi  8 (Kop' / k + 2 M)          against 8 (Kop' + 2 M) for f_matvec_dot (Kop' = Kop without Dinv)
+// (T level 0: Kop = 24, M = 4: 38 -> 24 / k + 14 doubles per element and column; matvec: Kop' = 24, 32 -> 24 / k + 8.)
 #pragma once
 #include "kernels_fused.cuh"
-
-#define MULTI_MAX_COLS 8
 
 // Per-column vectors of one multi-column leg (device pointers at element 0 of the level).
 struct MultiCols {
@@ -221,5 +222,80 @@ inline int fused_up_multi(const MatDesc& d, int mc, const TransferMap& tm, int n
         FUSED_COMBOS(X)
 #undef X
         default: return FUSED_NA;
+    }
+}
+
+// ---- y = A x with x . y for every column (the matvec of amg1d_dev_pcg_multi) ---------------------------------------
+struct MatvecCols {
+    const double* x[MULTI_MAX_COLS];
+    double* y[MULTI_MAX_COLS];
+    double* partial[MULTI_MAX_COLS];   // per-block x . y partial sums of the column, or nullptr
+};
+
+// Operators of at most this many doubles per element (A_lo, A_di, A_up: every 1 x 1 .. 4 x 4 class, 5 x 5 .. 7 x 7
+// compressed) stay in registers across the column loop; larger ones are re-read from the element tile per column,
+// columns after the first finding it in L1 / L2 (a register copy of a 9 x 9 dense operator would be 243 doubles).
+template <int M, int ST>
+struct MatvecOpInRegs { static constexpr bool value = 2 * OpShape<M, ST>::NO + M * M <= 64; };
+
+// Grid and one element per thread as f_matvec_dot; per column the operator application is stream_Ax's FMA order
+// (reg_Ax is the same sequence on the register copy), so each column's y and partial sums are f_matvec_dot's bits.
+template <int M, int ST>
+__global__ void __launch_bounds__(256) f_matvec_dot_multi(const double* __restrict__ mat, int K, int ilo, int iup,
+                                                          const __grid_constant__ MatvecCols cols, int k, int64_t n) {
+    using S = OpShape<M, ST>;
+    constexpr bool REG = MatvecOpInRegs<M, ST>::value;
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool active = e < n;
+    const double* T = mat + (e >> 5) * (int64_t)K * AMG1D_TILE + (e & 31);
+    RegOp<M, ST> A;
+    if constexpr (REG) {
+        if (active) {
+#pragma unroll
+            for (int q = 0; q < S::NO; ++q) A.lo[q] = T[q * AMG1D_TILE];
+#pragma unroll
+            for (int q = 0; q < M * M; ++q) A.di[q] = T[(S::O_DI + q) * AMG1D_TILE];
+#pragma unroll
+            for (int q = 0; q < S::NO; ++q) A.up[q] = T[(S::O_UP + q) * AMG1D_TILE];
+        }
+    }
+#pragma unroll 1
+    for (int c = 0; c < k; ++c) {
+        if (c) __syncthreads();                  // block_sum's shared scratch is reused by the next column
+        double s = 0.0;
+        if (active) {
+            const double* x = cols.x[c];
+            double xl[M], xc[M], xr[M], yy[M];
+            load_vec<M>(x + e * M, xc);
+            load_neighbours<M, ST>(x, e, ilo, iup, xl, xr);
+            if constexpr (REG) reg_Ax<M, ST>(A, ilo, iup, xl, xc, xr, yy);
+            else stream_Ax<M, ST>(T, ilo, iup, xl, xc, xr, yy);
+            store_vec<M>(cols.y[c] + e * M, yy);
+#pragma unroll
+            for (int i = 0; i < M; ++i) s = fma(xc[i], yy[i], s);
+        }
+        if (cols.partial[c]) {
+            s = block_sum(s);
+            if (threadIdx.x == 0) cols.partial[c][blockIdx.x] = s;
+        }
+    }
+}
+
+// Exactly fused_matvec_dot's predicate and grid: where it returns false the caller runs op_matvec_dot per column.
+inline bool fused_matvec_dot_multi(const MatDesc& d, const double* mat, const MatvecCols& cols, int k, int64_t n,
+                                   int64_t partial_cap, int* nblocks, cudaStream_t st) {
+    const int64_t grid = (n + 255) / 256;
+    if (grid > partial_cap || !fast_tier_ok(d)) return false;
+    *nblocks = (int)grid;
+    switch (d.m * 4 + d.st) {
+#define Y(MM, SS)                                                                                                   \
+    case MM * 4 + SS:                                                                                               \
+        f_matvec_dot_multi<MM, SS><<<(unsigned)grid, 256, 0, st>>>(mat, d.K, d.ilo, d.iup, cols, k, n);             \
+        return true;
+#define X(MM) Y(MM, 0) Y(MM, 1) Y(MM, 2)
+        FUSED_FOR_M(X)
+#undef X
+#undef Y
+        default: return false;
     }
 }

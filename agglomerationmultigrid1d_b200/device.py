@@ -352,6 +352,16 @@ class DeviceHierarchy:
         iters = [int(it[c]) for c in range(k)]
         return iters, [res[c * maxiter:c * maxiter + iters[c]].copy() for c in range(k)]
 
+    def dev_pcg_multi(self, maxiter, tol, nPre=3, nPost=3, alpha=2.0 / 3.0):
+        """``pcg`` on every column of the set (each column bit-identical to ``dev_pcg`` on it alone); returns
+        (iters, [res per column]).  The solutions stay on the device; the right-hand sides are consumed."""
+        k = self.info("multi_columns")
+        res = np.zeros(max(maxiter, 1) * max(k, 1))
+        it = (C.c_int * max(k, 1))()
+        self._ck(self._lib.amg1d_dev_pcg_multi(self._h, maxiter, tol, nPre, nPost, alpha, it, capi.dptr(res)))
+        iters = [int(it[c]) for c in range(k)]
+        return iters, [res[c * maxiter:c * maxiter + iters[c]].copy() for c in range(k)]
+
     def dev_get_solutions(self):
         k = self.info("multi_columns")
         X = np.zeros((self.n_dof[0], max(k, 1)), order="F")

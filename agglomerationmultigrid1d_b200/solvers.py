@@ -7,6 +7,7 @@ libamg1d.so (the GPU).  There is no CPU implementation behind them.
     ldiv(H, b) -> b overwritten / ldiv(y, H, b) -> y overwritten            src/solvers.jl:63-92
         (b, y may be n_dof x k matrices: the columns share V-cycles, up to 8 at a time)
     pcg(H, x0, b, maxiter, tol) -> (x, iter, res)      CG with ldiv! as preconditioner (the hook's purpose)
+        (x0, b may be n_dof x k matrices: every column its own CG, up to 8 columns sharing V-cycles)
     multigrid(H, x0, b, maxiter, tol) -> (x, iter, res, err)                src/solvers.jl:116-139
     iterative_smoother_solve(A, smoother, x0, b; maxiter, tol, alpha)       src/solvers.jl:189-213
     apply_smoother(S, B; alpha) -> alpha * S^-1 B                           src/smoother.jl:52-81
@@ -62,8 +63,25 @@ def pcg(H, x0, b, maxiter, tol, nPre=3, nPost=3, alpha=2.0 / 3.0):
     """Conjugate gradients preconditioned with ``ldiv!(z, H, r)`` - the use the reference's ``ldiv!``
     methods are written for (src/solvers.jl:63-92: MeshHierarchy as the ``Pl`` of a Krylov solver); the
     reference itself ships no driver.  Returns (x, iter, res) with res[i] = ||r_i||_2 and the stop rule of
-    ``multigrid`` (res < tol ||b||)."""
-    return _device_of(H).pcg(x0, b, maxiter, tol, nPre=nPre, nPost=nPost, alpha=alpha)
+    ``multigrid`` (res < tol ||b||).  A 2-D b (n_dof x k, any k; x0 of the same shape) runs every column as
+    the 1-D call would, up to 8 columns at a time through the multi-column set, and returns (X, iters, res) with
+    iters a list and res a list of per-column histories."""
+    dev = _device_of(H)
+    if np.ndim(b) == 2:
+        B = np.asarray(b, dtype=np.float64)
+        X0 = np.asarray(x0, dtype=np.float64)
+        if X0.shape != B.shape:
+            raise ValueError(f"DimensionMismatch: x0 {X0.shape} vs b {B.shape}")
+        X = np.empty(B.shape, order="F")
+        iters, res = [], []
+        for c0 in range(0, B.shape[1], MAX_COLS):
+            dev.dev_set_problems(X0[:, c0:c0 + MAX_COLS], B[:, c0:c0 + MAX_COLS])
+            it, r = dev.dev_pcg_multi(maxiter, tol, nPre=nPre, nPost=nPost, alpha=alpha)
+            X[:, c0:c0 + MAX_COLS] = dev.dev_get_solutions()
+            iters += it
+            res += r
+        return X, iters, res
+    return dev.pcg(x0, b, maxiter, tol, nPre=nPre, nPost=nPost, alpha=alpha)
 
 
 def multigrid(H, x0, b, maxiter, tol, u_exact=None, with_error=True):

@@ -283,6 +283,18 @@ int amg1d_dev_residual_norms(amg1d_t* h, double* res);             /* k values |
  * leaves the set of cycled columns, so its iterate, iters[c] and res history equal amg1d_dev_solve on it alone. */
 int amg1d_dev_solve_multi(amg1d_t* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters,
                           double* res);
+/* amg1d_dev_pcg on every column of the multi-column set: iters (k ints), res (maxiter x k, column-major).
+ * Initial guess = the column's resident iterate; the solution becomes it; the column's right-hand side is consumed
+ * (it becomes the CG residual).  Every column's iters[c], res history and solution are bit-identical to
+ * amg1d_dev_pcg on it alone; a column that meets its stop rule (or whose residual turns non-finite) leaves the set of
+ * cycled columns, one with b = 0 or an x0 that already solves it never enters it.  AMG1D_ERR_ARG for a non-finite
+ * column before the first iteration, and after the others finished for a column that broke down (the message names
+ * the column).  Afterwards amg1d_dev_vcycle_multi / _residual_norms / _solve_multi / _pcg_multi return
+ * AMG1D_ERR_STATE until a set is installed again; amg1d_dev_get_solutions returns the solutions.  The per-column CG
+ * vectors (three level-0 vectors) are allocated at the first call and grown with k.  The product A p reads level
+ * 0's operator once for all columns, and the CG updates and reductions run one launch for all columns. */
+int amg1d_dev_pcg_multi(amg1d_t* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters,
+                        double* res);
 int amg1d_dev_get_solutions(amg1d_t* h, double* X);                /* device -> host, n_dof_host x k */
 
 int amg1d_synchronize(amg1d_t* h);
@@ -338,6 +350,9 @@ int64_t amg1d_get_info(amg1d_t* h, const char* key); /* "kernel_launches", "laun
                                                         "multi_legs:<level>" (1 = the multi-column
                                                         cycle reads the level's operator once for all
                                                         columns), "multi_launches_per_cycle",
+                                                        "multi_pcg_launches_per_iteration" (launches
+                                                        of the last amg1d_dev_pcg_multi iteration
+                                                        outside its V-cycle),
                                                         the option keys,
                                                         ... (-1: unknown key) */
 

@@ -225,6 +225,14 @@ function multigrid_resident_multi(D::DeviceHierarchy, maxiter::Integer, tol::Abs
         D.handle, maxiter, tol, 3, 3, 2.0 / 3.0, it, res))
     return Int.(it), [res[1:it[c], c] for c in 1:k]
 end
+# pcg on every column of the set; the right-hand sides are consumed, the solutions stay on the device (dev_solutions)
+function pcg_resident_multi(D::DeviceHierarchy, maxiter::Integer, tol::AbstractFloat)
+    k = get_info(D, "multi_columns"); res = zeros(maxiter, k); it = zeros(Cint, k)
+    amg1d_check(D.handle, ccall((:amg1d_dev_pcg_multi, libamg1d), Cint,
+        (Ptr{Cvoid}, Cint, Float64, Cint, Cint, Float64, Ptr{Cint}, Ptr{Float64}),
+        D.handle, maxiter, tol, 3, 3, 2.0 / 3.0, it, res))
+    return Int.(it), [res[1:it[c], c] for c in 1:k]
+end
 dev_solutions(D::DeviceHierarchy) = (X = Matrix{Float64}(undef, D.nDof[1], get_info(D, "multi_columns"));
     amg1d_check(D.handle, ccall((:amg1d_dev_get_solutions, libamg1d), Cint, (Ptr{Cvoid}, Ptr{Float64}), D.handle, X)); X)
 
@@ -238,6 +246,20 @@ function ldiv!(Y::AbstractMatrix, D::DeviceHierarchy, B::AbstractMatrix)
         Y[:, cols] = dev_solutions(D)
     end
     return
+end
+
+# pcg(D, X0, B, ...): every column as pcg(D, x0, b, ...), up to AMG1D_MAX_COLS columns sharing each V-cycle
+function pcg(D::DeviceHierarchy, X0::AbstractMatrix, B::AbstractMatrix, maxiter::Integer, tol::AbstractFloat)
+    size(X0) == size(B) || throw(DimensionMismatch("X0 $(size(X0)) vs B $(size(B))"))
+    X = similar(B, Float64); iters = Int[]; res = Vector{Vector{Float64}}()
+    for c0 in 1:AMG1D_MAX_COLS:size(B, 2)
+        cols = c0:min(c0 + AMG1D_MAX_COLS - 1, size(B, 2))
+        dev_set_problems!(D, X0[:, cols], B[:, cols])
+        it, r = pcg_resident_multi(D, maxiter, tol)
+        X[:, cols] = dev_solutions(D)
+        append!(iters, it); append!(res, r)
+    end
+    return X, iters, res
 end
 
 function apply_smoother(D::DeviceHierarchy, level::Integer, B::AbstractVecOrMat; alpha::Float64 = 1.0)
