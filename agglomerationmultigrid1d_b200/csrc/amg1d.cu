@@ -85,8 +85,6 @@ struct Level {
     int64_t n_host = 0;  // reference vector length
     double* mat = nullptr;
     int64_t* perm = nullptr;  // device, n*m entries, or null
-    DVec x[2], b;
-    int cur = 0;
     // host copy of the blocks, kept only for small levels (coarsest-level factorisation)
     std::vector<double> h_lo, h_di, h_up;
     int64_t mat_bytes = 0;
@@ -116,6 +114,26 @@ struct Transfer {
     int64_t cover_extra = 0; // sharded: ghost elements right of the slab that own coarse elements of this rank
 };
 
+// One problem on the hierarchy: the resident problem, or one column of the multi-column set.  Every operation that
+// reads or writes a vector, a buffer parity, a scalar slot or the reduction scratch is given the column it works on.
+struct Column {
+    struct Vecs { DVec x[2], b; int cur = 0; };   // x[cur]: the current iterate, x[1 - cur]: the other ping-pong buffer
+    std::vector<Vecs> lv;          // [level]; a level this rank does not hold has none (column_alloc)
+    double* scal = nullptr;        // device scalars (slot 0: ||b - A x||, 1: error, 2: ||b||, CG_* slots of the PCG)
+    double* partial = nullptr;     // reduction scratch: partial_cap first-stage partial sums + 256 second-stage ones
+    struct { DVec x, p, ap; } cg;  // level 0: CG solution, search direction, A p - allocated at the first CG call
+};
+
+// An instantiated V-cycle graph, keyed by the cycle parameters and the active columns (the resident cycle: mask 1)
+struct GraphEntry {
+    cudaGraphExec_t exec = nullptr;
+    int pre = -1, post = -1, norm = -1, zero0 = -1;
+    double alpha = 0.0;
+    unsigned mask = 0;
+    int64_t launches = 0;
+    uint64_t stamp = 0;
+};
+
 }  // namespace
 
 struct amg1d {
@@ -131,13 +149,12 @@ struct amg1d {
     DVec scratch;          // residual scratch, max level size
     double* stage = nullptr;  // host-ordered staging for permuted levels
     int64_t stage_len = 0;
-    double* partial = nullptr;
     int64_t partial_cap = 0;
-    bool norm_valid = false;   // d_scal[0] holds ||b - A x|| of the current level-0 iterate
+    Column res;                // the resident problem (its 64 device scalars are its own allocation)
+    bool norm_valid = false;   // res.scal[0] holds ||b - A x|| of the current level-0 iterate
     bool dev_problem = true;   // level 0's b / x still hold the device-resident problem (amg1d_dev_set_problem);
                                // cleared by the calls that stage through them (level-0 residual / smoother
                                // solve, amg1d_pcg) - the amg1d_dev_* calls then refuse to run on stale data
-    double* d_scal = nullptr;  // device scalars
     double* h_scal = nullptr;  // pinned host scalars
     double* coarse_fac = nullptr;
     // options
@@ -165,25 +182,15 @@ struct amg1d {
     int tail_start = -1;
     TailLevel* d_tail = nullptr;
     TailPlan tail_plan_ = {};
-    std::vector<TailLevel> tail_host;   // host copy of d_tail (the multi-column cycle patches in its columns' vectors)
+    std::vector<TailLevel> tail_host;   // d_tail without the vectors, which fill_tail patches in per column
     uint64_t tail_gen = 0;              // bumped by every build_tail
-    // graph cache: a few instantiated V-cycle graphs keyed by (nPre, nPost, alpha, norm, zero guess)
-    struct GraphEntry {
-        cudaGraphExec_t exec = nullptr;
-        int pre = -1, post = -1, norm = -1, zero0 = -1;
-        double alpha = 0.0;
-        int64_t launches = 0;
-        uint64_t stamp = 0;
-    };
-    GraphEntry graphs[4];
+    GraphEntry graphs[4];               // graph cache of the resident problem's V-cycle
     uint64_t graph_clock = 0;
     int64_t launches_per_cycle = 0;
     // block-cyclic-reduction direct solvers: coarsest level (when it has more than AMG1D_BCR_MIN
     // elements) and, built on demand, any level asked for through amg1d_direct_solve
     BcrSolver coarse_bcr;
     std::vector<BcrSolver> direct;
-    // conjugate gradients (amg1d_pcg): solution, search direction, A p - allocated at the first call
-    DVec cg_x, cg_p, cg_ap;
     int64_t launch_counter = 0;
     int64_t device_bytes = 0;
     // per-kernel event profiling (option "profile"): one (start, stop) pair per launch of a leg
@@ -223,25 +230,19 @@ struct amg1d {
         struct Nb { int64_t off[3] = {0, 0, 0}; int64_t n = 0; };   // byte offsets of x[0].p, x[1].p, b.p; owned n
         std::vector<Nb> nb[2];                       // per level, for the left / right neighbour
     } p2p;
-    // multi-column resident problems (amg1d_dev_set_problems ...): per column the three vectors of every level, kept
-    // apart from the single-column resident problem in L[l].x / L[l].b
+    // multi-column resident problems (amg1d_dev_set_problems ...): columns of their own, apart from the resident problem
     struct Multi {
-        struct ColLevel { DVec x[2], b; int cur = 0; };
-        std::vector<std::vector<ColLevel>> col;    // [column][level], grown on demand, never shrunk
-        std::vector<double*> partial;              // per column: ||b - A x||^2 partial sums (partial_cap + 256)
+        std::vector<Column> col;                   // grown on demand, never shrunk
         int k = 0;                                 // columns of the current set (0: none)
-        double* d_scal = nullptr;                  // MULTI_MAX_COLS x MULTI_SLOTS device scalars (slots as d_scal)
+        double* d_scal = nullptr;                  // MULTI_MAX_COLS x MULTI_SLOTS device scalars: col[c].scal is window c
         double* h_scal = nullptr;                  // pinned host copy
         TailLevel* d_tail = nullptr;               // MULTI_MAX_COLS x TAIL_MAXL descriptors of the single-CTA tail
         uint64_t tail_synced = ~0ull;              // tail_gen that d_tail was filled for
         bool norm_valid = false;                   // d_scal slot 0 of every column holds ||b - A x|| of its iterate
         bool rhs_consumed = false;                 // amg1d_dev_pcg_multi turned the right-hand sides into CG residuals
         int64_t launches_per_cycle = 0;
-        struct CgCol { DVec x, p, ap; };           // per column: CG solution, search direction, A p on level 0
-        std::vector<CgCol> cg;                     // grown by amg1d_dev_pcg_multi only
         int64_t pcg_launches = 0;                  // launches of the last PCG iteration outside the V-cycle
-        struct Graph { GraphEntry g; unsigned mask = 0; };   // keyed as graphs[] plus the active-column set
-        Graph graphs[4];
+        GraphEntry graphs[4];
     } multi;
 };
 
@@ -304,6 +305,51 @@ int vec_from_arena(amg1d* h, DVec& v, int64_t n, int m) {
     v.in_arena = true;
     h->p2p.used += bytes;
     return AMG1D_OK;
+}
+
+int64_t vec_bytes(const DVec& v) { return (PAD_FRONT + v.len + PAD_BACK) * 8; }
+
+void vec_release(amg1d* h, DVec& v) {
+    if (v.raw && !v.in_arena) h->device_bytes -= vec_bytes(v);
+    vec_free(v);
+}
+
+// everything column_alloc gave col (not its scalars, which belong to their owner)
+void column_free(amg1d* h, Column& col) {
+    for (auto& v : col.lv) { vec_release(h, v.x[0]); vec_release(h, v.x[1]); vec_release(h, v.b); }
+    col.lv.clear();
+    if (col.partial) { cudaFree(col.partial); h->device_bytes -= (h->partial_cap + 256) * 8; col.partial = nullptr; }
+    vec_release(h, col.cg.x); vec_release(h, col.cg.p); vec_release(h, col.cg.ap);
+}
+
+// What col still lacks: its vectors on every level this rank holds, with its reduction scratch, and with cg its level-0
+// CG vectors.  Vectors of sharded levels come from the peer-mapped arena (in the order x[0], b, x[1] its neighbours
+// expect); a proxy level holds no x[1].  A failure releases what this call took and clears the sticky CUDA error.
+int column_alloc(amg1d* h, Column& col, bool cg) {
+    const bool levels = col.lv.empty();
+    int rc = AMG1D_OK;
+    if (levels) {
+        col.lv.resize((size_t)h->n_levels);
+        for (int l = 0; l < h->n_levels && rc == AMG1D_OK; ++l) {
+            const Level& lv = h->L[l];
+            Column::Vecs& v = col.lv[(size_t)l];
+            if (!lv.present && !lv.proxy) continue;
+            const bool arena = lv.sharded && h->p2p.arena;
+            for (DVec* d : {&v.x[0], &v.b, &v.x[1]})
+                if (rc == AMG1D_OK && (d != &v.x[1] || lv.present))
+                    rc = arena ? vec_from_arena(h, *d, lv.n, lv.m) : vec_alloc(h, *d, lv.n, lv.m);
+        }
+        if (rc == AMG1D_OK) rc = dev_alloc(h, (void**)&col.partial, (h->partial_cap + 256) * 8);
+    }
+    if (rc == AMG1D_OK && cg && !col.cg.x.raw)
+        for (DVec* d : {&col.cg.x, &col.cg.p, &col.cg.ap})
+            if (rc == AMG1D_OK) rc = vec_alloc(h, *d, h->L[0].n, h->L[0].m);
+    if (rc != AMG1D_OK) {
+        if (levels) column_free(h, col);
+        else { vec_release(h, col.cg.x); vec_release(h, col.cg.p); vec_release(h, col.cg.ap); }
+        cudaGetLastError();                      // an out-of-memory status must not surface at the next launch check
+    }
+    return rc;
 }
 
 inline dim3 gblock(int m) {
@@ -488,15 +534,16 @@ int op_halo(amg1d* h, double* v, int64_t n, int m, double* v2 = nullptr, int64_t
 }
 
 // rank r's slab of the gather level's right-hand side -> rank 0 (which owns the whole level)
-int op_gather_rhs(amg1d* h, int g) {
+int op_gather_rhs(amg1d* h, Column& col, int g) {
     Level& lg = h->L[g];
+    double* b = col.lv[(size_t)g].b.p;
     NCK(g_nccl.GroupStart());
     if (h->rank == 0) {
         for (int r = 1; r < h->nranks; ++r)
-            NCK(g_nccl.Recv(lg.b.p + slab_start(lg.n_glob, h->nranks, r) * lg.m,
+            NCK(g_nccl.Recv(b + slab_start(lg.n_glob, h->nranks, r) * lg.m,
                             slab_size(lg.n_glob, h->nranks, r) * lg.m, ncclDouble, r, h->comm, h->stream));
     } else {
-        NCK(g_nccl.Send(lg.b.p, slab_size(lg.n_glob, h->nranks, h->rank) * lg.m, ncclDouble, 0, h->comm,
+        NCK(g_nccl.Send(b, slab_size(lg.n_glob, h->nranks, h->rank) * lg.m, ncclDouble, 0, h->comm,
                         h->stream));
     }
     NCK(g_nccl.GroupEnd());
@@ -505,12 +552,13 @@ int op_gather_rhs(amg1d* h, int g) {
 }
 
 // rank 0's solution of the gather level -> every rank's slab (with ghost elements)
-int op_scatter_sol(amg1d* h, int g) {
+int op_scatter_sol(amg1d* h, Column& col, int g) {
     Level& lg = h->L[g];
+    Column::Vecs& v = col.lv[(size_t)g];
     const int gd = h->ghost_depth;
     NCK(g_nccl.GroupStart());
     if (h->rank == 0) {
-        const double* x = lg.x[lg.cur].p;
+        const double* x = v.x[v.cur].p;
         for (int r = 1; r < h->nranks; ++r) {
             const int64_t e0 = slab_start(lg.n_glob, h->nranks, r) - gd;
             const int64_t e1 = slab_start(lg.n_glob, h->nranks, r) + slab_size(lg.n_glob, h->nranks, r) +
@@ -520,23 +568,25 @@ int op_scatter_sol(amg1d* h, int g) {
     } else {
         const int64_t cnt = (slab_size(lg.n_glob, h->nranks, h->rank) + gd +
                              (h->rank < h->nranks - 1 ? gd : 0)) * lg.m;
-        NCK(g_nccl.Recv(lg.x[0].p - (int64_t)gd * lg.m, cnt, ncclDouble, 0, h->comm, h->stream));
+        NCK(g_nccl.Recv(v.x[0].p - (int64_t)gd * lg.m, cnt, ncclDouble, 0, h->comm, h->stream));
     }
     NCK(g_nccl.GroupEnd());
     h->launch_counter++;
     return AMG1D_OK;
 }
 
-// d_scal[slot] currently holds a local SUM OF SQUARES: make it the global 2-norm
+// col.scal[slot] currently holds a local sum (of squares with take_sqrt): make it the global sum (2-norm)
 __global__ void k_sqrt_inplace(double* v, int slot) { v[slot] = sqrt(v[slot]); }
 int op_allreduce_max(amg1d* h, double* dptr, int count) {
     NCK(g_nccl.AllReduce(dptr, dptr, (size_t)count, ncclDouble, ncclMax, h->comm, h->stream));
     return AMG1D_OK;
 }
-int op_allreduce_norm(amg1d* h, int slot) {
-    NCK(g_nccl.AllReduce(h->d_scal + slot, h->d_scal + slot, 1, ncclDouble, ncclSum, h->comm, h->stream));
-    k_sqrt_inplace<<<1, 1, 0, h->stream>>>(h->d_scal, slot);
-    h->launch_counter += 2;
+int op_allreduce_norm(amg1d* h, Column& col, int slot, bool take_sqrt) {
+    NCK(g_nccl.AllReduce(col.scal + slot, col.scal + slot, 1, ncclDouble, ncclSum, h->comm, h->stream));
+    h->launch_counter++;
+    if (!take_sqrt) return AMG1D_OK;
+    k_sqrt_inplace<<<1, 1, 0, h->stream>>>(col.scal, slot);
+    h->launch_counter++;
     LAUNCH_CHECK();
     return AMG1D_OK;
 }
@@ -594,7 +644,7 @@ void p2p_close(amg1d* h) {
 }
 
 // exchange the arena handles and map both neighbours' arenas; every rank takes the same decision
-int p2p_connect(amg1d* h) {
+int p2p_connect(amg1d* h, Column& col) {
     amg1d::P2P& P = h->p2p;
     if (!P.arena) return AMG1D_OK;
     P2PXchg mine;
@@ -605,7 +655,8 @@ int p2p_connect(amg1d* h) {
         const Level& lv = h->L[l];
         if (!lv.sharded) continue;
         ++mine.n_sharded;
-        const DVec* v[3] = {&lv.x[0], &lv.x[1], &lv.b};
+        const Column::Vecs& cv = col.lv[(size_t)l];
+        const DVec* v[3] = {&cv.x[0], &cv.x[1], &cv.b};
         for (int k = 0; k < 3; ++k) {
             if (!v[k]->in_arena) mine.ok = 0;
             mine.off[l][k] = reinterpret_cast<const char*>(v[k]->p) - P.arena;
@@ -653,8 +704,9 @@ unsigned long long* p2p_my_flag(amg1d* h, int side, int ch) {
     return (nbr < 0 || nbr >= h->nranks) ? nullptr : h->p2p.flags + side * h->p2p.n_ch + ch;
 }
 
-// push the edges of level l's vector `vec` (0 / 1: x buffers, 2: b) - and optionally of level l2's vector vec2 - on channel ch
-int op_p2p_push(amg1d* h, int ch, int l, int vec, int l2 = -1, int vec2 = 0) {
+// push the edges of col's vector `vec` (0 / 1: x buffers, 2: b) on level l - and optionally of its vector vec2 on level
+// l2 - on channel ch
+int op_p2p_push(amg1d* h, Column& col, int ch, int l, int vec, int l2 = -1, int vec2 = 0) {
     amg1d::P2P& P = h->p2p;
     HaloPush a;
     memset(&a, 0, sizeof a);
@@ -663,7 +715,8 @@ int op_p2p_push(amg1d* h, int ch, int l, int vec, int l2 = -1, int vec2 = 0) {
     for (int p = 0; p < 2; ++p) {
         if (lv_[p] < 0) continue;
         Level& lv = h->L[lv_[p]];
-        const DVec& v = vc_[p] == 2 ? lv.b : lv.x[vc_[p]];
+        const Column::Vecs& cv = col.lv[(size_t)lv_[p]];
+        const DVec& v = vc_[p] == 2 ? cv.b : cv.x[vc_[p]];
         a.src[p] = v.p;
         a.n[p] = lv.n;
         a.m[p] = lv.m;
@@ -762,14 +815,14 @@ int op_p2p_wait_for(amg1d* h, const HaloLeg& hl) {
     return AMG1D_OK;
 }
 #else
-int op_p2p_push(amg1d* h, int, int, int, int = -1, int = 0) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
+int op_p2p_push(amg1d* h, Column&, int, int, int, int = -1, int = 0) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 int op_p2p_begin_cycle(amg1d* h) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 HaloLeg make_halo_leg(amg1d*, int, bool, int) { HaloLeg hl; memset(&hl, 0, sizeof hl); return hl; }
 int op_p2p_wait_for(amg1d* h, const HaloLeg&) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 int op_halo(amg1d* h, double*, int64_t, int, double* = nullptr, int64_t = 0, int = 0) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
-int op_gather_rhs(amg1d* h, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
-int op_scatter_sol(amg1d* h, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
-int op_allreduce_norm(amg1d* h, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
+int op_gather_rhs(amg1d* h, Column&, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
+int op_scatter_sol(amg1d* h, Column&, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
+int op_allreduce_norm(amg1d* h, Column&, int, bool) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 int op_allreduce_max(amg1d* h, double*, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 #endif
 
@@ -843,99 +896,79 @@ int op_coarse(amg1d* h, const double* b, double* x) {
     return AMG1D_OK;
 }
 
-// out slot <- || a - c ||_2 (c may be null)
-int op_norm(amg1d* h, const double* a, const double* c, int64_t n, int slot) {
+// col's slot <- || a - c ||_2 (c may be null)
+int op_norm(amg1d* h, Column& col, const double* a, const double* c, int64_t n, int slot) {
     int nb = (int)std::min<int64_t>(AMG1D_RED_BLOCKS, (n + AMG1D_RED_THREADS - 1) / AMG1D_RED_THREADS);
     if (nb < 1) nb = 1;
-    k_sqdiff_partial<<<nb, AMG1D_RED_THREADS, 0, h->stream>>>(a, c, n, h->partial);
-    k_reduce_final<<<1, AMG1D_RED_THREADS, 0, h->stream>>>(h->partial, nb, h->d_scal, slot,
+    k_sqdiff_partial<<<nb, AMG1D_RED_THREADS, 0, h->stream>>>(a, c, n, col.partial);
+    k_reduce_final<<<1, AMG1D_RED_THREADS, 0, h->stream>>>(col.partial, nb, col.scal, slot,
                                                            h->nranks > 1 ? 0 : 1);
     h->launch_counter += 2;
     LAUNCH_CHECK();
-    if (h->nranks > 1) RET(op_allreduce_norm(h, slot));
+    if (h->nranks > 1) RET(op_allreduce_norm(h, col, slot, true));
     return AMG1D_OK;
 }
 
-// d_scal[slot] = sqrt(sum partial[0..np)); long arrays go through a second stage of 256 partial sums
-int op_reduce_partials(amg1d* h, int64_t np, int slot) {
-    const double* src = h->partial;
+// col's slot <- sum col.partial[0..np), square-rooted with take_sqrt, summed over the ranks in the sharded case; long
+// arrays go through a second stage of 256 partial sums
+int op_reduce_partials(amg1d* h, Column& col, int64_t np, int slot, bool take_sqrt) {
+    const double* src = col.partial;
     if (np > 8192) {
-        double* stage2 = h->partial + h->partial_cap;   // 256 extra slots behind the first stage
-        k_sum_partial<<<256, AMG1D_RED_THREADS, 0, h->stream>>>(h->partial, np, stage2);
+        double* stage2 = col.partial + h->partial_cap;   // 256 extra slots behind the first stage
+        k_sum_partial<<<256, AMG1D_RED_THREADS, 0, h->stream>>>(col.partial, np, stage2);
         h->launch_counter++;
         src = stage2;
         np = 256;
     }
-    k_reduce_final<<<1, AMG1D_RED_THREADS, 0, h->stream>>>(src, (int)np, h->d_scal, slot,
-                                                           h->nranks > 1 ? 0 : 1);
+    k_reduce_final<<<1, AMG1D_RED_THREADS, 0, h->stream>>>(src, (int)np, col.scal, slot,
+                                                           take_sqrt && h->nranks == 1 ? 1 : 0);
     h->launch_counter++;
     LAUNCH_CHECK();
-    if (h->nranks > 1) RET(op_allreduce_norm(h, slot));
+    if (h->nranks > 1) RET(op_allreduce_norm(h, col, slot, take_sqrt));
     return AMG1D_OK;
 }
 
-// || b - A x ||_2 on level l into slot
-int op_resnorm(amg1d* h, int l, int slot) {
+// || b - A x ||_2 of col on level l into its slot
+int op_resnorm(amg1d* h, Column& col, int l, int slot) {
     Level& lv = h->L[l];
-    if (lv.sharded) RET(op_halo(h, lv.x[lv.cur].p, lv.n, lv.m));
+    Column::Vecs& v = col.lv[(size_t)l];
+    if (lv.sharded) RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m));
     if (h->opt_fused) {
         int nb = 0;
-        if (fused_resnorm(lv.md, lv.mat, lv.b.p, lv.x[lv.cur].p, lv.n, h->partial, h->partial_cap, &nb,
+        if (fused_resnorm(lv.md, lv.mat, v.b.p, v.x[v.cur].p, lv.n, col.partial, h->partial_cap, &nb,
                           h->stream)) {
             h->launch_counter++;
             LAUNCH_CHECK();
-            return op_reduce_partials(h, nb, slot);
+            return op_reduce_partials(h, col, nb, slot, true);
         }
     }
-    RET(op_apply(h, l, lv.b.p, lv.x[lv.cur].p, h->scratch.p, 1));
-    return op_norm(h, h->scratch.p, nullptr, lv.n * lv.m, slot);
+    RET(op_apply(h, l, v.b.p, v.x[v.cur].p, h->scratch.p, 1));
+    return op_norm(h, col, h->scratch.p, nullptr, lv.n * lv.m, slot);
 }
 
-// d_scal[slot] = sum partial[0..np) (no square root), summed over the ranks in the sharded case
-int op_sum_partials(amg1d* h, int64_t np, int slot) {
-    const double* src = h->partial;
-    if (np > 8192) {
-        double* stage2 = h->partial + h->partial_cap;
-        k_sum_partial<<<256, AMG1D_RED_THREADS, 0, h->stream>>>(h->partial, np, stage2);
-        h->launch_counter++;
-        src = stage2;
-        np = 256;
-    }
-    k_reduce_final<<<1, AMG1D_RED_THREADS, 0, h->stream>>>(src, (int)np, h->d_scal, slot, 0);
-    h->launch_counter++;
-    LAUNCH_CHECK();
-#ifdef AMG1D_WITH_NCCL
-    if (h->nranks > 1) {
-        NCK(g_nccl.AllReduce(h->d_scal + slot, h->d_scal + slot, 1, ncclDouble, ncclSum, h->comm, h->stream));
-        h->launch_counter++;
-    }
-#endif
-    return AMG1D_OK;
-}
-
-// slot <- a . c over the owned entries
-int op_dot(amg1d* h, const double* a, const double* c, int64_t n, int slot) {
+// col's slot <- a . c over the owned entries
+int op_dot(amg1d* h, Column& col, const double* a, const double* c, int64_t n, int slot) {
     int nb = (int)std::min<int64_t>(AMG1D_RED_BLOCKS, (n + AMG1D_RED_THREADS - 1) / AMG1D_RED_THREADS);
     if (nb < 1) nb = 1;
-    k_dot_partial<<<nb, AMG1D_RED_THREADS, 0, h->stream>>>(a, c, n, h->partial);
+    k_dot_partial<<<nb, AMG1D_RED_THREADS, 0, h->stream>>>(a, c, n, col.partial);
     h->launch_counter++;
     LAUNCH_CHECK();
-    return op_sum_partials(h, nb, slot);
+    return op_reduce_partials(h, col, nb, slot, false);
 }
 
-// y = A x on level l (x must carry valid ghost elements), slot <- x . y when slot >= 0
-int op_matvec_dot(amg1d* h, int l, double* x, double* y, int slot) {
+// y = A x on level l (x must carry valid ghost elements), col's slot <- x . y when slot >= 0
+int op_matvec_dot(amg1d* h, Column& col, int l, double* x, double* y, int slot) {
     Level& lv = h->L[l];
     if (lv.sharded) RET(op_halo(h, x, lv.n, lv.m));
     int nb = 0;
-    if (h->opt_fused && fused_matvec_dot(lv.md, lv.mat, x, y, lv.n, slot >= 0 ? h->partial : nullptr,
+    if (h->opt_fused && fused_matvec_dot(lv.md, lv.mat, x, y, lv.n, slot >= 0 ? col.partial : nullptr,
                                          h->partial_cap, &nb, h->stream)) {
         h->launch_counter++;
         LAUNCH_CHECK();
-        return slot >= 0 ? op_sum_partials(h, nb, slot) : AMG1D_OK;
+        return slot >= 0 ? op_reduce_partials(h, col, nb, slot, false) : AMG1D_OK;
     }
     RET(op_apply(h, l, nullptr, x, y, 0));
-    return slot >= 0 ? op_dot(h, x, y, lv.n * lv.m, slot) : AMG1D_OK;
+    return slot >= 0 ? op_dot(h, col, x, y, lv.n * lv.m, slot) : AMG1D_OK;
 }
 
 int prof_mark(amg1d* h, int level, int leg) {
@@ -950,39 +983,41 @@ int prof_mark(amg1d* h, int level, int leg) {
 
 // ---- the V-cycle (src/solvers.jl:19-50) ------------------------------------------------------------
 // Down leg of level l: nPre sweeps (zero guess on l > 0), residual, restriction into level l+1's rhs.
-int leg_down(amg1d* h, int l, int nPre, double alpha, bool zero0) {
+int leg_down(amg1d* h, Column& col, int l, int nPre, double alpha, bool zero0) {
     Level& lv = h->L[l];
     Transfer& t = h->T[l];
     Level& lc = h->L[l + 1];
+    Column::Vecs& v = col.lv[(size_t)l];
+    Column::Vecs& vc = col.lv[(size_t)l + 1];
     const bool zero = l > 0 || zero0;         // zero0: level 0 starts from a zero guess too (ldiv!, PCG)
-    if (zero) lv.cur = 0;
+    if (zero) v.cur = 0;
     RET(prof_mark(h, l, 0));
     // ghosts of the incoming iterate (peer-memory mode: they arrived with the last up leg's push, or with
     // amg1d_dev_set_problem's exchange)
-    if (lv.sharded && !zero && !h->p2p.on) RET(op_halo(h, lv.x[lv.cur].p, lv.n, lv.m));
+    if (lv.sharded && !zero && !h->p2p.on) RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m));
     // fused: nPre sweeps + residual + restriction in one pass over the operator
     if (h->opt_fused && t.fusable && !lv.smooth_tri) {
-        const int ob = zero ? 0 : 1 - lv.cur;
+        const int ob = zero ? 0 : 1 - v.cur;
         cudaError_t le = cudaSuccess;
         const bool p2p = h->p2p.on && lv.sharded;
         // peer-memory exchange done by the leg itself: wait for the rhs ghosts, push the pre-smoothed edges + coarse rhs
         const HaloLeg hl = p2p ? make_halo_leg(h, l, true, ob) : HaloLeg();
-        int fr = fused_down(lv.md, t.mc, make_map_closed(t), nPre, zero, lv.mat, make_pat(h, l), lv.b.p, lv.x[lv.cur].p,
-                            lv.x[ob].p, tp0(t), tp1(t), lc.b.p, lv.n, lv.n + (lv.gr ? t.cover_extra : 0),
+        int fr = fused_down(lv.md, t.mc, make_map_closed(t), nPre, zero, lv.mat, make_pat(h, l), v.b.p, v.x[v.cur].p,
+                            v.x[ob].p, tp0(t), tp1(t), vc.b.p, lv.n, lv.n + (lv.gr ? t.cover_extra : 0),
                             alpha, make_slab(h, l), h->stream, h->opt_pdl != 0, &le, leg_rec(h, lv, t.mc), hl);
         if (fr == FUSED_NA && h->opt_rows) {    // large blocks: one thread per block row; exchange by stand-alone kernels
             if (p2p) RET(op_p2p_wait_for(h, hl));
-            fr = rows_down(lv.md, t.mc, make_map_closed(t), nPre, zero, lv.mat, make_pat(h, l), lv.b.p, lv.x[lv.cur].p,
-                           lv.x[ob].p, tp0(t), tp1(t), lc.b.p, lv.n, lv.n + (lv.gr ? t.cover_extra : 0), alpha,
+            fr = rows_down(lv.md, t.mc, make_map_closed(t), nPre, zero, lv.mat, make_pat(h, l), v.b.p, v.x[v.cur].p,
+                           v.x[ob].p, tp0(t), tp1(t), vc.b.p, lv.n, lv.n + (lv.gr ? t.cover_extra : 0), alpha,
                            make_slab(h, l), h->opt_rows, rows_rpt(h, l), h->stream, h->opt_pdl != 0, &le);
             if (fr == FUSED_OK && p2p) {
-                if (lc.sharded) RET(op_p2p_push(h, 2 * l, l, ob, l + 1, 2));
-                else RET(op_p2p_push(h, 2 * l, l, ob));
+                if (lc.sharded) RET(op_p2p_push(h, col, 2 * l, l, ob, l + 1, 2));
+                else RET(op_p2p_push(h, col, 2 * l, l, ob));
             }
         }
         if (fr == FUSED_ERR) return fail(h, AMG1D_ERR_CUDA, "f_down launch failed on level %d: %s", l, cudaGetErrorString(le));
         if (fr == FUSED_OK) {
-            lv.cur = ob;
+            v.cur = ob;
             h->launch_counter++;
             LAUNCH_CHECK();
             RET(prof_mark(h, l, 0));
@@ -992,33 +1027,34 @@ int leg_down(amg1d* h, int l, int nPre, double alpha, bool zero0) {
     if (lv.sharded)
         return fail(h, AMG1D_ERR_UNSUPPORTED, "level %d: sharded levels need the fused kernels "
                     "(a block size / transfer with a fused leg, closed-form transfer, option fused = 1)", l);
-    if (zero && nPre == 0) CK(cudaMemsetAsync(lv.x[0].p, 0, (size_t)lv.x[0].len * 8, h->stream));
+    if (zero && nPre == 0) CK(cudaMemsetAsync(v.x[0].p, 0, (size_t)v.x[0].len * 8, h->stream));
     for (int s = 0; s < nPre; ++s) {
         if (zero && s == 0) {
-            RET(op_sweep(h, l, lv.b.p, lv.x[0].p, lv.x[0].p, alpha, 1));  // x = alpha Dinv b
+            RET(op_sweep(h, l, v.b.p, v.x[0].p, v.x[0].p, alpha, 1));  // x = alpha Dinv b
         } else {
-            RET(op_sweep(h, l, lv.b.p, lv.x[lv.cur].p, lv.x[1 - lv.cur].p, alpha, 0));
-            lv.cur = 1 - lv.cur;
+            RET(op_sweep(h, l, v.b.p, v.x[v.cur].p, v.x[1 - v.cur].p, alpha, 0));
+            v.cur = 1 - v.cur;
         }
     }
     if (h->opt_fused && t.single_parent_uniform &&
-        fused_residual_restrict(lv.md, t.mc, make_map_closed(t), lv.mat, lv.b.p, lv.x[lv.cur].p, t.P0,
-                                lc.b.p, lv.n, h->stream)) {
+        fused_residual_restrict(lv.md, t.mc, make_map_closed(t), lv.mat, v.b.p, v.x[v.cur].p, t.P0,
+                                vc.b.p, lv.n, h->stream)) {
         h->launch_counter++;
         LAUNCH_CHECK();
     } else {
-        RET(op_apply(h, l, lv.b.p, lv.x[lv.cur].p, h->scratch.p, 1));
-        RET(op_restrict(h, l, h->scratch.p, lc.b.p));
+        RET(op_apply(h, l, v.b.p, v.x[v.cur].p, h->scratch.p, 1));
+        RET(op_restrict(h, l, h->scratch.p, vc.b.p));
     }
     return prof_mark(h, l, 0);
 }
 
 // Up leg of level l: x += L x_c, nPost sweeps; optionally ||b - A x|| of the result (level 0).
-int leg_up(amg1d* h, int l, int nPost, double alpha, bool fuse_norm, bool* norm_done, bool* halo_pushed) {
+int leg_up(amg1d* h, Column& col, int l, int nPost, double alpha, bool fuse_norm, bool* norm_done, bool* halo_pushed) {
     *halo_pushed = false;
     Level& lv = h->L[l];
     Transfer& t = h->T[l];
-    Level& lc = h->L[l + 1];
+    Column::Vecs& v = col.lv[(size_t)l];
+    Column::Vecs& vc = col.lv[(size_t)l + 1];
     RET(prof_mark(h, l, 1));
     if (h->opt_fused && t.fusable && !lv.smooth_tri) {
         int nb = 0;
@@ -1026,29 +1062,29 @@ int leg_up(amg1d* h, int l, int nPost, double alpha, bool fuse_norm, bool* norm_
         const bool p2p = h->p2p.on && lv.sharded;
         // Level 0's edges are pushed from inside the kernel only if the leg writes buffer 0, where the next cycle
         // reads them (a zero-guess cycle ends in buffer 1 and is copied over: enqueue_vcycle pushes after that copy)
-        const int ob = 1 - lv.cur;
+        const int ob = 1 - v.cur;
         const bool push_inside = l > 0 || ob == 0;
         const HaloLeg hl = p2p ? make_halo_leg(h, l, false, push_inside ? ob : -1) : HaloLeg();
-        int fr = fused_up(lv.md, t.mc, make_map_closed(t), nPost, lv.mat, make_pat(h, l), lv.b.p, lv.x[lv.cur].p,
-                          lv.x[1 - lv.cur].p, tp0(t), tp1(t), lc.x[lc.cur].p, lv.n, alpha,
-                          fuse_norm ? h->partial : nullptr, h->partial_cap, &nb, make_slab(h, l),
+        int fr = fused_up(lv.md, t.mc, make_map_closed(t), nPost, lv.mat, make_pat(h, l), v.b.p, v.x[v.cur].p,
+                          v.x[1 - v.cur].p, tp0(t), tp1(t), vc.x[vc.cur].p, lv.n, alpha,
+                          fuse_norm ? col.partial : nullptr, h->partial_cap, &nb, make_slab(h, l),
                           h->stream, h->opt_pdl != 0, &le, leg_rec(h, lv, t.mc), hl);
         if (fr == FUSED_OK && p2p && push_inside) *halo_pushed = true;
         if (fr == FUSED_NA && h->opt_rows) {
             if (p2p) RET(op_p2p_wait_for(h, hl));
-            fr = rows_up(lv.md, t.mc, make_map_closed(t), nPost, lv.mat, make_pat(h, l), lv.b.p, lv.x[lv.cur].p,
-                         lv.x[1 - lv.cur].p, tp0(t), tp1(t), lc.x[lc.cur].p, lv.n, alpha,
-                         fuse_norm ? h->partial : nullptr, h->partial_cap, &nb, make_slab(h, l), h->opt_rows,
+            fr = rows_up(lv.md, t.mc, make_map_closed(t), nPost, lv.mat, make_pat(h, l), v.b.p, v.x[v.cur].p,
+                         v.x[1 - v.cur].p, tp0(t), tp1(t), vc.x[vc.cur].p, lv.n, alpha,
+                         fuse_norm ? col.partial : nullptr, h->partial_cap, &nb, make_slab(h, l), h->opt_rows,
                          rows_rpt(h, l), h->stream, h->opt_pdl != 0, &le);
         }
         if (fr == FUSED_ERR) return fail(h, AMG1D_ERR_CUDA, "f_up launch failed on level %d: %s", l, cudaGetErrorString(le));
         if (fr == FUSED_OK) {
-            lv.cur = 1 - lv.cur;
+            v.cur = 1 - v.cur;
             h->launch_counter++;
             LAUNCH_CHECK();
             RET(prof_mark(h, l, 1));
             if (fuse_norm) {
-                RET(op_reduce_partials(h, nb, 0));
+                RET(op_reduce_partials(h, col, nb, 0, true));
                 *norm_done = true;
             }
             return AMG1D_OK;
@@ -1056,15 +1092,15 @@ int leg_up(amg1d* h, int l, int nPost, double alpha, bool fuse_norm, bool* norm_
     }
     if (lv.sharded)
         return fail(h, AMG1D_ERR_UNSUPPORTED, "level %d: sharded levels need the fused kernels", l);
-    RET(op_prolong(h, l, lc.x[lc.cur].p, lv.x[lv.cur].p, 1));
+    RET(op_prolong(h, l, vc.x[vc.cur].p, v.x[v.cur].p, 1));
     for (int s = 0; s < nPost; ++s) {
-        RET(op_sweep(h, l, lv.b.p, lv.x[lv.cur].p, lv.x[1 - lv.cur].p, alpha, 0));
-        lv.cur = 1 - lv.cur;
+        RET(op_sweep(h, l, v.b.p, v.x[v.cur].p, v.x[1 - v.cur].p, alpha, 0));
+        v.cur = 1 - v.cur;
     }
     return prof_mark(h, l, 1);
 }
 
-int enqueue_vcycle(amg1d* h, int nPre, int nPost, double alpha, bool want_norm, bool zero0) {
+int enqueue_vcycle(amg1d* h, Column& col, int nPre, int nPost, double alpha, bool want_norm, bool zero0) {
     const int nl = h->n_levels;
     const int g = h->gather_level;          // -1 on a single GPU: every level is local
     bool norm_done = false;
@@ -1085,107 +1121,127 @@ int enqueue_vcycle(amg1d* h, int nPre, int nPost, double alpha, bool want_norm, 
     for (int l = 0; l < nl - 1 && l < ts; ++l) {
         Level& lv = h->L[l];
         if (!lv.present) break;                       // ranks > 0 stop at the gather level
-        RET(leg_down(h, l, nPre, alpha, zero0));
+        RET(leg_down(h, col, l, nPre, alpha, zero0));
         if (lv.sharded) {
             Level& lc = h->L[l + 1];
+            Column::Vecs& v = col.lv[(size_t)l];
             // ghosts of the pre-smoothed iterate (for the up leg) and of the coarse rhs, in one exchange
             if (p2p) {                    // the leg exchanged its edges itself (leg_down)
-                if (!lc.sharded) RET(op_gather_rhs(h, l + 1));        // slabs -> rank 0
-            } else if (lc.sharded) RET(op_halo(h, lv.x[lv.cur].p, lv.n, lv.m, lc.b.p, lc.n, lc.m));
+                if (!lc.sharded) RET(op_gather_rhs(h, col, l + 1));        // slabs -> rank 0
+            } else if (lc.sharded) RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m, col.lv[(size_t)l + 1].b.p, lc.n, lc.m));
             else {
-                RET(op_halo(h, lv.x[lv.cur].p, lv.n, lv.m));
-                RET(op_gather_rhs(h, l + 1));                         // slabs -> rank 0
+                RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m));
+                RET(op_gather_rhs(h, col, l + 1));                         // slabs -> rank 0
             }
         }
     }
     // ---- coarse tail in one CTA, or just the coarsest level: exact solve (src/solvers.jl:39) ----
     if (ts < nl) {
-        for (int l = ts; l < nl; ++l) h->L[l].cur = 0;
+        for (int l = ts; l < nl; ++l) col.lv[(size_t)l].cur = 0;
         cudaError_t te = tail_launch(h->L[ts].m, h->d_tail, nl - ts, h->coarse_fac, nPre, nPost, alpha,
                                      h->tail_plan_, h->stream, h->opt_pdl != 0);
         if (te != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "f_tail launch failed: %s", cudaGetErrorString(te));
         h->launch_counter++;
     } else if (h->L[nl - 1].present) {
-        Level& lv = h->L[nl - 1];
-        if (nl > 1 || zero0) lv.cur = 0;
-        RET(op_coarse(h, lv.b.p, lv.x[lv.cur].p));   // single level: x = A \ b overwrites x
+        Column::Vecs& v = col.lv[(size_t)nl - 1];
+        if (nl > 1 || zero0) v.cur = 0;
+        RET(op_coarse(h, v.b.p, v.x[v.cur].p));   // single level: x = A \ b overwrites x
     }
     // ---- up ----
     for (int l = std::min(nl - 2, ts - 1); l >= 0; --l) {
         Level& lv = h->L[l];
         Level& lc = h->L[l + 1];
+        Column::Vecs& v = col.lv[(size_t)l];
         if (!lv.present) continue;
-        if (lv.sharded && !lc.sharded) RET(op_scatter_sol(h, l + 1));   // rank 0 -> slabs (+ ghosts)
+        if (lv.sharded && !lc.sharded) RET(op_scatter_sol(h, col, l + 1));   // rank 0 -> slabs (+ ghosts)
         bool pushed = false;
-        RET(leg_up(h, l, nPost, alpha, want_norm && l == 0, &norm_done, &pushed));
+        RET(leg_up(h, col, l, nPost, alpha, want_norm && l == 0, &norm_done, &pushed));
         if (p2p && lv.sharded) {
             if (l == 0) u0_pushed = pushed;
-            else if (!pushed) RET(op_p2p_push(h, 2 * l + 1, l, lv.cur));   // (a leg without the fused exchange)
-        } else if (lv.sharded && l > 0) RET(op_halo(h, lv.x[lv.cur].p, lv.n, lv.m));   // for level l-1's prolongation
+            else if (!pushed) RET(op_p2p_push(h, col, 2 * l + 1, l, v.cur));   // (a leg without the fused exchange)
+        } else if (lv.sharded && l > 0) RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m));   // for level l-1's prolongation
     }
-    Level& l0 = h->L[0];
-    if (l0.cur != 0) {
-        CK(cudaMemcpyAsync(l0.x[0].p, l0.x[1].p, (size_t)l0.x[0].len * 8, cudaMemcpyDeviceToDevice,
+    Column::Vecs& v0 = col.lv[0];
+    if (v0.cur != 0) {
+        CK(cudaMemcpyAsync(v0.x[0].p, v0.x[1].p, (size_t)v0.x[0].len * 8, cudaMemcpyDeviceToDevice,
                            h->stream));
-        l0.cur = 0;
+        v0.cur = 0;
     }
     // level 0's corrected iterate: the incoming iterate of the next cycle, and the signal that this rank's up
     // leg no longer reads the ghosts which the neighbours' next down leg overwrites
-    if (p2p && l0.sharded && !u0_pushed) RET(op_p2p_push(h, 1, 0, 0));
-    if (want_norm && !norm_done) RET(op_resnorm(h, 0, 0));
+    if (p2p && h->L[0].sharded && !u0_pushed) RET(op_p2p_push(h, col, 1, 0, 0));
+    if (want_norm && !norm_done) RET(op_resnorm(h, col, 0, 0));
     return AMG1D_OK;
 }
 
-int run_vcycle(amg1d* h, int nPre, int nPost, double alpha, bool want_norm, bool zero0 = false) {
-    if (nPre < 0 || nPost < 0) return fail(h, AMG1D_ERR_ARG, "nPre and nPost must be >= 0");
+// One V-cycle through enqueue(): replayed from the cache's graph for key, which a miss captures and instantiates in the
+// least recently used entry; enqueued directly with option graph off or profile on.  *launches: kernels of one cycle.
+// parity0: the level-0 iterates of the cycled columns are in buffer 0, as a capture assumes.
+template <class Enqueue>
+int replay_vcycle(amg1d* h, GraphEntry (&cache)[4], const GraphEntry& key, bool parity0, int64_t* launches,
+                  Enqueue enqueue) {
     if (!h->opt_graph || h->opt_profile) {
         const int64_t c0 = h->launch_counter;
-        RET(enqueue_vcycle(h, nPre, nPost, alpha, want_norm, zero0));
-        h->launches_per_cycle = h->launch_counter - c0;
-        h->norm_valid = want_norm;
+        RET(enqueue());
+        *launches = h->launch_counter - c0;
         return AMG1D_OK;
     }
-    amg1d::GraphEntry* ge = nullptr;
-    for (auto& g : h->graphs)
-        if (g.exec && g.pre == nPre && g.post == nPost && g.alpha == alpha && g.norm == (int)want_norm &&
-            g.zero0 == (int)zero0)
+    GraphEntry* ge = nullptr;
+    for (auto& g : cache)
+        if (g.exec && g.mask == key.mask && g.pre == key.pre && g.post == key.post && g.alpha == key.alpha &&
+            g.norm == key.norm && g.zero0 == key.zero0)
             ge = &g;
     if (!ge) {
-        ge = &h->graphs[0];                               // free slot, else the least recently used one
-        for (auto& g : h->graphs) if (!g.exec) { ge = &g; break; } else if (g.stamp < ge->stamp) ge = &g;
+        ge = &cache[0];                                   // free slot, else the least recently used one
+        for (auto& g : cache) if (!g.exec) { ge = &g; break; } else if (g.stamp < ge->stamp) ge = &g;
         if (ge->exec) { cudaGraphExecDestroy(ge->exec); ge->exec = nullptr; }
-        if (h->L[0].cur != 0) return fail(h, AMG1D_ERR_STATE, "internal: level-0 buffer parity");
+        if (!parity0) return fail(h, AMG1D_ERR_STATE, "internal: level-0 buffer parity");
         cudaGraph_t g = nullptr;
         const int64_t c0 = h->launch_counter;
         CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
-        int rc = enqueue_vcycle(h, nPre, nPost, alpha, want_norm, zero0);
+        int rc = enqueue();
         cudaError_t ce = cudaStreamEndCapture(h->stream, &g);
         if (rc != AMG1D_OK) { if (g) cudaGraphDestroy(g); return rc; }
         if (ce != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(ce));
-        ge->launches = h->launch_counter - c0;
+        const int64_t n = h->launch_counter - c0;
         h->launch_counter = c0;
-        ce = cudaGraphInstantiate(&ge->exec, g, 0);
+        cudaGraphExec_t exec = nullptr;
+        ce = cudaGraphInstantiate(&exec, g, 0);
         cudaGraphDestroy(g);
-        if (ce != cudaSuccess) { ge->exec = nullptr; return fail(h, AMG1D_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(ce)); }
-        ge->pre = nPre; ge->post = nPost; ge->alpha = alpha; ge->norm = (int)want_norm; ge->zero0 = (int)zero0;
+        if (ce != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(ce));
+        *ge = key;
+        ge->exec = exec;
+        ge->launches = n;
     }
     ge->stamp = ++h->graph_clock;
     CK(cudaGraphLaunch(ge->exec, h->stream));
-    h->launches_per_cycle = ge->launches;
+    *launches = ge->launches;
     h->launch_counter += ge->launches;
+    return AMG1D_OK;
+}
+
+// V-cycle of the resident problem (col is h->res: the tail descriptors d_tail and the graph cache graphs[] hold its
+// vectors)
+int run_vcycle(amg1d* h, Column& col, int nPre, int nPost, double alpha, bool want_norm, bool zero0 = false) {
+    if (nPre < 0 || nPost < 0) return fail(h, AMG1D_ERR_ARG, "nPre and nPost must be >= 0");
+    GraphEntry key;
+    key.pre = nPre; key.post = nPost; key.alpha = alpha; key.norm = (int)want_norm; key.zero0 = (int)zero0; key.mask = 1;
+    RET(replay_vcycle(h, h->graphs, key, col.lv[0].cur == 0, &h->launches_per_cycle,
+                      [&] { return enqueue_vcycle(h, col, nPre, nPost, alpha, want_norm, zero0); }));
     h->norm_valid = want_norm;
     return AMG1D_OK;
 }
 
-void invalidate_graph(amg1d* h) {
-    for (auto& g : h->graphs) {
+void release_graphs(GraphEntry (&cache)[4]) {
+    for (auto& g : cache) {
         if (g.exec) cudaGraphExecDestroy(g.exec);
-        g = amg1d::GraphEntry();
+        g = GraphEntry();
     }
-    for (auto& g : h->multi.graphs) {
-        if (g.g.exec) cudaGraphExecDestroy(g.g.exec);
-        g = amg1d::Multi::Graph();
-    }
+}
+
+void invalidate_graph(amg1d* h) {
+    release_graphs(h->graphs);
+    release_graphs(h->multi.graphs);
     h->norm_valid = false;
     h->multi.norm_valid = false;
 }
@@ -1239,10 +1295,36 @@ int to_host(amg1d* h, int l, const double* dev, double* host) {
     return AMG1D_OK;
 }
 
-int read_scalars(amg1d* h, int count) {
-    CK(cudaMemcpyAsync(h->h_scal, h->d_scal, sizeof(double) * count, cudaMemcpyDeviceToHost, h->stream));
+int read_scalars(amg1d* h, Column& col, int count) {
+    CK(cudaMemcpyAsync(h->h_scal, col.scal, sizeof(double) * count, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return p2p_check(h);
+}
+
+// multigrid() (src/solvers.jl) on the resident problem: V-cycles until ||b - A x|| < tol ||b|| or maxiter; with d_exact
+// also err[i] = ||x - u_exact|| of every iterate (NaN without it)
+int multigrid_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters, double* res,
+                  double* err, const double* d_exact) {
+    Column::Vecs& v0 = h->res.lv[0];
+    int rc = op_norm(h, h->res, v0.b.p, nullptr, v0.b.len, 2);
+    int it = 0;
+    for (int i = 0; i < maxiter && rc == AMG1D_OK; ++i) {
+        rc = run_vcycle(h, h->res, nPre, nPost, alpha, true);
+        if (rc != AMG1D_OK) break;
+        if (d_exact) {
+            rc = op_norm(h, h->res, v0.x[v0.cur].p, d_exact, v0.x[0].len, 1);
+            if (rc != AMG1D_OK) break;
+        }
+        rc = read_scalars(h, h->res, 3);
+        if (rc != AMG1D_OK) break;
+        res[i] = h->h_scal[0];
+        if (err) err[i] = d_exact ? h->h_scal[1] : NAN;
+        it = i + 1;
+        if (res[i] < tol * h->h_scal[2]) break;
+    }
+    RET(rc);
+    *iters = it;
+    return AMG1D_OK;
 }
 
 // dense m x m inverse with partial pivoting (Gauss-Jordan), column-major; returns false if singular
@@ -1327,6 +1409,16 @@ int factor_coarsest(amg1d* h) {
     return AMG1D_OK;
 }
 
+// tail_host with col's x[0] and b: the descriptors f_tail reads for that column (tail_host covers [n_levels - size, n_levels))
+void fill_tail(const amg1d* h, const Column& col, TailLevel* out) {
+    const size_t ts = (size_t)h->n_levels - h->tail_host.size();
+    for (size_t i = 0; i < h->tail_host.size(); ++i) {
+        out[i] = h->tail_host[i];
+        out[i].x = col.lv[ts + i].x[0].p;
+        out[i].b = col.lv[ts + i].b.p;
+    }
+}
+
 // Single-CTA coarse tail (kernels_fused.cuh, f_tail): the longest suffix of levels [ts, n_levels) that
 // are unsharded, have at most min(coarse_cta_elems, TAIL_B) elements, share one block size, use block
 // smoothers and single-parent closed-form transfers, and whose operators + vectors fit the CTA's
@@ -1369,8 +1461,6 @@ int build_tail(amg1d* h) {
         d.md = lv.md;
         d.mat = lv.mat;
         d.n = lv.n;
-        d.x = lv.x[0].p;
-        d.b = lv.b.p;
         d.op_off = op_off; d.op_len = (int)(amg1d_tiles(lv.n) * lv.K * AMG1D_TILE);
         d.vec_off = vec_off;
         d.p_off = p_off; d.p_len = 0;
@@ -1384,9 +1474,10 @@ int build_tail(amg1d* h) {
     h->tail_plan_ = tail_plan(m, op_off, vec_off, p_off);
     cudaError_t e = tail_configure(m, (size_t)h->tail_plan_.total * 8);
     if (e != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "f_tail configuration failed: %s", cudaGetErrorString(e));
+    h->tail_host = tl;
+    fill_tail(h, h->res, tl.data());
     RET(dev_alloc(h, (void**)&h->d_tail, (int64_t)(tl.size() * sizeof(TailLevel))));
     CK(cudaMemcpy(h->d_tail, tl.data(), tl.size() * sizeof(TailLevel), cudaMemcpyHostToDevice));
-    h->tail_host = tl;
     h->tail_start = ts;
     return AMG1D_OK;
 }
@@ -1407,44 +1498,10 @@ int check_dev_problem(amg1d* h) {
 }
 
 // ---- multi-column resident problems (amg1d_dev_set_problems ...) ----------------------------------------------------
-// Column c of the set has its own x[0], x[1], b (and buffer parity) on every level.  Levels whose legs have a fused
-// multi-column kernel (kernels_multi.cuh) run one launch for all active columns; every other operation of the cycle -
-// the row-per-thread and generic tiers, the single-CTA tail, the coarse solve - runs its single-column code once per
-// column with that column's vectors swapped into the level (ColumnBind), so per column it is exactly the single-column
-// cycle.
-
-// Swaps column c's vectors, buffer parities, scalar slots and reduction scratch with the handle's own for as long as it
-// lives (the swap is its own inverse).
-struct ColumnBind {
-    amg1d* h;
-    int c;
-    double* scal;
-    double* part;
-    ColumnBind(amg1d* h_, int c_)
-        : h(h_), c(c_), scal(h_->multi.d_scal + c_ * MULTI_SLOTS), part(h_->multi.partial[(size_t)c_]) { swap(); }
-    ~ColumnBind() { swap(); }
-    void swap() {
-        auto& cl = h->multi.col[(size_t)c];
-        for (int l = 0; l < h->n_levels; ++l) {
-            Level& lv = h->L[l];
-            std::swap(lv.x[0], cl[(size_t)l].x[0]);
-            std::swap(lv.x[1], cl[(size_t)l].x[1]);
-            std::swap(lv.b, cl[(size_t)l].b);
-            std::swap(lv.cur, cl[(size_t)l].cur);
-        }
-        std::swap(h->d_scal, scal);
-        std::swap(h->partial, part);
-    }
-};
-
-int64_t vec_bytes(const DVec& v) { return (PAD_FRONT + v.len + PAD_BACK) * 8; }
-
-void multi_free_column(amg1d* h, std::vector<amg1d::Multi::ColLevel>& cl, double* partial) {
-    for (auto& v : cl)
-        for (DVec* d : {&v.x[0], &v.x[1], &v.b})
-            if (d->raw) { h->device_bytes -= vec_bytes(*d); vec_free(*d); }
-    if (partial) { cudaFree(partial); h->device_bytes -= (h->partial_cap + 256) * 8; }
-}
+// Each column of the set has its own vectors on every level.  Levels whose legs have a fused multi-column kernel
+// (kernels_multi.cuh) run one launch for all active columns; every other operation of the cycle - the row-per-thread and
+// generic tiers, the single-CTA tail, the coarse solve - runs its single-column code once per column, so per column it
+// is exactly the single-column cycle.
 
 // storage for k columns: the set only grows; a failed allocation releases what it took and leaves the rest as it was
 int multi_alloc(amg1d* h, int k) {
@@ -1453,41 +1510,22 @@ int multi_alloc(amg1d* h, int k) {
     if (!M.h_scal) CK(cudaMallocHost(&M.h_scal, MULTI_MAX_COLS * MULTI_SLOTS * 8));
     if (!M.d_tail) RET(dev_alloc(h, (void**)&M.d_tail, (int64_t)(MULTI_MAX_COLS * TAIL_MAXL * sizeof(TailLevel))));
     while ((int)M.col.size() < k) {
-        std::vector<amg1d::Multi::ColLevel> cl((size_t)h->n_levels);
-        double* part = nullptr;
-        int rc = AMG1D_OK;
-        for (int l = 0; l < h->n_levels && rc == AMG1D_OK; ++l) {
-            const Level& lv = h->L[l];
-            rc = vec_alloc(h, cl[(size_t)l].x[0], lv.n, lv.m);
-            if (rc == AMG1D_OK) rc = vec_alloc(h, cl[(size_t)l].x[1], lv.n, lv.m);
-            if (rc == AMG1D_OK) rc = vec_alloc(h, cl[(size_t)l].b, lv.n, lv.m);
-        }
-        if (rc == AMG1D_OK) rc = dev_alloc(h, (void**)&part, (h->partial_cap + 256) * 8);
-        if (rc != AMG1D_OK) {
-            multi_free_column(h, cl, part);
-            cudaGetLastError();                  // an out-of-memory status must not surface at the next launch check
-            return fail(h, rc, "column %d of the multi-column set: %s", (int)M.col.size(), h->err.c_str());
-        }
-        M.col.push_back(std::move(cl));
-        M.partial.push_back(part);
+        Column col;
+        col.scal = M.d_scal + M.col.size() * MULTI_SLOTS;
+        const int rc = column_alloc(h, col, false);
+        if (rc != AMG1D_OK) return fail(h, rc, "column %d of the multi-column set: %s", (int)M.col.size(), h->err.c_str());
+        M.col.push_back(std::move(col));
         M.tail_synced = ~0ull;
     }
     return AMG1D_OK;
 }
 
-// descriptors of the single-CTA tail for every column: the handle's own with the columns' vectors (before capture)
+// descriptors of the single-CTA tail for every column (before capture)
 int multi_sync_tail(amg1d* h) {
     amg1d::Multi& M = h->multi;
     if (h->tail_start <= 0 || M.tail_synced == h->tail_gen) return AMG1D_OK;
-    const int ts = h->tail_start;
     std::vector<TailLevel> all((size_t)MULTI_MAX_COLS * TAIL_MAXL);
-    for (size_t c = 0; c < M.col.size(); ++c)
-        for (size_t i = 0; i < h->tail_host.size(); ++i) {
-            TailLevel d = h->tail_host[i];
-            d.x = M.col[c][(size_t)ts + i].x[0].p;
-            d.b = M.col[c][(size_t)ts + i].b.p;
-            all[c * TAIL_MAXL + i] = d;
-        }
+    for (size_t c = 0; c < M.col.size(); ++c) fill_tail(h, M.col[c], &all[c * TAIL_MAXL]);
     CK(cudaMemcpyAsync(M.d_tail, all.data(), all.size() * sizeof(TailLevel), cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     M.tail_synced = h->tail_gen;
@@ -1518,14 +1556,14 @@ int leg_down_multi(amg1d* h, int l, const int* act, int na, int nPre, double alp
         MultiCols mc = {};
         int ob[MULTI_MAX_COLS];
         for (int i = 0; i < na; ++i) {
-            auto& cl = M.col[(size_t)act[i]];
-            auto& v = cl[(size_t)l];
+            Column& col = M.col[(size_t)act[i]];
+            Column::Vecs& v = col.lv[(size_t)l];
             if (zero) v.cur = 0;
             ob[i] = zero ? 0 : 1 - v.cur;
             mc.b[i] = v.b.p;
             mc.xin[i] = v.x[v.cur].p;
             mc.xout[i] = v.x[ob[i]].p;
-            mc.xc[i] = cl[(size_t)l + 1].b.p;
+            mc.xc[i] = col.lv[(size_t)l + 1].b.p;
         }
         RET(prof_mark(h, l, 0));
         cudaError_t le = cudaSuccess;
@@ -1534,17 +1572,14 @@ int leg_down_multi(amg1d* h, int l, const int* act, int na, int nPre, double alp
                                         leg_rec(h, lv, t.mc));
         if (fr == FUSED_ERR) return fail(h, AMG1D_ERR_CUDA, "f_down_multi launch failed on level %d: %s", l, cudaGetErrorString(le));
         if (fr == FUSED_OK) {
-            for (int i = 0; i < na; ++i) M.col[(size_t)act[i]][(size_t)l].cur = ob[i];
+            for (int i = 0; i < na; ++i) M.col[(size_t)act[i]].lv[(size_t)l].cur = ob[i];
             h->launch_counter++;
             LAUNCH_CHECK();
             return prof_mark(h, l, 0);
         }
         RET(prof_unmark(h, l, 0));
     }
-    for (int i = 0; i < na; ++i) {
-        ColumnBind cb(h, act[i]);
-        RET(leg_down(h, l, nPre, alpha, zero0));
-    }
+    for (int i = 0; i < na; ++i) RET(leg_down(h, M.col[(size_t)act[i]], l, nPre, alpha, zero0));
     return AMG1D_OK;
 }
 
@@ -1556,14 +1591,14 @@ int leg_up_multi(amg1d* h, int l, const int* act, int na, int nPost, double alph
     if (multi_leg_level(h, l)) {
         MultiCols mc = {};
         for (int i = 0; i < na; ++i) {
-            auto& cl = M.col[(size_t)act[i]];
-            auto& v = cl[(size_t)l];
-            auto& vc = cl[(size_t)l + 1];
+            Column& col = M.col[(size_t)act[i]];
+            Column::Vecs& v = col.lv[(size_t)l];
+            Column::Vecs& vc = col.lv[(size_t)l + 1];
             mc.b[i] = v.b.p;
             mc.xin[i] = v.x[v.cur].p;
             mc.xout[i] = v.x[1 - v.cur].p;
             mc.xc[i] = vc.x[vc.cur].p;
-            mc.partial[i] = norm ? M.partial[(size_t)act[i]] : nullptr;
+            mc.partial[i] = norm ? col.partial : nullptr;
         }
         RET(prof_mark(h, l, 1));
         cudaError_t le = cudaSuccess;
@@ -1573,14 +1608,13 @@ int leg_up_multi(amg1d* h, int l, const int* act, int na, int nPost, double alph
                                       h->opt_pdl != 0, &le, leg_rec(h, lv, t.mc));
         if (fr == FUSED_ERR) return fail(h, AMG1D_ERR_CUDA, "f_up_multi launch failed on level %d: %s", l, cudaGetErrorString(le));
         if (fr == FUSED_OK) {
-            for (int i = 0; i < na; ++i) { auto& v = M.col[(size_t)act[i]][(size_t)l]; v.cur = 1 - v.cur; }
+            for (int i = 0; i < na; ++i) { auto& v = M.col[(size_t)act[i]].lv[(size_t)l]; v.cur = 1 - v.cur; }
             h->launch_counter++;
             LAUNCH_CHECK();
             RET(prof_mark(h, l, 1));
             if (norm)
                 for (int i = 0; i < na; ++i) {
-                    ColumnBind cb(h, act[i]);
-                    RET(op_reduce_partials(h, nb, 0));
+                    RET(op_reduce_partials(h, M.col[(size_t)act[i]], nb, 0, true));
                     done[i] = true;
                 }
             return AMG1D_OK;
@@ -1588,9 +1622,8 @@ int leg_up_multi(amg1d* h, int l, const int* act, int na, int nPost, double alph
         RET(prof_unmark(h, l, 1));
     }
     for (int i = 0; i < na; ++i) {
-        ColumnBind cb(h, act[i]);
         bool pushed = false;
-        RET(leg_up(h, l, nPost, alpha, norm, &done[i], &pushed));
+        RET(leg_up(h, M.col[(size_t)act[i]], l, nPost, alpha, norm, &done[i], &pushed));
     }
     return AMG1D_OK;
 }
@@ -1605,7 +1638,7 @@ int enqueue_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, 
     for (int l = 0; l < nl - 1 && l < ts; ++l) RET(leg_down_multi(h, l, act, na, nPre, alpha, zero0));
     if (ts < nl) {
         for (int i = 0; i < na; ++i) {
-            for (int l = ts; l < nl; ++l) M.col[(size_t)act[i]][(size_t)l].cur = 0;
+            for (int l = ts; l < nl; ++l) M.col[(size_t)act[i]].lv[(size_t)l].cur = 0;
             cudaError_t te = tail_launch(h->L[ts].m, M.d_tail + (size_t)act[i] * TAIL_MAXL, nl - ts, h->coarse_fac,
                                          nPre, nPost, alpha, h->tail_plan_, h->stream, h->opt_pdl != 0);
             if (te != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "f_tail launch failed: %s", cudaGetErrorString(te));
@@ -1613,24 +1646,21 @@ int enqueue_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, 
         }
     } else {
         for (int i = 0; i < na; ++i) {
-            ColumnBind cb(h, act[i]);
-            Level& lv = h->L[nl - 1];
-            if (nl > 1 || zero0) lv.cur = 0;
-            RET(op_coarse(h, lv.b.p, lv.x[lv.cur].p));
+            Column::Vecs& v = M.col[(size_t)act[i]].lv[(size_t)nl - 1];
+            if (nl > 1 || zero0) v.cur = 0;
+            RET(op_coarse(h, v.b.p, v.x[v.cur].p));
         }
     }
     for (int l = std::min(nl - 2, ts - 1); l >= 0; --l)
         RET(leg_up_multi(h, l, act, na, nPost, alpha, want_norm && l == 0, done));
     for (int i = 0; i < na; ++i) {
-        auto& v = M.col[(size_t)act[i]][0];
+        Column& col = M.col[(size_t)act[i]];
+        auto& v = col.lv[0];
         if (v.cur != 0) {
             CK(cudaMemcpyAsync(v.x[0].p, v.x[1].p, (size_t)v.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
             v.cur = 0;
         }
-        if (want_norm && !done[i]) {
-            ColumnBind cb(h, act[i]);
-            RET(op_resnorm(h, 0, 0));
-        }
+        if (want_norm && !done[i]) RET(op_resnorm(h, col, 0, 0));
     }
     return AMG1D_OK;
 }
@@ -1640,45 +1670,15 @@ int run_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, doub
     if (nPre < 0 || nPost < 0) return fail(h, AMG1D_ERR_ARG, "nPre and nPost must be >= 0");
     amg1d::Multi& M = h->multi;
     RET(multi_sync_tail(h));
-    if (!h->opt_graph || h->opt_profile) {
-        const int64_t c0 = h->launch_counter;
-        RET(enqueue_vcycle_multi(h, act, na, nPre, nPost, alpha, want_norm, zero0));
-        M.launches_per_cycle = h->launch_counter - c0;
-        return AMG1D_OK;
+    GraphEntry key;
+    key.pre = nPre; key.post = nPost; key.alpha = alpha; key.norm = (int)want_norm; key.zero0 = (int)zero0;
+    bool parity0 = true;
+    for (int i = 0; i < na; ++i) {
+        key.mask |= 1u << act[i];
+        parity0 = parity0 && M.col[(size_t)act[i]].lv[0].cur == 0;
     }
-    unsigned mask = 0;
-    for (int i = 0; i < na; ++i) mask |= 1u << act[i];
-    amg1d::Multi::Graph* ge = nullptr;
-    for (auto& g : M.graphs)
-        if (g.g.exec && g.mask == mask && g.g.pre == nPre && g.g.post == nPost && g.g.alpha == alpha &&
-            g.g.norm == (int)want_norm && g.g.zero0 == (int)zero0)
-            ge = &g;
-    if (!ge) {
-        ge = &M.graphs[0];
-        for (auto& g : M.graphs) if (!g.g.exec) { ge = &g; break; } else if (g.g.stamp < ge->g.stamp) ge = &g;
-        if (ge->g.exec) { cudaGraphExecDestroy(ge->g.exec); ge->g.exec = nullptr; }
-        for (int i = 0; i < na; ++i)
-            if (M.col[(size_t)act[i]][0].cur != 0) return fail(h, AMG1D_ERR_STATE, "internal: level-0 buffer parity");
-        cudaGraph_t g = nullptr;
-        const int64_t c0 = h->launch_counter;
-        CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
-        int rc = enqueue_vcycle_multi(h, act, na, nPre, nPost, alpha, want_norm, zero0);
-        cudaError_t ce = cudaStreamEndCapture(h->stream, &g);
-        if (rc != AMG1D_OK) { if (g) cudaGraphDestroy(g); return rc; }
-        if (ce != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(ce));
-        ge->g.launches = h->launch_counter - c0;
-        h->launch_counter = c0;
-        ce = cudaGraphInstantiate(&ge->g.exec, g, 0);
-        cudaGraphDestroy(g);
-        if (ce != cudaSuccess) { ge->g.exec = nullptr; return fail(h, AMG1D_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(ce)); }
-        ge->g.pre = nPre; ge->g.post = nPost; ge->g.alpha = alpha; ge->g.norm = (int)want_norm; ge->g.zero0 = (int)zero0;
-        ge->mask = mask;
-    }
-    ge->g.stamp = ++h->graph_clock;
-    CK(cudaGraphLaunch(ge->g.exec, h->stream));
-    M.launches_per_cycle = ge->g.launches;
-    h->launch_counter += ge->g.launches;
-    return AMG1D_OK;
+    return replay_vcycle(h, M.graphs, key, parity0, &M.launches_per_cycle,
+                         [&] { return enqueue_vcycle_multi(h, act, na, nPre, nPost, alpha, want_norm, zero0); });
 }
 
 // need_rhs: the call reads the set's right-hand sides, which amg1d_dev_pcg_multi consumes
@@ -2036,15 +2036,14 @@ int amg1d_destroy(amg1d_t* h) {
     if (!h) return AMG1D_OK;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
-    for (auto& g : h->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
-    for (auto& g : h->multi.graphs) if (g.g.exec) cudaGraphExecDestroy(g.g.exec);
-    for (auto& cl : h->multi.col) for (auto& v : cl) { vec_free(v.x[0]); vec_free(v.x[1]); vec_free(v.b); }
-    for (double* p : h->multi.partial) cudaFree(p);
-    for (auto& g : h->multi.cg) { vec_free(g.x); vec_free(g.p); vec_free(g.ap); }
+    release_graphs(h->graphs);
+    release_graphs(h->multi.graphs);
+    for (auto& col : h->multi.col) column_free(h, col);
+    column_free(h, h->res);
     if (h->multi.d_scal) cudaFree(h->multi.d_scal);
     if (h->multi.h_scal) cudaFreeHost(h->multi.h_scal);
     if (h->multi.d_tail) cudaFree(h->multi.d_tail);
-    vec_free(h->cg_x); vec_free(h->cg_p); vec_free(h->cg_ap);
+    if (h->res.scal) cudaFree(h->res.scal);
     for (auto& pr : h->prof) for (auto ev : pr.ev) cudaEventDestroy(ev);
     for (auto& lv : h->L) {
         if (lv.mat_alloc) cudaFree(lv.mat_alloc);
@@ -2052,7 +2051,6 @@ int amg1d_destroy(amg1d_t* h) {
         if (lv.pat) cudaFree(lv.pat);
         free_flux(h, lv);
         if (lv.perm) cudaFree(lv.perm);
-        vec_free(lv.x[0]); vec_free(lv.x[1]); vec_free(lv.b);
     }
     for (auto& t : h->T) {
         if (t.parent) cudaFree(t.parent);
@@ -2062,8 +2060,6 @@ int amg1d_destroy(amg1d_t* h) {
     }
     vec_free(h->scratch);
     if (h->stage) cudaFree(h->stage);
-    if (h->partial) cudaFree(h->partial);
-    if (h->d_scal) cudaFree(h->d_scal);
     if (h->h_scal) cudaFreeHost(h->h_scal);
     if (h->coarse_fac) cudaFree(h->coarse_fac);
     if (h->d_tail) cudaFree(h->d_tail);
@@ -2613,26 +2609,14 @@ int amg1d_finalize(amg1d_t* h) {
 #ifdef AMG1D_WITH_NCCL
     if (h->nranks > 1 && h->opt_p2p) RET(p2p_alloc_arena(h));
 #endif
-    for (int l = 0; l < h->n_levels; ++l) {
-        Level& lv = h->L[l];
+    for (const Level& lv : h->L) {
         if (!lv.present && !lv.proxy) continue;
-        if (lv.sharded && h->p2p.arena) {             // peer-mapped (halo_p2p.cuh)
-            RET(vec_from_arena(h, lv.x[0], lv.n, lv.m));
-            RET(vec_from_arena(h, lv.b, lv.n, lv.m));
-            RET(vec_from_arena(h, lv.x[1], lv.n, lv.m));
-            maxlen = std::max(maxlen, lv.n * lv.m);
-            h->partial_cap = std::max<int64_t>(h->partial_cap, lv.n / (lv.m > 5 ? 16 : FUSED_B / 2) + 16);
-            continue;
-        }
-        RET(vec_alloc(h, lv.x[0], lv.n, lv.m));
-        RET(vec_alloc(h, lv.b, lv.n, lv.m));
-        if (lv.present) RET(vec_alloc(h, lv.x[1], lv.n, lv.m));
         maxlen = std::max(maxlen, lv.n * lv.m);
         h->partial_cap = std::max<int64_t>(h->partial_cap, lv.n / (lv.m > 5 ? 16 : FUSED_B / 2) + 16);
     }
+    RET(column_alloc(h, h->res, false));
     RET(vec_alloc(h, h->scratch, maxlen, 1));
-    RET(dev_alloc(h, (void**)&h->partial, (h->partial_cap + 256) * 8));
-    RET(dev_alloc(h, (void**)&h->d_scal, 64 * 8));
+    RET(dev_alloc(h, (void**)&h->res.scal, 64 * 8));
     CK(cudaMallocHost(&h->h_scal, 64 * 8));
     if (h->L[h->n_levels - 1].present) RET(factor_coarsest(h));
     RET(build_tail(h));
@@ -2652,7 +2636,7 @@ int amg1d_finalize(amg1d_t* h) {
     for (auto& lv : h->L) free_flux(h, lv);
     CK(cudaStreamSynchronize(h->stream));
 #ifdef AMG1D_WITH_NCCL
-    if (h->nranks > 1) RET(p2p_connect(h));           // collective: every rank reaches this point or none does
+    if (h->nranks > 1) RET(p2p_connect(h, h->res));           // collective: every rank reaches this point or none does
 #endif
     h->finalized = true;
     return AMG1D_OK;
@@ -2662,35 +2646,37 @@ int amg1d_finalize(amg1d_t* h) {
 int amg1d_dev_set_problem(amg1d_t* h, const double* x0, const double* b) {
     RET(check_ready(h));
     Level& l0 = h->L[0];
+    Column::Vecs& v0 = h->res.lv[0];
     h->norm_valid = false;
     if (!b && !h->dev_problem)
         return fail(h, AMG1D_ERR_STATE, "amg1d_dev_set_problem: b == NULL keeps the resident right-hand side, but that "
                     "was overwritten by a per-level host operation");
     if (b) {
-        RET(to_device(h, 0, b, l0.b.p));
-        if (l0.sharded) RET(op_halo(h, l0.b.p, l0.n, l0.m));
+        RET(to_device(h, 0, b, v0.b.p));
+        if (l0.sharded) RET(op_halo(h, v0.b.p, l0.n, l0.m));
         h->dev_problem = true;
     }
-    if (l0.cur != 0) l0.cur = 0;
-    if (x0) RET(to_device(h, 0, x0, l0.x[0].p));
-    else CK(cudaMemsetAsync(l0.x[0].p, 0, (size_t)l0.x[0].len * 8, h->stream));
+    if (v0.cur != 0) v0.cur = 0;
+    if (x0) RET(to_device(h, 0, x0, v0.x[0].p));
+    else CK(cudaMemsetAsync(v0.x[0].p, 0, (size_t)v0.x[0].len * 8, h->stream));
     // ghosts of the new iterate.  (The two-sided exchange also orders this call after the neighbours' last
     // peer-memory push of an earlier cycle, which targets the same ghost slots.)
-    if (l0.sharded) RET(op_halo(h, l0.x[0].p, l0.n, l0.m));
+    if (l0.sharded) RET(op_halo(h, v0.x[0].p, l0.n, l0.m));
     return AMG1D_OK;
 }
 
 int amg1d_dev_fill_rhs_random(amg1d_t* h, uint64_t seed) {
     RET(check_ready(h));
     Level& l0 = h->L[0];
+    Column::Vecs& v0 = h->res.lv[0];
     if (l0.perm) return fail(h, AMG1D_ERR_UNSUPPORTED, "random rhs only for unpermuted (DG) fine levels");
     h->norm_valid = false;
-    k_fill_random<<<1184, 256, 0, h->stream>>>(l0.b.p, l0.b.len, seed, l0.start * l0.m);
+    k_fill_random<<<1184, 256, 0, h->stream>>>(v0.b.p, v0.b.len, seed, l0.start * l0.m);
     LAUNCH_CHECK();
     h->dev_problem = true;
-    l0.cur = 0;
-    CK(cudaMemsetAsync(l0.x[0].p, 0, (size_t)l0.x[0].len * 8, h->stream));
-    if (l0.sharded) RET(op_halo(h, l0.b.p, l0.n, l0.m, l0.x[0].p, l0.n, l0.m));
+    v0.cur = 0;
+    CK(cudaMemsetAsync(v0.x[0].p, 0, (size_t)v0.x[0].len * 8, h->stream));
+    if (l0.sharded) RET(op_halo(h, v0.b.p, l0.n, l0.m, v0.x[0].p, l0.n, l0.m));
     return AMG1D_OK;
 }
 
@@ -2699,6 +2685,7 @@ int amg1d_dev_assemble_rhs(amg1d_t* h, int kind, int nq, const double* xi, const
                            int n_fix, const int64_t* fix_slot, const double* fix_val, const int* fix_op) {
     RET(check_ready(h));
     Level& l0 = h->L[0];
+    Column::Vecs& v0 = h->res.lv[0];
     if (kind < 0 || kind > 1) return fail(h, AMG1D_ERR_ARG, "kind must be 0 (DG-type level) or 1 (CG level in group form)");
     if (!xi || !W || !terms || nq < 1 || nq > AMG1D_RHS_MAXQ || n_basis < 1 || n_basis > AMG1D_RHS_MAXM ||
         n_terms < 1 || n_terms > AMG1D_RHS_MAXT)
@@ -2731,16 +2718,16 @@ int amg1d_dev_assemble_rhs(amg1d_t* h, int kind, int nq, const double* xi, const
     h->norm_valid = false;
     // the slab with its ghost elements (their right-hand side feeds the recomputed halo of the fused legs)
     const int64_t e0 = -(int64_t)l0.gl, e1 = l0.n + l0.gr;
-    CK(cudaMemsetAsync(l0.b.p + e0 * l0.m, 0, (size_t)(e1 - e0) * l0.m * 8, h->stream));
+    CK(cudaMemsetAsync(v0.b.p + e0 * l0.m, 0, (size_t)(e1 - e0) * l0.m * 8, h->stream));
     k_assemble_rhs<<<(unsigned)((e1 - e0 + 127) / 128), 128, 0, h->stream>>>(sp, dvert.p && vertices ? dvert.p : nullptr,
-                                                                          l0.start, e0, e1, e1 * l0.m, l0.b.p, 0);
+                                                                          l0.start, e0, e1, e1 * l0.m, v0.b.p, 0);
     h->launch_counter++;
     LAUNCH_CHECK();
     if (kind == 1 && l0.gl) {
         // the first ghost group's vertex also receives fe[1] of the element left of it, which no thread of this
         // rank visits: recompute that one element's contribution
         k_assemble_rhs<<<1, 1, 0, h->stream>>>(sp, dvert.p && vertices ? dvert.p : nullptr, l0.start, e0 - 1, e0,
-                                               e1 * l0.m, l0.b.p, 1);
+                                               e1 * l0.m, v0.b.p, 1);
         h->launch_counter++;
         LAUNCH_CHECK();
     }
@@ -2749,15 +2736,15 @@ int amg1d_dev_assemble_rhs(amg1d_t* h, int kind, int nq, const double* xi, const
         CK(cudaMemcpyAsync(dfs.p, fix_slot, (size_t)n_fix * 8, cudaMemcpyHostToDevice, h->stream));
         CK(cudaMemcpyAsync(dfv.p, fix_val, (size_t)n_fix * 8, cudaMemcpyHostToDevice, h->stream));
         CK(cudaMemcpyAsync(dfo.p, fix_op, (size_t)n_fix * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-        k_apply_fixes<<<1, 32, 0, h->stream>>>(l0.b.p, l0.start * l0.m, e0 * l0.m, e1 * l0.m, n_fix,
+        k_apply_fixes<<<1, 32, 0, h->stream>>>(v0.b.p, l0.start * l0.m, e0 * l0.m, e1 * l0.m, n_fix,
                                                reinterpret_cast<const int64_t*>(dfs.p), dfv.p,
                                                reinterpret_cast<const int*>(dfo.p));
         h->launch_counter++;
         LAUNCH_CHECK();
     }
-    l0.cur = 0;
-    CK(cudaMemsetAsync(l0.x[0].p, 0, (size_t)l0.x[0].len * 8, h->stream));
-    if (l0.sharded) RET(op_halo(h, l0.x[0].p, l0.n, l0.m));      // (zero ghosts; orders this call after earlier pushes)
+    v0.cur = 0;
+    CK(cudaMemsetAsync(v0.x[0].p, 0, (size_t)v0.x[0].len * 8, h->stream));
+    if (l0.sharded) RET(op_halo(h, v0.x[0].p, l0.n, l0.m));      // (zero ghosts; orders this call after earlier pushes)
     CK(cudaStreamSynchronize(h->stream));         // the staging buffers above are released on return
     h->dev_problem = true;
     return AMG1D_OK;
@@ -2766,39 +2753,25 @@ int amg1d_dev_assemble_rhs(amg1d_t* h, int kind, int nq, const double* xi, const
 int amg1d_dev_get_rhs(amg1d_t* h, double* b) {
     RET(check_dev_problem(h));
     if (!b) return fail(h, AMG1D_ERR_ARG, "null b");
-    return to_host(h, 0, h->L[0].b.p, b);
+    return to_host(h, 0, h->res.lv[0].b.p, b);
 }
 
 int amg1d_dev_solve(amg1d_t* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters, double* res) {
     RET(check_dev_problem(h));
     if (!res || !iters) return fail(h, AMG1D_ERR_ARG, "null argument");
     if (maxiter < 0) return fail(h, AMG1D_ERR_ARG, "maxiter must be >= 0");
-    Level& l0 = h->L[0];
-    int rc = op_norm(h, l0.b.p, nullptr, l0.b.len, 2);
-    int it = 0;
-    for (int i = 0; i < maxiter && rc == AMG1D_OK; ++i) {
-        rc = run_vcycle(h, nPre, nPost, alpha, true);
-        if (rc != AMG1D_OK) break;
-        rc = read_scalars(h, 3);
-        if (rc != AMG1D_OK) break;
-        res[i] = h->h_scal[0];
-        it = i + 1;
-        if (res[i] < tol * h->h_scal[2]) break;
-    }
-    RET(rc);
-    *iters = it;
-    return AMG1D_OK;
+    return multigrid_run(h, maxiter, tol, nPre, nPost, alpha, iters, res, nullptr, nullptr);
 }
 
 int amg1d_dev_vcycle(amg1d_t* h, int nPre, int nPost, double alpha, int with_residual_norm) {
     RET(check_dev_problem(h));
-    return run_vcycle(h, nPre, nPost, alpha, with_residual_norm != 0);
+    return run_vcycle(h, h->res, nPre, nPost, alpha, with_residual_norm != 0);
 }
 
 int amg1d_dev_residual_norm(amg1d_t* h, double* res) {
     RET(check_dev_problem(h));
-    if (!h->norm_valid) RET(op_resnorm(h, 0, 0));
-    RET(read_scalars(h, 1));
+    if (!h->norm_valid) RET(op_resnorm(h, h->res, 0, 0));
+    RET(read_scalars(h, h->res, 1));
     if (res) *res = h->h_scal[0];
     return AMG1D_OK;
 }
@@ -2806,8 +2779,9 @@ int amg1d_dev_residual_norm(amg1d_t* h, double* res) {
 int amg1d_dev_rhs_norm(amg1d_t* h, double* nb) {
     RET(check_dev_problem(h));
     // slot 2 (as amg1d_solve): slot 0 caches ||b - A x|| of a norm-fused V-cycle (norm_valid) and must survive
-    RET(op_norm(h, h->L[0].b.p, nullptr, h->L[0].b.len, 2));
-    RET(read_scalars(h, 3));
+    Column::Vecs& v0 = h->res.lv[0];
+    RET(op_norm(h, h->res, v0.b.p, nullptr, v0.b.len, 2));
+    RET(read_scalars(h, h->res, 3));
     if (nb) *nb = h->h_scal[2];
     return AMG1D_OK;
 }
@@ -2815,7 +2789,7 @@ int amg1d_dev_rhs_norm(amg1d_t* h, double* nb) {
 int amg1d_dev_get_solution(amg1d_t* h, double* x) {
     RET(check_ready(h));
     if (!x) return fail(h, AMG1D_ERR_ARG, "null x");
-    return to_host(h, 0, h->L[0].x[h->L[0].cur].p, x);
+    return to_host(h, 0, h->res.lv[0].x[h->res.lv[0].cur].p, x);
 }
 
 // ---- multi-column resident problems ----------------------------------------------------------------------------
@@ -2829,7 +2803,7 @@ int amg1d_dev_set_problems(amg1d_t* h, int k, const double* X0, const double* B)
     M.k = 0;
     M.norm_valid = false;
     for (int c = 0; c < k; ++c) {
-        auto& v = M.col[(size_t)c][0];
+        auto& v = M.col[(size_t)c].lv[0];
         RET(to_device(h, 0, B + c * nh, v.b.p));
         v.cur = 0;
         if (X0) RET(to_device(h, 0, X0 + c * nh, v.x[0].p));
@@ -2849,7 +2823,7 @@ int amg1d_dev_fill_rhs_random_multi(amg1d_t* h, int k, uint64_t seed) {
     amg1d::Multi& M = h->multi;
     M.norm_valid = false;
     for (int c = 0; c < k; ++c) {
-        auto& v = M.col[(size_t)c][0];
+        auto& v = M.col[(size_t)c].lv[0];
         k_fill_random<<<1184, 256, 0, h->stream>>>(v.b.p, v.b.len, seed + (uint64_t)c, l0.start * l0.m);
         LAUNCH_CHECK();
         v.cur = 0;
@@ -2875,10 +2849,7 @@ int amg1d_dev_residual_norms(amg1d_t* h, double* res) {
     RET(check_multi(h, true));
     amg1d::Multi& M = h->multi;
     if (!M.norm_valid)
-        for (int c = 0; c < M.k; ++c) {
-            ColumnBind cb(h, c);
-            RET(op_resnorm(h, 0, 0));
-        }
+        for (int c = 0; c < M.k; ++c) RET(op_resnorm(h, M.col[(size_t)c], 0, 0));
     RET(read_multi_scalars(h));
     if (res)
         for (int c = 0; c < M.k; ++c) res[c] = M.h_scal[c * MULTI_SLOTS];
@@ -2894,8 +2865,8 @@ int amg1d_dev_solve_multi(amg1d_t* h, int maxiter, double tol, int nPre, int nPo
     const int k = M.k;
     for (int c = 0; c < k; ++c) {
         iters[c] = 0;
-        ColumnBind cb(h, c);
-        RET(op_norm(h, h->L[0].b.p, nullptr, h->L[0].b.len, 2));
+        Column& col = M.col[(size_t)c];
+        RET(op_norm(h, col, col.lv[0].b.p, nullptr, col.lv[0].b.len, 2));
     }
     M.norm_valid = false;
     int act[MULTI_MAX_COLS];
@@ -2922,7 +2893,7 @@ int amg1d_dev_get_solutions(amg1d_t* h, double* X) {
     if (!X) return fail(h, AMG1D_ERR_ARG, "null X");
     const int64_t nh = h->L[0].n_host;
     for (int c = 0; c < h->multi.k; ++c) {
-        auto& v = h->multi.col[(size_t)c][0];
+        auto& v = h->multi.col[(size_t)c].lv[0];
         RET(to_host(h, 0, v.x[v.cur].p, X + c * nh));
     }
     return AMG1D_OK;
@@ -2938,10 +2909,10 @@ void* amg1d_stream(amg1d_t* h) { return h ? (void*)h->stream : nullptr; }
 
 void* amg1d_dev_ptr(amg1d_t* h, int level, int which) {
     if (!valid_level(h, level) || !h->finalized) return nullptr;
-    Level& lv = h->L[level];
+    Column::Vecs& v = h->res.lv[(size_t)level];
     switch (which) {
-        case AMG1D_VEC_X: return lv.x[lv.cur].p;
-        case AMG1D_VEC_B: return lv.b.p;
+        case AMG1D_VEC_X: return v.x[v.cur].p;
+        case AMG1D_VEC_B: return v.b.p;
         case AMG1D_VEC_R: return h->scratch.p;
         default: return nullptr;
     }
@@ -2951,8 +2922,8 @@ int amg1d_vcycle(amg1d_t* h, double* x, const double* b, int nPre, int nPost, do
     RET(check_ready(h));
     if (!x || !b) return fail(h, AMG1D_ERR_ARG, "null vector");
     RET(amg1d_dev_set_problem(h, x, b));
-    RET(run_vcycle(h, nPre, nPost, alpha, false));
-    return to_host(h, 0, h->L[0].x[h->L[0].cur].p, x);
+    RET(run_vcycle(h, h->res, nPre, nPost, alpha, false));
+    return to_host(h, 0, h->res.lv[0].x[h->res.lv[0].cur].p, x);
 }
 
 int amg1d_solve(amg1d_t* h, double* x, const double* b, int maxiter, double tol, int nPre,
@@ -2961,46 +2932,28 @@ int amg1d_solve(amg1d_t* h, double* x, const double* b, int maxiter, double tol,
     RET(check_ready(h));
     if (!x || !b || !res || !iters) return fail(h, AMG1D_ERR_ARG, "null argument");
     if (maxiter < 0) return fail(h, AMG1D_ERR_ARG, "maxiter must be >= 0");
-    Level& l0 = h->L[0];
+    Column::Vecs& v0 = h->res.lv[0];
     RET(amg1d_dev_set_problem(h, x, b));
     DevBuf exact;
-    double* d_exact = nullptr;
     if (err && u_exact) {
-        CK(exact.alloc(l0.x[0].len + 8));
-        d_exact = exact.p;
-        RET(to_device(h, 0, u_exact, d_exact));
+        CK(exact.alloc(v0.x[0].len + 8));
+        RET(to_device(h, 0, u_exact, exact.p));
     }
-    int rc = op_norm(h, l0.b.p, nullptr, l0.b.len, 2);
-    int it = 0;
-    for (int i = 0; i < maxiter && rc == AMG1D_OK; ++i) {
-        rc = run_vcycle(h, nPre, nPost, alpha, true);
-        if (rc != AMG1D_OK) break;
-        if (d_exact) {
-            rc = op_norm(h, l0.x[l0.cur].p, d_exact, l0.x[0].len, 1);
-            if (rc != AMG1D_OK) break;
-        }
-        rc = read_scalars(h, 3);
-        if (rc != AMG1D_OK) break;
-        res[i] = h->h_scal[0];
-        if (err) err[i] = d_exact ? h->h_scal[1] : NAN;
-        it = i + 1;
-        if (res[i] < tol * h->h_scal[2]) break;
-    }
-    RET(rc);
-    *iters = it;
-    return to_host(h, 0, l0.x[l0.cur].p, x);
+    RET(multigrid_run(h, maxiter, tol, nPre, nPost, alpha, iters, res, err, exact.p));
+    return to_host(h, 0, v0.x[v0.cur].p, x);
 }
 
 int amg1d_ldiv(amg1d_t* h, double* y, const double* b, int nPre, int nPost, double alpha) {
     RET(check_ready(h));
     if (!y || !b) return fail(h, AMG1D_ERR_ARG, "null vector");
     Level& l0 = h->L[0];
+    Column::Vecs& v0 = h->res.lv[0];
     h->norm_valid = false;
-    RET(to_device(h, 0, b, l0.b.p));
-    if (l0.sharded) RET(op_halo(h, l0.b.p, l0.n, l0.m));
-    l0.cur = 0;
-    RET(run_vcycle(h, nPre, nPost, alpha, false, true));      // zero guess: x0 is neither uploaded nor read
-    return to_host(h, 0, l0.x[l0.cur].p, y);
+    RET(to_device(h, 0, b, v0.b.p));
+    if (l0.sharded) RET(op_halo(h, v0.b.p, l0.n, l0.m));
+    v0.cur = 0;
+    RET(run_vcycle(h, h->res, nPre, nPost, alpha, false, true));      // zero guess: x0 is neither uploaded nor read
+    return to_host(h, 0, v0.x[v0.cur].p, y);
 }
 
 // multigrid_v_cycle / ldiv! on `count` independent problems, software-pipelined over PCIe: while problem k runs its
@@ -3016,6 +2969,7 @@ int amg1d_vcycle_batch(amg1d_t* h, int count, double* const* x, const double* co
         if (!x[k] || !b[k]) return fail(h, AMG1D_ERR_ARG, "null vector %d", k);
     if (count == 0) return AMG1D_OK;
     Level& l0 = h->L[0];
+    Column::Vecs& v0 = h->res.lv[0];
     amg1d::Pipe& P = h->pipe;
     if (!P.s_in) {
         CK(cudaStreamCreateWithFlags(&P.s_in, cudaStreamNonBlocking));
@@ -3050,27 +3004,27 @@ int amg1d_vcycle_batch(amg1d_t* h, int count, double* const* x, const double* co
         CK(cudaEventRecord(P.ev_in[sl], P.s_in));
         // ---- compute stream
         CK(cudaStreamWaitEvent(h->stream, P.ev_in[sl], 0));
-        l0.cur = 0;
+        v0.cur = 0;
         if (l0.perm) {
-            k_gather_perm<<<gp, 256, 0, h->stream>>>(l0.perm, P.st_b[sl], l0.b.p, ns);
-            if (!zero_guess) k_gather_perm<<<gp, 256, 0, h->stream>>>(l0.perm, P.st_x[sl], l0.x[0].p, ns);
+            k_gather_perm<<<gp, 256, 0, h->stream>>>(l0.perm, P.st_b[sl], v0.b.p, ns);
+            if (!zero_guess) k_gather_perm<<<gp, 256, 0, h->stream>>>(l0.perm, P.st_x[sl], v0.x[0].p, ns);
             LAUNCH_CHECK();
         } else {
-            CK(cudaMemcpyAsync(l0.b.p, P.st_b[sl], bytes, cudaMemcpyDeviceToDevice, h->stream));
-            if (!zero_guess) CK(cudaMemcpyAsync(l0.x[0].p, P.st_x[sl], bytes, cudaMemcpyDeviceToDevice, h->stream));
+            CK(cudaMemcpyAsync(v0.b.p, P.st_b[sl], bytes, cudaMemcpyDeviceToDevice, h->stream));
+            if (!zero_guess) CK(cudaMemcpyAsync(v0.x[0].p, P.st_x[sl], bytes, cudaMemcpyDeviceToDevice, h->stream));
         }
         CK(cudaEventRecord(P.ev_used[sl], h->stream));
         if (l0.sharded) {
-            if (zero_guess) RET(op_halo(h, l0.b.p, l0.n, l0.m));
-            else RET(op_halo(h, l0.b.p, l0.n, l0.m, l0.x[0].p, l0.n, l0.m));
+            if (zero_guess) RET(op_halo(h, v0.b.p, l0.n, l0.m));
+            else RET(op_halo(h, v0.b.p, l0.n, l0.m, v0.x[0].p, l0.n, l0.m));
         }
-        RET(run_vcycle(h, nPre, nPost, alpha, false, zero_guess != 0));
+        RET(run_vcycle(h, h->res, nPre, nPost, alpha, false, zero_guess != 0));
         if (k >= 2) CK(cudaStreamWaitEvent(h->stream, P.ev_out[sl], 0));      // the iterate of problem k - 2 has left
         if (l0.perm) {
-            k_scatter_perm<<<gp, 256, 0, h->stream>>>(l0.perm, l0.x[l0.cur].p, P.st_o[sl], ns);
+            k_scatter_perm<<<gp, 256, 0, h->stream>>>(l0.perm, v0.x[v0.cur].p, P.st_o[sl], ns);
             LAUNCH_CHECK();
         } else {
-            CK(cudaMemcpyAsync(P.st_o[sl], l0.x[l0.cur].p, bytes, cudaMemcpyDeviceToDevice, h->stream));
+            CK(cudaMemcpyAsync(P.st_o[sl], v0.x[v0.cur].p, bytes, cudaMemcpyDeviceToDevice, h->stream));
         }
         CK(cudaEventRecord(P.ev_done[sl], h->stream));
         // ---- copy-out stream
@@ -3087,31 +3041,23 @@ int amg1d_vcycle_batch(amg1d_t* h, int count, double* const* x, const double* co
 }  // extern "C"
 
 namespace {
-// Conjugate gradients preconditioned with one V-cycle (ldiv!(z, H, r)); expects the initial guess in cg_x and the
-// right-hand side in level 0's rhs buffer, which becomes the residual.  The solution is left in cg_x.
-int pcg_alloc(amg1d* h) {
+// Conjugate gradients preconditioned with one V-cycle (ldiv!(z, H, r)) on the resident problem col; expects the initial
+// guess in col.cg.x and the right-hand side in its level-0 rhs buffer, which becomes the residual.  The solution is left
+// in col.cg.x.
+int pcg_run(amg1d* h, Column& col, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters, double* res) {
     Level& l0 = h->L[0];
-    if (!h->cg_x.raw) {
-        RET(vec_alloc(h, h->cg_x, l0.n, l0.m));
-        RET(vec_alloc(h, h->cg_p, l0.n, l0.m));
-        RET(vec_alloc(h, h->cg_ap, l0.n, l0.m));
-    }
-    return AMG1D_OK;
-}
-
-int pcg_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters, double* res) {
-    Level& l0 = h->L[0];
+    Column::Vecs& v0 = col.lv[0];
     const int64_t N = l0.n * l0.m;
     h->norm_valid = false;
     h->dev_problem = false;                   // level 0's rhs buffer becomes the CG residual
-    double* X = h->cg_x.p;
-    double* P = h->cg_p.p;
-    double* AP = h->cg_ap.p;
-    double* R = l0.b.p;                       // the residual lives in the level's rhs buffer: it IS the
+    double* X = col.cg.x.p;
+    double* P = col.cg.p.p;
+    double* AP = col.cg.ap.p;
+    double* R = v0.b.p;                       // the residual lives in the level's rhs buffer: it IS the
                                               // right-hand side of every preconditioner application
-    RET(op_norm(h, R, nullptr, N, CG_NB));                       // ||b||
+    RET(op_norm(h, col, R, nullptr, N, CG_NB));                       // ||b||
     // r = b - A x0
-    RET(op_matvec_dot(h, 0, X, AP, -1));
+    RET(op_matvec_dot(h, col, 0, X, AP, -1));
     {
         int nb = (int)std::min<int64_t>(AMG1D_RED_BLOCKS, (N + AMG1D_RED_THREADS - 1) / AMG1D_RED_THREADS);
         k_axpy<<<nb, AMG1D_RED_THREADS, 0, h->stream>>>(R, AP, N, -1.0);
@@ -3122,8 +3068,8 @@ int pcg_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double alpha
     const int nbv = (int)std::max<int64_t>(1, std::min<int64_t>(AMG1D_RED_BLOCKS, (N + AMG1D_RED_THREADS - 1) / AMG1D_RED_THREADS));
     // the initial residual is tested first: b = 0 or an x0 that already solves the system returns x0 with
     // iters = 0 (r.z = p.Ap = 0 would otherwise make the first step 0 / 0)
-    RET(op_norm(h, R, nullptr, N, CG_RES));
-    RET(read_scalars(h, 3));
+    RET(op_norm(h, col, R, nullptr, N, CG_RES));
+    RET(read_scalars(h, col, 3));
     if (!std::isfinite(h->h_scal[CG_RES]) || !std::isfinite(h->h_scal[CG_NB]))
         return fail(h, AMG1D_ERR_ARG, "amg1d_pcg: non-finite right-hand side or initial guess");
     *iters = 0;
@@ -3131,24 +3077,24 @@ int pcg_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double alpha
     for (int i = 0; i < maxiter; ++i) {
         // z = M^-1 r: one V-cycle from a zero guess with rhs r (already in place); z = level-0 iterate
         if (l0.sharded) { rc = op_halo(h, R, l0.n, l0.m); if (rc) break; }
-        l0.cur = 0;
-        rc = run_vcycle(h, nPre, nPost, alpha, false, true);
+        v0.cur = 0;
+        rc = run_vcycle(h, col, nPre, nPost, alpha, false, true);
         if (rc) break;
-        double* Z = l0.x[l0.cur].p;
-        rc = op_dot(h, R, Z, N, i == 0 ? CG_RZ : CG_RZ_NEW);
+        double* Z = v0.x[v0.cur].p;
+        rc = op_dot(h, col, R, Z, N, i == 0 ? CG_RZ : CG_RZ_NEW);
         if (rc) break;
-        if (i > 0) { k_cg_beta<<<1, 1, 0, h->stream>>>(h->d_scal); h->launch_counter++; }
-        k_cg_direction<<<nbv, AMG1D_RED_THREADS, 0, h->stream>>>(P, Z, N, h->d_scal, i == 0 ? 1 : 0);
+        if (i > 0) { k_cg_beta<<<1, 1, 0, h->stream>>>(col.scal); h->launch_counter++; }
+        k_cg_direction<<<nbv, AMG1D_RED_THREADS, 0, h->stream>>>(P, Z, N, col.scal, i == 0 ? 1 : 0);
         h->launch_counter++;
-        rc = op_matvec_dot(h, 0, P, AP, CG_PAP);
+        rc = op_matvec_dot(h, col, 0, P, AP, CG_PAP);
         if (rc) break;
-        k_cg_alpha<<<1, 1, 0, h->stream>>>(h->d_scal);
-        k_cg_update<<<nbv, AMG1D_RED_THREADS, 0, h->stream>>>(X, R, P, AP, N, h->d_scal, h->partial);
+        k_cg_alpha<<<1, 1, 0, h->stream>>>(col.scal);
+        k_cg_update<<<nbv, AMG1D_RED_THREADS, 0, h->stream>>>(X, R, P, AP, N, col.scal, col.partial);
         h->launch_counter += 2;
         { cudaError_t e_ = cudaGetLastError(); if (e_ != cudaSuccess) { rc = fail(h, AMG1D_ERR_CUDA, "pcg kernels: %s", cudaGetErrorString(e_)); break; } }
-        rc = op_reduce_partials(h, nbv, CG_RES);                 // ||r||_2
+        rc = op_reduce_partials(h, col, nbv, CG_RES, true);       // ||r||_2
         if (rc) break;
-        rc = read_scalars(h, 3);
+        rc = read_scalars(h, col, 3);
         if (rc) break;
         res[i] = h->h_scal[CG_RES];
         it = i + 1;
@@ -3163,46 +3109,26 @@ int pcg_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double alpha
 }
 
 // ---- pcg_run on every column of the multi-column set (amg1d_dev_pcg_multi) --------------------------------------
-// Column c's level-0 CG vectors; allocated at the first call and grown with k, a failed allocation releases what it took.
-int pcg_multi_alloc(amg1d* h, int k) {
-    amg1d::Multi& M = h->multi;
-    const Level& l0 = h->L[0];
-    while ((int)M.cg.size() < k) {
-        amg1d::Multi::CgCol g;
-        int rc = vec_alloc(h, g.x, l0.n, l0.m);
-        if (rc == AMG1D_OK) rc = vec_alloc(h, g.p, l0.n, l0.m);
-        if (rc == AMG1D_OK) rc = vec_alloc(h, g.ap, l0.n, l0.m);
-        if (rc != AMG1D_OK) {
-            for (DVec* d : {&g.x, &g.p, &g.ap})
-                if (d->raw) { h->device_bytes -= vec_bytes(*d); vec_free(*d); }
-            cudaGetLastError();                  // an out-of-memory status must not surface at the next launch check
-            return fail(h, rc, "CG vectors of column %d of the multi-column set: %s", (int)M.cg.size(), h->err.c_str());
-        }
-        M.cg.push_back(g);
-    }
-    return AMG1D_OK;
-}
-
 // The vectors, reduction scratch and scalar windows of the active columns act[0..na), entry i for column act[i].
 struct CgMultiVecs {
     ColVecs X, R, P, AP, Z, part, scal;
     CgMultiVecs(amg1d* h, const int* act, int na) : X(), R(), P(), AP(), Z(), part(), scal() {
         amg1d::Multi& M = h->multi;
         for (int i = 0; i < na; ++i) {
-            const int c = act[i];
-            auto& v = M.col[(size_t)c][0];
-            X.v[i] = M.cg[(size_t)c].x.p;
-            P.v[i] = M.cg[(size_t)c].p.p;
-            AP.v[i] = M.cg[(size_t)c].ap.p;
+            Column& col = M.col[(size_t)act[i]];
+            auto& v = col.lv[0];
+            X.v[i] = col.cg.x.p;
+            P.v[i] = col.cg.p.p;
+            AP.v[i] = col.cg.ap.p;
             R.v[i] = v.b.p;                      // the residual lives in the column's level-0 rhs buffer, as in pcg_run
             Z.v[i] = v.x[v.cur].p;               // the preconditioned residual: the column's level-0 iterate
-            part.v[i] = M.partial[(size_t)c];
-            scal.v[i] = M.d_scal + c * MULTI_SLOTS;
+            part.v[i] = col.partial;
+            scal.v[i] = col.scal;
         }
     }
 };
 
-// op_sum_partials (take_sqrt 0) / op_reduce_partials (take_sqrt 1) of every active column in one launch per stage
+// op_reduce_partials of every active column in one launch per stage
 int reduce_partials_multi(amg1d* h, const CgMultiVecs& v, int na, int64_t np, int slot, int take_sqrt) {
     ColVecs src = v.part;
     if (np > 8192) {
@@ -3219,9 +3145,9 @@ int reduce_partials_multi(amg1d* h, const CgMultiVecs& v, int na, int64_t np, in
     return AMG1D_OK;
 }
 
-// op_matvec_dot(h, 0, x_c, y_c, slot) for every active column: one launch that reads level 0's operator once where
+// op_matvec_dot(h, col, 0, x_c, y_c, slot) for every active column: one launch that reads level 0's operator once where
 // op_matvec_dot would take the fused kernel (the same predicate, hence the same partial sums), its own code per
-// column (ColumnBind) elsewhere
+// column elsewhere
 int matvec_dot_multi(amg1d* h, const int* act, int na, const CgMultiVecs& v, const ColVecs& x, const ColVecs& y,
                      int slot) {
     Level& l0 = h->L[0];
@@ -3237,10 +3163,7 @@ int matvec_dot_multi(amg1d* h, const int* act, int na, const CgMultiVecs& v, con
         LAUNCH_CHECK();
         return slot >= 0 ? reduce_partials_multi(h, v, na, nb, slot, 0) : AMG1D_OK;
     }
-    for (int i = 0; i < na; ++i) {
-        ColumnBind cb(h, act[i]);
-        RET(op_matvec_dot(h, 0, x.v[i], y.v[i], slot));
-    }
+    for (int i = 0; i < na; ++i) RET(op_matvec_dot(h, h->multi.col[(size_t)act[i]], 0, x.v[i], y.v[i], slot));
     return AMG1D_OK;
 }
 
@@ -3251,15 +3174,18 @@ int pcg_multi_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double
     amg1d::Multi& M = h->multi;
     const int k = M.k;
     const int64_t N = l0.n * l0.m;
-    const size_t bytes = (size_t)l0.x[0].len * 8;
-    RET(pcg_multi_alloc(h, k));
+    const size_t bytes = (size_t)M.col[0].lv[0].x[0].len * 8;
+    for (int c = 0; c < k; ++c) {
+        const int rc = column_alloc(h, M.col[(size_t)c], true);
+        if (rc != AMG1D_OK) return fail(h, rc, "CG vectors of column %d of the multi-column set: %s", c, h->err.c_str());
+    }
     int act[MULTI_MAX_COLS];
     int na = k;
     for (int c = 0; c < k; ++c) {
         act[c] = c;
         iters[c] = 0;
-        auto& v = M.col[(size_t)c][0];
-        CK(cudaMemcpyAsync(M.cg[(size_t)c].x.p, v.x[v.cur].p, bytes, cudaMemcpyDeviceToDevice, h->stream));
+        auto& v = M.col[(size_t)c].lv[0];
+        CK(cudaMemcpyAsync(M.col[(size_t)c].cg.x.p, v.x[v.cur].p, bytes, cudaMemcpyDeviceToDevice, h->stream));
     }
     M.norm_valid = false;
     M.rhs_consumed = true;
@@ -3319,9 +3245,9 @@ int pcg_multi_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double
         na = keep;
     }
     for (int c = 0; c < k; ++c) {                                  // the solutions become the resident iterates
-        auto& v = M.col[(size_t)c][0];
+        auto& v = M.col[(size_t)c].lv[0];
         v.cur = 0;
-        CK(cudaMemcpyAsync(v.x[0].p, M.cg[(size_t)c].x.p, bytes, cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpyAsync(v.x[0].p, M.col[(size_t)c].cg.x.p, bytes, cudaMemcpyDeviceToDevice, h->stream));
     }
     for (int c = 0; c < k; ++c)
         if (iters[c] > 0 && !std::isfinite(res[(int64_t)c * maxiter + iters[c] - 1]))
@@ -3339,23 +3265,23 @@ int amg1d_pcg(amg1d_t* h, double* x, const double* b, int maxiter, double tol, i
     RET(check_ready(h));
     if (!x || !b || !res || !iters) return fail(h, AMG1D_ERR_ARG, "null argument");
     if (maxiter < 0) return fail(h, AMG1D_ERR_ARG, "maxiter must be >= 0");
-    RET(pcg_alloc(h));
-    RET(to_device(h, 0, b, h->L[0].b.p));
-    RET(to_device(h, 0, x, h->cg_x.p));
-    RET(pcg_run(h, maxiter, tol, nPre, nPost, alpha, iters, res));
-    return to_host(h, 0, h->cg_x.p, x);
+    RET(column_alloc(h, h->res, true));
+    RET(to_device(h, 0, b, h->res.lv[0].b.p));
+    RET(to_device(h, 0, x, h->res.cg.x.p));
+    RET(pcg_run(h, h->res, maxiter, tol, nPre, nPost, alpha, iters, res));
+    return to_host(h, 0, h->res.cg.x.p, x);
 }
 
 int amg1d_dev_pcg(amg1d_t* h, int maxiter, double tol, int nPre, int nPost, double alpha, int* iters, double* res) {
     RET(check_dev_problem(h));
     if (!res || !iters) return fail(h, AMG1D_ERR_ARG, "null argument");
     if (maxiter < 0) return fail(h, AMG1D_ERR_ARG, "maxiter must be >= 0");
-    Level& l0 = h->L[0];
-    RET(pcg_alloc(h));
-    CK(cudaMemcpyAsync(h->cg_x.p, l0.x[l0.cur].p, (size_t)l0.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
-    RET(pcg_run(h, maxiter, tol, nPre, nPost, alpha, iters, res));
-    l0.cur = 0;                                                  // the solution becomes the resident iterate
-    CK(cudaMemcpyAsync(l0.x[0].p, h->cg_x.p, (size_t)l0.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
+    Column::Vecs& v0 = h->res.lv[0];
+    RET(column_alloc(h, h->res, true));
+    CK(cudaMemcpyAsync(h->res.cg.x.p, v0.x[v0.cur].p, (size_t)v0.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
+    RET(pcg_run(h, h->res, maxiter, tol, nPre, nPost, alpha, iters, res));
+    v0.cur = 0;                                                  // the solution becomes the resident iterate
+    CK(cudaMemcpyAsync(v0.x[0].p, h->res.cg.x.p, (size_t)v0.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
     return AMG1D_OK;
 }
 
@@ -3374,7 +3300,8 @@ int amg1d_apply_smoother(amg1d_t* h, int level, double* Y, const double* B, int6
     if (!valid_level(h, level)) return fail(h, AMG1D_ERR_ARG, "level %d out of range", level);
     if (!Y || !B || n_rhs < 1) return fail(h, AMG1D_ERR_ARG, "bad arguments");
     Level& lv = h->L[level];
-    double* in = lv.x[1 - lv.cur].p;  // free ping-pong buffer as input staging
+    Column::Vecs& v = h->res.lv[(size_t)level];
+    double* in = v.x[1 - v.cur].p;  // free ping-pong buffer as input staging
     for (int64_t c = 0; c < n_rhs; ++c) {
         RET(to_device(h, level, B + c * lv.n_host, in));
         if (lv.smooth_tri)
@@ -3396,31 +3323,33 @@ int amg1d_smoother_solve(amg1d_t* h, int level, double* x, const double* b, int 
     if (!valid_level(h, level)) return fail(h, AMG1D_ERR_ARG, "level %d out of range", level);
     if (!x || !b || !res || !iters) return fail(h, AMG1D_ERR_ARG, "null argument");
     Level& lv = h->L[level];
+    Column& col = h->res;
+    Column::Vecs& v = col.lv[(size_t)level];
     invalidate_graph(h);
     if (level == 0) h->dev_problem = false;    // stages b and x in level 0's own vectors
-    lv.cur = 0;
-    RET(to_device(h, level, b, lv.b.p));
-    RET(to_device(h, level, x, lv.x[0].p));
+    v.cur = 0;
+    RET(to_device(h, level, b, v.b.p));
+    RET(to_device(h, level, x, v.x[0].p));
     DevBuf exact;
     double* d_exact = nullptr;
     if (err && u_exact) {
-        CK(exact.alloc(lv.x[0].len + 8));
+        CK(exact.alloc(v.x[0].len + 8));
         d_exact = exact.p;
         RET(to_device(h, level, u_exact, d_exact));
     }
-    int rc = op_norm(h, lv.b.p, nullptr, lv.b.len, 2);
+    int rc = op_norm(h, col, v.b.p, nullptr, v.b.len, 2);
     int it = 0;
     for (int i = 0; i < maxiter && rc == AMG1D_OK; ++i) {
-        rc = op_sweep(h, level, lv.b.p, lv.x[lv.cur].p, lv.x[1 - lv.cur].p, alpha, 0);
+        rc = op_sweep(h, level, v.b.p, v.x[v.cur].p, v.x[1 - v.cur].p, alpha, 0);
         if (rc != AMG1D_OK) break;
-        lv.cur = 1 - lv.cur;
-        rc = op_resnorm(h, level, 0);
+        v.cur = 1 - v.cur;
+        rc = op_resnorm(h, col, level, 0);
         if (rc != AMG1D_OK) break;
         if (d_exact) {
-            rc = op_norm(h, lv.x[lv.cur].p, d_exact, lv.x[0].len, 1);
+            rc = op_norm(h, col, v.x[v.cur].p, d_exact, v.x[0].len, 1);
             if (rc != AMG1D_OK) break;
         }
-        rc = read_scalars(h, 3);
+        rc = read_scalars(h, col, 3);
         if (rc != AMG1D_OK) break;
         res[i] = h->h_scal[0];
         if (err) err[i] = d_exact ? h->h_scal[1] : NAN;
@@ -3429,10 +3358,10 @@ int amg1d_smoother_solve(amg1d_t* h, int level, double* x, const double* b, int 
     }
     RET(rc);
     *iters = it;
-    rc = to_host(h, level, lv.x[lv.cur].p, x);
-    if (lv.cur != 0) {
-        CK(cudaMemcpyAsync(lv.x[0].p, lv.x[1].p, (size_t)lv.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
-        lv.cur = 0;
+    rc = to_host(h, level, v.x[v.cur].p, x);
+    if (v.cur != 0) {
+        CK(cudaMemcpyAsync(v.x[0].p, v.x[1].p, (size_t)v.x[0].len * 8, cudaMemcpyDeviceToDevice, h->stream));
+        v.cur = 0;
     }
     return rc;
 }
@@ -3442,11 +3371,11 @@ static int apply_common(amg1d_t* h, int level, double* out, const double* x, con
     if (h->nranks > 1) return fail(h, AMG1D_ERR_UNSUPPORTED, "per-level host operations are single-GPU only");
     if (!valid_level(h, level)) return fail(h, AMG1D_ERR_ARG, "level %d out of range", level);
     if (!out || !x || (mode && !b)) return fail(h, AMG1D_ERR_ARG, "null vector");
-    Level& lv = h->L[level];
+    Column::Vecs& v = h->res.lv[(size_t)level];
     invalidate_graph(h);
-    double* xin = lv.x[1 - lv.cur].p;
+    double* xin = v.x[1 - v.cur].p;
     RET(to_device(h, level, x, xin));
-    double* bin = lv.b.p;  // clobbers the level rhs: amg1d_vcycle / amg1d_solve re-upload it, the device-resident
+    double* bin = v.b.p;  // clobbers the level rhs: amg1d_vcycle / amg1d_solve re-upload it, the device-resident
     if (mode) {            // problem (level 0) is marked stale so that amg1d_dev_vcycle refuses to use it
         if (level == 0) h->dev_problem = false;
         RET(to_device(h, level, b, bin));
@@ -3469,12 +3398,12 @@ int amg1d_restrict(amg1d_t* h, int level, double* rc, const double* rf) {
     if (level < 0 || level >= h->n_levels - 1) return fail(h, AMG1D_ERR_ARG, "transfer %d out of range", level);
     if (!rc || !rf) return fail(h, AMG1D_ERR_ARG, "null vector");
     invalidate_graph(h);
-    Level& lf = h->L[level];
-    Level& lc = h->L[level + 1];
-    double* fin = lf.x[1 - lf.cur].p;
+    Column::Vecs& vf = h->res.lv[(size_t)level];
+    Column::Vecs& vc = h->res.lv[(size_t)level + 1];
+    double* fin = vf.x[1 - vf.cur].p;
     RET(to_device(h, level, rf, fin));
-    RET(op_restrict(h, level, fin, lc.b.p));
-    return to_host(h, level + 1, lc.b.p, rc);
+    RET(op_restrict(h, level, fin, vc.b.p));
+    return to_host(h, level + 1, vc.b.p, rc);
 }
 
 int amg1d_prolong(amg1d_t* h, int level, double* xf, const double* xc) {
@@ -3483,9 +3412,8 @@ int amg1d_prolong(amg1d_t* h, int level, double* xf, const double* xc) {
     if (level < 0 || level >= h->n_levels - 1) return fail(h, AMG1D_ERR_ARG, "transfer %d out of range", level);
     if (!xf || !xc) return fail(h, AMG1D_ERR_ARG, "null vector");
     invalidate_graph(h);
-    Level& lf = h->L[level];
-    Level& lc = h->L[level + 1];
-    double* cin = lc.x[1 - lc.cur].p;
+    Column::Vecs& vc = h->res.lv[(size_t)level + 1];
+    double* cin = vc.x[1 - vc.cur].p;
     RET(to_device(h, level + 1, xc, cin));
     RET(op_prolong(h, level, cin, h->scratch.p, 0));
     return to_host(h, level, h->scratch.p, xf);
@@ -3497,8 +3425,8 @@ int amg1d_coarse_solve(amg1d_t* h, double* x, const double* b) {
     if (!x || !b) return fail(h, AMG1D_ERR_ARG, "null vector");
     invalidate_graph(h);
     const int l = h->n_levels - 1;
-    Level& lv = h->L[l];
-    double* bin = lv.x[1 - lv.cur].p;
+    Column::Vecs& v = h->res.lv[(size_t)l];
+    double* bin = v.x[1 - v.cur].p;
     RET(to_device(h, l, b, bin));
     RET(op_coarse(h, bin, h->scratch.p));
     return to_host(h, l, h->scratch.p, x);
@@ -3509,12 +3437,12 @@ int amg1d_direct_solve(amg1d_t* h, int level, double* x, const double* b) {
     if (h->nranks > 1) return fail(h, AMG1D_ERR_UNSUPPORTED, "per-level host operations are single-GPU only");
     if (!valid_level(h, level)) return fail(h, AMG1D_ERR_ARG, "level %d out of range", level);
     if (!x || !b) return fail(h, AMG1D_ERR_ARG, "null vector");
-    Level& lv = h->L[level];
     if (h->direct.size() < (size_t)h->n_levels) h->direct.resize((size_t)h->n_levels);
     BcrSolver& S = h->direct[(size_t)level];
     if (!S.ready()) RET(bcr_factor(h, S, level));
     invalidate_graph(h);
-    double* bin = lv.x[1 - lv.cur].p;            // free ping-pong buffer as input staging
+    Column::Vecs& v = h->res.lv[(size_t)level];
+    double* bin = v.x[1 - v.cur].p;              // free ping-pong buffer as input staging
     RET(to_device(h, level, b, bin));
     CK(S.solve(bin, h->scratch.p, h->stream, &h->launch_counter));
     return to_host(h, level, h->scratch.p, x);
