@@ -124,6 +124,9 @@ struct Column {
     struct { DVec x, p, ap; } cg;  // level 0: CG solution, search direction, A p - allocated at the first CG call
 };
 
+// one slab vector of a halo exchange (op_halo): local element 0, owned elements, block size
+struct HaloVec { double* p; int64_t n; int m; };
+
 // An instantiated V-cycle graph, keyed by the cycle parameters and the active columns (the resident cycle: mask 1)
 struct GraphEntry {
     cudaGraphExec_t exec = nullptr;
@@ -314,6 +317,11 @@ void vec_release(amg1d* h, DVec& v) {
     vec_free(v);
 }
 
+// The peer-mapped arena (halo_p2p.cuh) holds one column, the resident problem: only its slab edges travel through peer
+// memory.  The columns of the multi-column set live in ordinary allocations and exchange their edges through NCCL.
+bool arena_column(const amg1d* h, const Column& col) { return &col == &h->res; }
+bool peer_column(const amg1d* h, const Column& col) { return h->p2p.on && arena_column(h, col); }
+
 // everything column_alloc gave col (not its scalars, which belong to their owner)
 void column_free(amg1d* h, Column& col) {
     for (auto& v : col.lv) { vec_release(h, v.x[0]); vec_release(h, v.x[1]); vec_release(h, v.b); }
@@ -323,8 +331,9 @@ void column_free(amg1d* h, Column& col) {
 }
 
 // What col still lacks: its vectors on every level this rank holds, with its reduction scratch, and with cg its level-0
-// CG vectors.  Vectors of sharded levels come from the peer-mapped arena (in the order x[0], b, x[1] its neighbours
-// expect); a proxy level holds no x[1].  A failure releases what this call took and clears the sticky CUDA error.
+// CG vectors.  The resident problem's vectors of sharded levels come from the peer-mapped arena (in the order x[0], b,
+// x[1] its neighbours expect); a proxy level holds no x[1].  A failure releases what this call took and clears the
+// sticky CUDA error.
 int column_alloc(amg1d* h, Column& col, bool cg) {
     const bool levels = col.lv.empty();
     int rc = AMG1D_OK;
@@ -334,7 +343,7 @@ int column_alloc(amg1d* h, Column& col, bool cg) {
             const Level& lv = h->L[l];
             Column::Vecs& v = col.lv[(size_t)l];
             if (!lv.present && !lv.proxy) continue;
-            const bool arena = lv.sharded && h->p2p.arena;
+            const bool arena = lv.sharded && h->p2p.arena && arena_column(h, col);
             for (DVec* d : {&v.x[0], &v.b, &v.x[1]})
                 if (rc == AMG1D_OK && (d != &v.x[1] || lv.present))
                     rc = arena ? vec_from_arena(h, *d, lv.n, lv.m) : vec_alloc(h, *d, lv.n, lv.m);
@@ -507,17 +516,15 @@ Slab make_slab(amg1d* h, int l) {
                         __FILE__, __LINE__);                                                   \
     } while (0)
 
-// Exchange ghost_depth edge elements of a slab vector with both neighbour ranks.
-// v points at local element 0; n = owned elements; m = block size.  A second vector (v2 != nullptr)
-// travels in the same NCCL group: one communication kernel instead of two (the exchanges are latency
-// bound: 4 x m doubles each way).
-int op_halo(amg1d* h, double* v, int64_t n, int m, double* v2 = nullptr, int64_t n2 = 0, int m2 = 0) {
+// Exchange ghost_depth edge elements of nv slab vectors with both neighbour ranks, all in one NCCL group: one
+// communication kernel however many vectors travel (the exchanges are latency bound: 4 x m doubles each way).
+// v[i].p points at local element 0; n = owned elements; m = block size.
+int op_halo(amg1d* h, const HaloVec* v, int nv) {
     NCK(g_nccl.GroupStart());
-    for (int k = 0; k < 2; ++k) {
-        double* p = k == 0 ? v : v2;
-        if (!p) continue;
-        const int64_t nn = k == 0 ? n : n2;
-        const int mm = k == 0 ? m : m2;
+    for (int k = 0; k < nv; ++k) {
+        double* p = v[k].p;
+        const int64_t nn = v[k].n;
+        const int mm = v[k].m;
         const int64_t cnt = (int64_t)h->ghost_depth * mm;
         if (h->rank > 0) {
             NCK(g_nccl.Send(p, cnt, ncclDouble, h->rank - 1, h->comm, h->stream));
@@ -533,42 +540,52 @@ int op_halo(amg1d* h, double* v, int64_t n, int m, double* v2 = nullptr, int64_t
     return AMG1D_OK;
 }
 
-// rank r's slab of the gather level's right-hand side -> rank 0 (which owns the whole level)
-int op_gather_rhs(amg1d* h, Column& col, int g) {
+// the same for one vector, or two (v2 != nullptr)
+int op_halo(amg1d* h, double* v, int64_t n, int m, double* v2 = nullptr, int64_t n2 = 0, int m2 = 0) {
+    const HaloVec hv[2] = {{v, n, m}, {v2, n2, m2}};
+    return op_halo(h, hv, v2 ? 2 : 1);
+}
+
+// every listed column's slab of the gather level's right-hand side -> rank 0 (which owns the whole level)
+int op_gather_rhs(amg1d* h, Column* const* cols, int nc, int g) {
     Level& lg = h->L[g];
-    double* b = col.lv[(size_t)g].b.p;
     NCK(g_nccl.GroupStart());
-    if (h->rank == 0) {
-        for (int r = 1; r < h->nranks; ++r)
-            NCK(g_nccl.Recv(b + slab_start(lg.n_glob, h->nranks, r) * lg.m,
-                            slab_size(lg.n_glob, h->nranks, r) * lg.m, ncclDouble, r, h->comm, h->stream));
-    } else {
-        NCK(g_nccl.Send(b, slab_size(lg.n_glob, h->nranks, h->rank) * lg.m, ncclDouble, 0, h->comm,
-                        h->stream));
+    for (int c = 0; c < nc; ++c) {
+        double* b = cols[c]->lv[(size_t)g].b.p;
+        if (h->rank == 0) {
+            for (int r = 1; r < h->nranks; ++r)
+                NCK(g_nccl.Recv(b + slab_start(lg.n_glob, h->nranks, r) * lg.m,
+                                slab_size(lg.n_glob, h->nranks, r) * lg.m, ncclDouble, r, h->comm, h->stream));
+        } else {
+            NCK(g_nccl.Send(b, slab_size(lg.n_glob, h->nranks, h->rank) * lg.m, ncclDouble, 0, h->comm,
+                            h->stream));
+        }
     }
     NCK(g_nccl.GroupEnd());
     h->launch_counter++;
     return AMG1D_OK;
 }
 
-// rank 0's solution of the gather level -> every rank's slab (with ghost elements)
-int op_scatter_sol(amg1d* h, Column& col, int g) {
+// rank 0's solution of the gather level -> every rank's slab (with ghost elements), for every listed column
+int op_scatter_sol(amg1d* h, Column* const* cols, int nc, int g) {
     Level& lg = h->L[g];
-    Column::Vecs& v = col.lv[(size_t)g];
     const int gd = h->ghost_depth;
     NCK(g_nccl.GroupStart());
-    if (h->rank == 0) {
-        const double* x = v.x[v.cur].p;
-        for (int r = 1; r < h->nranks; ++r) {
-            const int64_t e0 = slab_start(lg.n_glob, h->nranks, r) - gd;
-            const int64_t e1 = slab_start(lg.n_glob, h->nranks, r) + slab_size(lg.n_glob, h->nranks, r) +
-                               (r < h->nranks - 1 ? gd : 0);
-            NCK(g_nccl.Send(x + e0 * lg.m, (e1 - e0) * lg.m, ncclDouble, r, h->comm, h->stream));
+    for (int c = 0; c < nc; ++c) {
+        Column::Vecs& v = cols[c]->lv[(size_t)g];
+        if (h->rank == 0) {
+            const double* x = v.x[v.cur].p;
+            for (int r = 1; r < h->nranks; ++r) {
+                const int64_t e0 = slab_start(lg.n_glob, h->nranks, r) - gd;
+                const int64_t e1 = slab_start(lg.n_glob, h->nranks, r) + slab_size(lg.n_glob, h->nranks, r) +
+                                   (r < h->nranks - 1 ? gd : 0);
+                NCK(g_nccl.Send(x + e0 * lg.m, (e1 - e0) * lg.m, ncclDouble, r, h->comm, h->stream));
+            }
+        } else {
+            const int64_t cnt = (slab_size(lg.n_glob, h->nranks, h->rank) + gd +
+                                 (h->rank < h->nranks - 1 ? gd : 0)) * lg.m;
+            NCK(g_nccl.Recv(v.x[0].p - (int64_t)gd * lg.m, cnt, ncclDouble, 0, h->comm, h->stream));
         }
-    } else {
-        const int64_t cnt = (slab_size(lg.n_glob, h->nranks, h->rank) + gd +
-                             (h->rank < h->nranks - 1 ? gd : 0)) * lg.m;
-        NCK(g_nccl.Recv(v.x[0].p - (int64_t)gd * lg.m, cnt, ncclDouble, 0, h->comm, h->stream));
     }
     NCK(g_nccl.GroupEnd());
     h->launch_counter++;
@@ -819,9 +836,10 @@ int op_p2p_push(amg1d* h, Column&, int, int, int, int = -1, int = 0) { return fa
 int op_p2p_begin_cycle(amg1d* h) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 HaloLeg make_halo_leg(amg1d*, int, bool, int) { HaloLeg hl; memset(&hl, 0, sizeof hl); return hl; }
 int op_p2p_wait_for(amg1d* h, const HaloLeg&) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
+int op_halo(amg1d* h, const HaloVec*, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 int op_halo(amg1d* h, double*, int64_t, int, double* = nullptr, int64_t = 0, int = 0) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
-int op_gather_rhs(amg1d* h, Column&, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
-int op_scatter_sol(amg1d* h, Column&, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
+int op_gather_rhs(amg1d* h, Column* const*, int, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
+int op_scatter_sol(amg1d* h, Column* const*, int, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 int op_allreduce_norm(amg1d* h, Column&, int, bool) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 int op_allreduce_max(amg1d* h, double*, int) { return fail(h, AMG1D_ERR_UNSUPPORTED, "built without NCCL"); }
 #endif
@@ -956,10 +974,11 @@ int op_dot(amg1d* h, Column& col, const double* a, const double* c, int64_t n, i
     return op_reduce_partials(h, col, nb, slot, false);
 }
 
-// y = A x on level l (x must carry valid ghost elements), col's slot <- x . y when slot >= 0
-int op_matvec_dot(amg1d* h, Column& col, int l, double* x, double* y, int slot) {
+// y = A x on level l, col's slot <- x . y when slot >= 0; a sharded level first exchanges x's ghosts unless the caller
+// did (halo = false)
+int op_matvec_dot(amg1d* h, Column& col, int l, double* x, double* y, int slot, bool halo = true) {
     Level& lv = h->L[l];
-    if (lv.sharded) RET(op_halo(h, x, lv.n, lv.m));
+    if (lv.sharded && halo) RET(op_halo(h, x, lv.n, lv.m));
     int nb = 0;
     if (h->opt_fused && fused_matvec_dot(lv.md, lv.mat, x, y, lv.n, slot >= 0 ? col.partial : nullptr,
                                          h->partial_cap, &nb, h->stream)) {
@@ -983,23 +1002,24 @@ int prof_mark(amg1d* h, int level, int leg) {
 
 // ---- the V-cycle (src/solvers.jl:19-50) ------------------------------------------------------------
 // Down leg of level l: nPre sweeps (zero guess on l > 0), residual, restriction into level l+1's rhs.
-int leg_down(amg1d* h, Column& col, int l, int nPre, double alpha, bool zero0) {
+// ghosts_in: the caller already exchanged the ghosts of the incoming iterate (the multi-column cycle, for all columns).
+int leg_down(amg1d* h, Column& col, int l, int nPre, double alpha, bool zero0, bool ghosts_in = false) {
     Level& lv = h->L[l];
     Transfer& t = h->T[l];
     Level& lc = h->L[l + 1];
     Column::Vecs& v = col.lv[(size_t)l];
     Column::Vecs& vc = col.lv[(size_t)l + 1];
     const bool zero = l > 0 || zero0;         // zero0: level 0 starts from a zero guess too (ldiv!, PCG)
+    const bool p2p = peer_column(h, col) && lv.sharded;
     if (zero) v.cur = 0;
     RET(prof_mark(h, l, 0));
     // ghosts of the incoming iterate (peer-memory mode: they arrived with the last up leg's push, or with
     // amg1d_dev_set_problem's exchange)
-    if (lv.sharded && !zero && !h->p2p.on) RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m));
+    if (lv.sharded && !zero && !p2p && !ghosts_in) RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m));
     // fused: nPre sweeps + residual + restriction in one pass over the operator
     if (h->opt_fused && t.fusable && !lv.smooth_tri) {
         const int ob = zero ? 0 : 1 - v.cur;
         cudaError_t le = cudaSuccess;
-        const bool p2p = h->p2p.on && lv.sharded;
         // peer-memory exchange done by the leg itself: wait for the rhs ghosts, push the pre-smoothed edges + coarse rhs
         const HaloLeg hl = p2p ? make_halo_leg(h, l, true, ob) : HaloLeg();
         int fr = fused_down(lv.md, t.mc, make_map_closed(t), nPre, zero, lv.mat, make_pat(h, l), v.b.p, v.x[v.cur].p,
@@ -1059,7 +1079,7 @@ int leg_up(amg1d* h, Column& col, int l, int nPost, double alpha, bool fuse_norm
     if (h->opt_fused && t.fusable && !lv.smooth_tri) {
         int nb = 0;
         cudaError_t le = cudaSuccess;
-        const bool p2p = h->p2p.on && lv.sharded;
+        const bool p2p = peer_column(h, col) && lv.sharded;
         // Level 0's edges are pushed from inside the kernel only if the leg writes buffer 0, where the next cycle
         // reads them (a zero-guess cycle ends in buffer 1 and is copied over: enqueue_vcycle pushes after that copy)
         const int ob = 1 - v.cur;
@@ -1100,21 +1120,31 @@ int leg_up(amg1d* h, Column& col, int l, int nPost, double alpha, bool fuse_norm
     return prof_mark(h, l, 1);
 }
 
+// a sharded cycle's legs read at most ghost_depth elements beyond the slab
+int check_ghost_depth(amg1d* h, int nPre, int nPost) {
+    if (h->gather_level < 0) return AMG1D_OK;
+    int need = std::max(nPre, nPost) + 1;         // one halo exchange serves a whole fused leg
+    for (int l = 0; l < h->n_levels - 1; ++l)
+        if (h->L[l].sharded) need = std::max(need, std::max(nPre, nPost) + 1 + h->T[l].reach);
+    if (need > h->ghost_depth)
+        return fail(h, AMG1D_ERR_ARG, "nPre / nPost need ghost_depth >= %d (option \"ghost_depth\", "
+                    "before the first level is set)", need);
+    return AMG1D_OK;
+}
+
+// levels [ts, nl) run inside the single-CTA tail kernel (rank 0 holds them; ts > gather level)
+int tail_begin(const amg1d* h) {
+    return (h->tail_start > 0 && h->L[h->tail_start].present) ? h->tail_start : h->n_levels;
+}
+
 int enqueue_vcycle(amg1d* h, Column& col, int nPre, int nPost, double alpha, bool want_norm, bool zero0) {
     const int nl = h->n_levels;
     const int g = h->gather_level;          // -1 on a single GPU: every level is local
     bool norm_done = false;
-    if (g >= 0) {
-        int need = std::max(nPre, nPost) + 1;         // one halo exchange serves a whole fused leg
-        for (int l = 0; l < nl - 1; ++l)
-            if (h->L[l].sharded) need = std::max(need, std::max(nPre, nPost) + 1 + h->T[l].reach);
-        if (need > h->ghost_depth)
-            return fail(h, AMG1D_ERR_ARG, "nPre / nPost need ghost_depth >= %d (option \"ghost_depth\", "
-                        "before the first level is set)", need);
-    }
-    // levels [ts, nl) run inside the single-CTA tail kernel (rank 0 holds them; ts > gather level)
-    const int ts = (h->tail_start > 0 && h->L[h->tail_start].present) ? h->tail_start : nl;
-    const bool p2p = g >= 0 && h->p2p.on;       // slab edges through peer memory (halo_p2p.cuh) instead of NCCL
+    RET(check_ghost_depth(h, nPre, nPost));
+    const int ts = tail_begin(h);
+    const bool p2p = g >= 0 && peer_column(h, col);   // slab edges through peer memory (halo_p2p.cuh) instead of NCCL
+    Column* self = &col;
     bool u0_pushed = false;
     if (p2p) RET(op_p2p_begin_cycle(h));
     // ---- down ----
@@ -1127,11 +1157,11 @@ int enqueue_vcycle(amg1d* h, Column& col, int nPre, int nPost, double alpha, boo
             Column::Vecs& v = col.lv[(size_t)l];
             // ghosts of the pre-smoothed iterate (for the up leg) and of the coarse rhs, in one exchange
             if (p2p) {                    // the leg exchanged its edges itself (leg_down)
-                if (!lc.sharded) RET(op_gather_rhs(h, col, l + 1));        // slabs -> rank 0
+                if (!lc.sharded) RET(op_gather_rhs(h, &self, 1, l + 1));   // slabs -> rank 0
             } else if (lc.sharded) RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m, col.lv[(size_t)l + 1].b.p, lc.n, lc.m));
             else {
                 RET(op_halo(h, v.x[v.cur].p, lv.n, lv.m));
-                RET(op_gather_rhs(h, col, l + 1));                         // slabs -> rank 0
+                RET(op_gather_rhs(h, &self, 1, l + 1));                    // slabs -> rank 0
             }
         }
     }
@@ -1153,7 +1183,7 @@ int enqueue_vcycle(amg1d* h, Column& col, int nPre, int nPost, double alpha, boo
         Level& lc = h->L[l + 1];
         Column::Vecs& v = col.lv[(size_t)l];
         if (!lv.present) continue;
-        if (lv.sharded && !lc.sharded) RET(op_scatter_sol(h, col, l + 1));   // rank 0 -> slabs (+ ghosts)
+        if (lv.sharded && !lc.sharded) RET(op_scatter_sol(h, &self, 1, l + 1));   // rank 0 -> slabs (+ ghosts)
         bool pushed = false;
         RET(leg_up(h, col, l, nPost, alpha, want_norm && l == 0, &norm_done, &pushed));
         if (p2p && lv.sharded) {
@@ -1520,6 +1550,23 @@ int multi_alloc(amg1d* h, int k) {
     return AMG1D_OK;
 }
 
+// Sharded handles: the outcome rc of a local allocation, agreed over all ranks.  Rank 0 also holds the levels below the
+// gather level, so an allocation can fail there alone; the other ranks must then fail too instead of posting exchanges
+// that rank 0 never matches.  Device slot 63 of the resident scalars carries the flag.
+int agree_alloc(amg1d* h, int rc) {
+    if (h->nranks == 1) return rc;
+    const std::string err = h->err;
+    double flag = rc != AMG1D_OK ? 1.0 : 0.0;
+    double* d = h->res.scal + 63;
+    CK(cudaMemcpyAsync(d, &flag, 8, cudaMemcpyHostToDevice, h->stream));
+    RET(op_allreduce_max(h, d, 1));
+    CK(cudaMemcpyAsync(&flag, d, 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (rc != AMG1D_OK) { h->err = err; return rc; }
+    if (flag != 0.0) return fail(h, AMG1D_ERR_NOMEM, "the multi-column storage did not fit on another rank");
+    return AMG1D_OK;
+}
+
 // descriptors of the single-CTA tail for every column (before capture)
 int multi_sync_tail(amg1d* h) {
     amg1d::Multi& M = h->multi;
@@ -1568,8 +1615,8 @@ int leg_down_multi(amg1d* h, int l, const int* act, int na, int nPre, double alp
         RET(prof_mark(h, l, 0));
         cudaError_t le = cudaSuccess;
         const int fr = fused_down_multi(lv.md, t.mc, make_map_closed(t), nPre, zero, lv.mat, make_pat(h, l), mc, na,
-                                        tp0(t), tp1(t), lv.n, alpha, make_slab(h, l), h->stream, h->opt_pdl != 0, &le,
-                                        leg_rec(h, lv, t.mc));
+                                        tp0(t), tp1(t), lv.n, lv.n + (lv.gr ? t.cover_extra : 0), alpha,
+                                        make_slab(h, l), h->stream, h->opt_pdl != 0, &le, leg_rec(h, lv, t.mc));
         if (fr == FUSED_ERR) return fail(h, AMG1D_ERR_CUDA, "f_down_multi launch failed on level %d: %s", l, cudaGetErrorString(le));
         if (fr == FUSED_OK) {
             for (int i = 0; i < na; ++i) M.col[(size_t)act[i]].lv[(size_t)l].cur = ob[i];
@@ -1579,7 +1626,7 @@ int leg_down_multi(amg1d* h, int l, const int* act, int na, int nPre, double alp
         }
         RET(prof_unmark(h, l, 0));
     }
-    for (int i = 0; i < na; ++i) RET(leg_down(h, M.col[(size_t)act[i]], l, nPre, alpha, zero0));
+    for (int i = 0; i < na; ++i) RET(leg_down(h, M.col[(size_t)act[i]], l, nPre, alpha, zero0, true));
     return AMG1D_OK;
 }
 
@@ -1628,14 +1675,44 @@ int leg_up_multi(amg1d* h, int l, const int* act, int na, int nPost, double alph
     return AMG1D_OK;
 }
 
-// enqueue_vcycle for the active columns act[0..na) of the multi-column set (single GPU)
+// the ghosts of level l's current iterate of every active column - and with coarse_rhs those of level l + 1's
+// right-hand side - in one exchange
+int halo_multi(amg1d* h, const int* act, int na, int l, bool coarse_rhs) {
+    HaloVec hv[2 * MULTI_MAX_COLS];
+    int nv = 0;
+    const Level& lv = h->L[l];
+    for (int i = 0; i < na; ++i) {
+        Column& col = h->multi.col[(size_t)act[i]];
+        Column::Vecs& v = col.lv[(size_t)l];
+        hv[nv++] = {v.x[v.cur].p, lv.n, lv.m};
+        if (coarse_rhs) hv[nv++] = {col.lv[(size_t)l + 1].b.p, h->L[l + 1].n, h->L[l + 1].m};
+    }
+    return op_halo(h, hv, nv);
+}
+
+// enqueue_vcycle for the active columns act[0..na) of the multi-column set.  On a sharded handle it follows the
+// NCCL schedule of enqueue_vcycle, each exchange point one NCCL group for all active columns.
 int enqueue_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, double alpha, bool want_norm,
                          bool zero0) {
     const int nl = h->n_levels;
-    const int ts = h->tail_start > 0 ? h->tail_start : nl;
+    RET(check_ghost_depth(h, nPre, nPost));
+    const int ts = tail_begin(h);
     amg1d::Multi& M = h->multi;
+    Column* cols[MULTI_MAX_COLS];
+    for (int i = 0; i < na; ++i) cols[i] = &M.col[(size_t)act[i]];
     bool done[MULTI_MAX_COLS] = {};
-    for (int l = 0; l < nl - 1 && l < ts; ++l) RET(leg_down_multi(h, l, act, na, nPre, alpha, zero0));
+    if (h->L[0].sharded && !zero0) RET(halo_multi(h, act, na, 0, false));     // ghosts of the incoming iterates
+    for (int l = 0; l < nl - 1 && l < ts; ++l) {
+        const Level& lv = h->L[l];
+        if (!lv.present) break;                       // ranks > 0 stop at the gather level
+        RET(leg_down_multi(h, l, act, na, nPre, alpha, zero0));
+        if (lv.sharded) {
+            // ghosts of the pre-smoothed iterates (for the up leg) and of the coarse right-hand sides, or the gather
+            const bool lc_sharded = h->L[l + 1].sharded;
+            RET(halo_multi(h, act, na, l, lc_sharded));
+            if (!lc_sharded) RET(op_gather_rhs(h, cols, na, l + 1));
+        }
+    }
     if (ts < nl) {
         for (int i = 0; i < na; ++i) {
             for (int l = ts; l < nl; ++l) M.col[(size_t)act[i]].lv[(size_t)l].cur = 0;
@@ -1644,15 +1721,20 @@ int enqueue_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, 
             if (te != cudaSuccess) return fail(h, AMG1D_ERR_CUDA, "f_tail launch failed: %s", cudaGetErrorString(te));
             h->launch_counter++;
         }
-    } else {
+    } else if (h->L[nl - 1].present) {
         for (int i = 0; i < na; ++i) {
             Column::Vecs& v = M.col[(size_t)act[i]].lv[(size_t)nl - 1];
             if (nl > 1 || zero0) v.cur = 0;
             RET(op_coarse(h, v.b.p, v.x[v.cur].p));
         }
     }
-    for (int l = std::min(nl - 2, ts - 1); l >= 0; --l)
+    for (int l = std::min(nl - 2, ts - 1); l >= 0; --l) {
+        const Level& lv = h->L[l];
+        if (!lv.present) continue;
+        if (lv.sharded && !h->L[l + 1].sharded) RET(op_scatter_sol(h, cols, na, l + 1));   // rank 0 -> slabs (+ ghosts)
         RET(leg_up_multi(h, l, act, na, nPost, alpha, want_norm && l == 0, done));
+        if (lv.sharded && l > 0) RET(halo_multi(h, act, na, l, false));       // for level l-1's prolongation
+    }
     for (int i = 0; i < na; ++i) {
         Column& col = M.col[(size_t)act[i]];
         auto& v = col.lv[0];
@@ -1684,9 +1766,6 @@ int run_vcycle_multi(amg1d* h, const int* act, int na, int nPre, int nPost, doub
 // need_rhs: the call reads the set's right-hand sides, which amg1d_dev_pcg_multi consumes
 int check_multi(amg1d* h, bool need_set, bool need_rhs = true) {
     RET(check_ready(h));
-    if (h->nranks > 1)
-        return fail(h, AMG1D_ERR_UNSUPPORTED, "multi-column problems run on a single GPU (this handle has %d ranks)",
-                    h->nranks);
     if (need_set && h->multi.k == 0)
         return fail(h, AMG1D_ERR_STATE, "no multi-column problem set (amg1d_dev_set_problems / amg1d_dev_fill_rhs_random_multi)");
     if (need_set && need_rhs && h->multi.rhs_consumed)
@@ -1698,6 +1777,19 @@ int check_multi(amg1d* h, bool need_set, bool need_rhs = true) {
 int check_cols(amg1d* h, int k) {
     if (k < 1 || k > MULTI_MAX_COLS) return fail(h, AMG1D_ERR_ARG, "column count %d outside [1, %d]", k, MULTI_MAX_COLS);
     return AMG1D_OK;
+}
+
+// a sharded level 0: the ghosts of the first k columns' right-hand sides and initial iterates, in one exchange
+int multi_halo_problems(amg1d* h, int k) {
+    const Level& l0 = h->L[0];
+    if (!l0.sharded) return AMG1D_OK;
+    HaloVec hv[2 * MULTI_MAX_COLS];
+    for (int c = 0; c < k; ++c) {
+        auto& v = h->multi.col[(size_t)c].lv[0];
+        hv[2 * c] = {v.b.p, l0.n, l0.m};
+        hv[2 * c + 1] = {v.x[0].p, l0.n, l0.m};
+    }
+    return op_halo(h, hv, 2 * k);
 }
 
 int read_multi_scalars(amg1d* h) {
@@ -2797,7 +2889,7 @@ int amg1d_dev_set_problems(amg1d_t* h, int k, const double* X0, const double* B)
     RET(check_multi(h, false));
     RET(check_cols(h, k));
     if (!B) return fail(h, AMG1D_ERR_ARG, "null B");
-    RET(multi_alloc(h, k));
+    RET(agree_alloc(h, multi_alloc(h, k)));
     amg1d::Multi& M = h->multi;
     const int64_t nh = h->L[0].n_host;
     M.k = 0;
@@ -2809,6 +2901,7 @@ int amg1d_dev_set_problems(amg1d_t* h, int k, const double* X0, const double* B)
         if (X0) RET(to_device(h, 0, X0 + c * nh, v.x[0].p));
         else CK(cudaMemsetAsync(v.x[0].p, 0, (size_t)v.x[0].len * 8, h->stream));
     }
+    RET(multi_halo_problems(h, k));
     M.k = k;
     M.rhs_consumed = false;
     return AMG1D_OK;
@@ -2819,7 +2912,7 @@ int amg1d_dev_fill_rhs_random_multi(amg1d_t* h, int k, uint64_t seed) {
     RET(check_cols(h, k));
     Level& l0 = h->L[0];
     if (l0.perm) return fail(h, AMG1D_ERR_UNSUPPORTED, "random rhs only for unpermuted (DG) fine levels");
-    RET(multi_alloc(h, k));
+    RET(agree_alloc(h, multi_alloc(h, k)));
     amg1d::Multi& M = h->multi;
     M.norm_valid = false;
     for (int c = 0; c < k; ++c) {
@@ -2829,6 +2922,7 @@ int amg1d_dev_fill_rhs_random_multi(amg1d_t* h, int k, uint64_t seed) {
         v.cur = 0;
         CK(cudaMemsetAsync(v.x[0].p, 0, (size_t)v.x[0].len * 8, h->stream));
     }
+    RET(multi_halo_problems(h, k));
     M.k = k;
     M.rhs_consumed = false;
     return AMG1D_OK;
@@ -3128,8 +3222,10 @@ struct CgMultiVecs {
     }
 };
 
-// op_reduce_partials of every active column in one launch per stage
-int reduce_partials_multi(amg1d* h, const CgMultiVecs& v, int na, int64_t np, int slot, int take_sqrt) {
+// op_reduce_partials of every active column in one launch per stage.  Sharded: the per-column all-reduce of
+// op_reduce_partials follows (count 1, square root after the sum), so that each column's sum has its bits.
+int reduce_partials_multi(amg1d* h, const int* act, const CgMultiVecs& v, int na, int64_t np, int slot,
+                          int take_sqrt) {
     ColVecs src = v.part;
     if (np > 8192) {
         ColVecs st2 = {};
@@ -3139,18 +3235,26 @@ int reduce_partials_multi(amg1d* h, const CgMultiVecs& v, int na, int64_t np, in
         src = st2;
         np = 256;
     }
-    k_reduce_final_multi<<<dim3(1, na), AMG1D_RED_THREADS, 0, h->stream>>>(src, (int)np, v.scal, slot, take_sqrt);
+    k_reduce_final_multi<<<dim3(1, na), AMG1D_RED_THREADS, 0, h->stream>>>(src, (int)np, v.scal, slot,
+                                                                           h->nranks > 1 ? 0 : take_sqrt);
     h->launch_counter++;
     LAUNCH_CHECK();
+    if (h->nranks > 1)
+        for (int i = 0; i < na; ++i) RET(op_allreduce_norm(h, h->multi.col[(size_t)act[i]], slot, take_sqrt != 0));
     return AMG1D_OK;
 }
 
 // op_matvec_dot(h, col, 0, x_c, y_c, slot) for every active column: one launch that reads level 0's operator once where
 // op_matvec_dot would take the fused kernel (the same predicate, hence the same partial sums), its own code per
-// column elsewhere
+// column elsewhere.  A sharded level 0 first exchanges the ghosts of every x_c in one group.
 int matvec_dot_multi(amg1d* h, const int* act, int na, const CgMultiVecs& v, const ColVecs& x, const ColVecs& y,
                      int slot) {
     Level& l0 = h->L[0];
+    if (l0.sharded) {
+        HaloVec hv[MULTI_MAX_COLS];
+        for (int i = 0; i < na; ++i) hv[i] = {x.v[i], l0.n, l0.m};
+        RET(op_halo(h, hv, na));
+    }
     MatvecCols mc = {};
     for (int i = 0; i < na; ++i) {
         mc.x[i] = x.v[i];
@@ -3161,9 +3265,9 @@ int matvec_dot_multi(amg1d* h, const int* act, int na, const CgMultiVecs& v, con
     if (h->opt_fused && fused_matvec_dot_multi(l0.md, l0.mat, mc, na, l0.n, h->partial_cap, &nb, h->stream)) {
         h->launch_counter++;
         LAUNCH_CHECK();
-        return slot >= 0 ? reduce_partials_multi(h, v, na, nb, slot, 0) : AMG1D_OK;
+        return slot >= 0 ? reduce_partials_multi(h, act, v, na, nb, slot, 0) : AMG1D_OK;
     }
-    for (int i = 0; i < na; ++i) RET(op_matvec_dot(h, h->multi.col[(size_t)act[i]], 0, x.v[i], y.v[i], slot));
+    for (int i = 0; i < na; ++i) RET(op_matvec_dot(h, h->multi.col[(size_t)act[i]], 0, x.v[i], y.v[i], slot, false));
     return AMG1D_OK;
 }
 
@@ -3175,10 +3279,12 @@ int pcg_multi_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double
     const int k = M.k;
     const int64_t N = l0.n * l0.m;
     const size_t bytes = (size_t)M.col[0].lv[0].x[0].len * 8;
-    for (int c = 0; c < k; ++c) {
-        const int rc = column_alloc(h, M.col[(size_t)c], true);
-        if (rc != AMG1D_OK) return fail(h, rc, "CG vectors of column %d of the multi-column set: %s", c, h->err.c_str());
+    int arc = AMG1D_OK;
+    for (int c = 0; c < k && arc == AMG1D_OK; ++c) {
+        arc = column_alloc(h, M.col[(size_t)c], true);
+        if (arc != AMG1D_OK) fail(h, arc, "CG vectors of column %d of the multi-column set: %s", c, h->err.c_str());
     }
+    RET(agree_alloc(h, arc));
     int act[MULTI_MAX_COLS];
     int na = k;
     for (int c = 0; c < k; ++c) {
@@ -3190,19 +3296,19 @@ int pcg_multi_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double
     M.norm_valid = false;
     M.rhs_consumed = true;
     const int nbv = (int)std::max<int64_t>(1, std::min<int64_t>(AMG1D_RED_BLOCKS, (N + AMG1D_RED_THREADS - 1) / AMG1D_RED_THREADS));
-    const dim3 gv(nbv, na), gs(1, na);
+    const dim3 gv(nbv, na);
     {
         const CgMultiVecs v(h, act, na);
         k_sqdiff_partial_multi<<<gv, AMG1D_RED_THREADS, 0, h->stream>>>(v.R, N, v.part);           // ||b||
-        k_reduce_final_multi<<<gs, AMG1D_RED_THREADS, 0, h->stream>>>(v.part, nbv, v.scal, CG_NB, 1);
-        h->launch_counter += 2;
+        h->launch_counter++;
         LAUNCH_CHECK();
+        RET(reduce_partials_multi(h, act, v, na, nbv, CG_NB, 1));
         RET(matvec_dot_multi(h, act, na, v, v.X, v.AP, -1));                                       // r = b - A x0
         k_axpy_multi<<<gv, AMG1D_RED_THREADS, 0, h->stream>>>(v.R, v.AP, N, -1.0);
         k_sqdiff_partial_multi<<<gv, AMG1D_RED_THREADS, 0, h->stream>>>(v.R, N, v.part);
-        k_reduce_final_multi<<<gs, AMG1D_RED_THREADS, 0, h->stream>>>(v.part, nbv, v.scal, CG_RES, 1);
-        h->launch_counter += 3;
+        h->launch_counter += 2;
         LAUNCH_CHECK();
+        RET(reduce_partials_multi(h, act, v, na, nbv, CG_RES, 1));
     }
     RET(read_multi_scalars(h));
     na = 0;
@@ -3213,7 +3319,13 @@ int pcg_multi_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double
         if (!(s[CG_NB] == 0.0 || s[CG_RES] <= tol * s[CG_NB])) act[na++] = c;   // pcg_run's initial-residual test
     }
     for (int i = 0; i < maxiter && na > 0; ++i) {
-        // z = M^-1 r: one multi-column V-cycle from a zero guess with right-hand sides r (already in place)
+        // z = M^-1 r: one multi-column V-cycle from a zero guess with right-hand sides r (already in place; a sharded
+        // level 0 first exchanges their ghosts, which the legs read)
+        if (l0.sharded) {
+            HaloVec hv[MULTI_MAX_COLS];
+            for (int j = 0; j < na; ++j) hv[j] = {M.col[(size_t)act[j]].lv[0].b.p, l0.n, l0.m};
+            RET(op_halo(h, hv, na));
+        }
         RET(run_vcycle_multi(h, act, na, nPre, nPost, alpha, false, true));
         const int64_t c0 = h->launch_counter;
         const CgMultiVecs v(h, act, na);
@@ -3221,7 +3333,7 @@ int pcg_multi_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double
         k_dot_partial_multi<<<g, AMG1D_RED_THREADS, 0, h->stream>>>(v.R, v.Z, N, v.part);
         h->launch_counter++;
         LAUNCH_CHECK();
-        RET(reduce_partials_multi(h, v, na, nbv, i == 0 ? CG_RZ : CG_RZ_NEW, 0));
+        RET(reduce_partials_multi(h, act, v, na, nbv, i == 0 ? CG_RZ : CG_RZ_NEW, 0));
         if (i > 0) { k_cg_beta_multi<<<1, na, 0, h->stream>>>(v.scal); h->launch_counter++; }
         k_cg_direction_multi<<<g, AMG1D_RED_THREADS, 0, h->stream>>>(v.P, v.Z, N, v.scal, i == 0 ? 1 : 0);
         h->launch_counter++;
@@ -3231,7 +3343,7 @@ int pcg_multi_run(amg1d* h, int maxiter, double tol, int nPre, int nPost, double
         k_cg_update_multi<<<g, AMG1D_RED_THREADS, 0, h->stream>>>(v.X, v.R, v.P, v.AP, N, v.scal, v.part);
         h->launch_counter += 2;
         LAUNCH_CHECK();
-        RET(reduce_partials_multi(h, v, na, nbv, CG_RES, 1));                                  // ||r||_2
+        RET(reduce_partials_multi(h, act, v, na, nbv, CG_RES, 1));                             // ||r||_2
         M.pcg_launches = h->launch_counter - c0;
         RET(read_multi_scalars(h));
         int keep = 0;
@@ -3587,7 +3699,7 @@ int64_t amg1d_get_info(amg1d_t* h, const char* key) {
     if (!strcmp(key, "multi_pcg_launches_per_iteration")) return h->multi.pcg_launches;
     if (!strncmp(key, "multi_legs:", 11)) {         // 1: the multi-column cycle reads this level's operator once for all
         const int l = atoi(key + 11);               //    columns (fused multi-column legs), 0: once per column
-        if (!valid_level(h, l) || !h->finalized || h->nranks > 1 || l + 1 >= h->n_levels) return 0;
+        if (!valid_level(h, l) || !h->finalized || !h->L[l].present || l + 1 >= h->n_levels) return 0;
         if (h->tail_start > 0 && l >= h->tail_start) return 0;
         return multi_leg_level(h, l) ? 1 : 0;
     }

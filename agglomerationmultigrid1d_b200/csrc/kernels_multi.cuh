@@ -14,7 +14,8 @@
 // Per column the arithmetic, its order and the window partition (fused_window) are those of the single-column leg, so
 // every column's iterate, coarse right-hand side and per-window ||b - A x||^2 partial sums are bit-identical to a
 // single-column cycle on that column.  Between columns the CTA synchronises: the exchange buffers restart at buf = 0
-// and the restriction buffer rs is reused.  Single GPU only (no slab exchange).
+// and the restriction buffer rs is reused.  On a slab-sharded level the kernels read the ghost windows (Slab) as the
+// single-column legs do; the slab edges travel between launches (NCCL, amg1d.cu), never from inside these kernels.
 //
 // Algorithmic bytes per element and column, k columns (FP64; Kop = doubles of the level's structure class, layout.cuh;
 // coarse block size MC, ratio R; rec: the inverse is not read):
@@ -163,12 +164,15 @@ inline bool fused_multi_available(const MatDesc& d, int mc) {
     }
 }
 
+// n_cover as for fused_down: the local elements whose coarse parents this rank gathers (past n on a slab whose right
+// neighbour's first children own coarse elements of this rank - two-parent transfers).
 inline int fused_down_multi(const MatDesc& d, int mc, const TransferMap& tm, int nsweep, bool zero, const double* mat,
                             const PatOp& po, const MultiCols& cols, int k, const double* P0, const double* P1, int64_t n,
-                            double alpha, const Slab& sl, cudaStream_t st, bool pdl, cudaError_t* err, int rec) {
+                            int64_t n_cover, double alpha, const Slab& sl, cudaStream_t st, bool pdl, cudaError_t* err,
+                            int rec) {
     const WinIdx w = fused_window(nsweep, tm, P1 != nullptr || tm.shift != 0 || tm.base != 0, sl);
     if (w.out < tm.ratio || w.out < FUSED_B / 2 || !fast_tier_ok(d)) return FUSED_NA;
-    const unsigned grid = (unsigned)((n + w.out - 1) / w.out);
+    const unsigned grid = (unsigned)((n_cover + w.out - 1) / w.out);
     if (multi_dv_form(d, mc, po, rec)) {
 #define DV(MM, MCC, SS)                                                                                               \
         if (d.m == MM && mc == MCC && d.st == SS) {                                                                   \

@@ -318,7 +318,8 @@ class DeviceHierarchy:
                              f"got {X.shape}")
 
     def dev_set_problems(self, X0, B):
-        """Upload k = B.shape[1] right-hand sides (and initial guesses X0, None = 0), each of shape (n_dof, k)."""
+        """Upload k = B.shape[1] right-hand sides (and initial guesses X0, None = 0), each of shape (n_dof, k).  On a
+        slab-sharded handle (dist=...) n_dof is this rank's slab (local_dofs), and every rank makes the same calls."""
         B = np.asfortranarray(B, dtype=np.float64)
         self._check_cols(B)
         if X0 is not None:

@@ -33,7 +33,8 @@ def multigrid_v_cycle(H, x0, b, nPre=3, nPost=3, alpha=2.0 / 3.0):
 
 def ldiv(*args):
     """``ldiv!(H, b)``: b <- one V-cycle from a zero guess; ``ldiv!(y, H, b)``: y <- the same.  A 2-D b (n_dof x k,
-    any k) is ``ldiv!(Y, H, B)``: every column as by the 1-D call, up to 8 columns per V-cycle."""
+    any k) is ``ldiv!(Y, H, B)``: every column as by the 1-D call, up to 8 columns per V-cycle.  On a slab-sharded
+    hierarchy b / y are this rank's slabs, as for the 1-D call."""
     if len(args) == 2:
         H, b = args
         out = b
@@ -65,7 +66,8 @@ def pcg(H, x0, b, maxiter, tol, nPre=3, nPost=3, alpha=2.0 / 3.0):
     reference itself ships no driver.  Returns (x, iter, res) with res[i] = ||r_i||_2 and the stop rule of
     ``multigrid`` (res < tol ||b||).  A 2-D b (n_dof x k, any k; x0 of the same shape) runs every column as
     the 1-D call would, up to 8 columns at a time through the multi-column set, and returns (X, iters, res) with
-    iters a list and res a list of per-column histories."""
+    iters a list and res a list of per-column histories.  On a slab-sharded hierarchy x0 / b are this rank's
+    slabs, as for the 1-D call."""
     dev = _device_of(H)
     if np.ndim(b) == 2:
         B = np.asarray(b, dtype=np.float64)

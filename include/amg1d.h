@@ -266,11 +266,16 @@ int amg1d_dev_get_solution(amg1d_t* h, double* x);                 /* device -> 
  * methods, time steppers and multi-load problems apply to many vectors.  One V-cycle serves all columns: on levels
  * with fused legs (amg1d_get_info("multi_legs:<level>") = 1) each leg reads the level's operator once for all columns;
  * the other levels, the coarse tail and the coarse solve run once per column.  Every column's iterate and residual
- * norm are bit-identical to the single-column calls on that column.  Single GPU handles only (AMG1D_ERR_UNSUPPORTED
- * otherwise).  The column set is separate device storage (three vectors per level and column, counted in
- * "device_bytes", allocated at the first call and grown when k grows): the single-column resident problem of
- * amg1d_dev_set_problem is neither read nor written by these calls, nor the column set by that one.  X0, B, X are
- * n_dof_host x k column-major (level 0's host vector length); X0 == NULL: zero initial guesses. */
+ * norm are bit-identical to the single-column calls on that column.  The column set is separate device storage
+ * (three vectors per level and column, counted in "device_bytes", allocated at the first call and grown when k grows):
+ * the single-column resident problem of amg1d_dev_set_problem is neither read nor written by these calls, nor the
+ * column set by that one.  X0, B, X are n_dof_host x k column-major (level 0's host vector length); X0 == NULL: zero
+ * initial guesses.
+ * Slab-sharded handles (amg1d_create_dist): X0, B and X are the rank's slabs (local_dofs x k, as the vectors of
+ * amg1d_dev_set_problem / amg1d_dev_get_solution there), and every rank makes every call with the same arguments (the
+ * calls are collective).  Each rank holds its slab of every column; the set's slab edges travel through NCCL, one
+ * group per exchange point for all columns, also where the resident problem uses peer memory.  Every column stays
+ * bit-identical to the single-column calls on the same handle. */
 #define AMG1D_MAX_COLS 8
 int amg1d_dev_set_problems(amg1d_t* h, int k, const double* X0, const double* B);   /* host -> device */
 /* column c gets exactly the b of amg1d_dev_fill_rhs_random(h, seed + c); x = 0 */
