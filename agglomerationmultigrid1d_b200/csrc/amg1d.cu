@@ -1799,17 +1799,37 @@ int read_multi_scalars(amg1d* h) {
     return AMG1D_OK;
 }
 
-// Structure class of a level (layout.cuh) from `nb` uploaded off-diagonal block sets.
-void detect_structure(const double* lo, const double* up, int64_t nb, int m, int* st, int* ilo, int* iup) {
+// ST_REPEAT is given to block-Jacobi 2 x 2 levels uploaded as patterns (amg1d_set_level_pattern) only.  m = 2:
+// the fused legs have that class for m = 2 only (kernels_fused.cuh), every other level keeps the class - and the
+// kernels - it had without it.  Patterns: an explicit level can also be formed on the device (install_from_blocks),
+// whose Galerkin products differ from the host's in the last bit of entries at rounding-noise level (1e-14 where a
+// ragged agglomeration leaves no exact zero), so a bitwise test could store the same level in two classes
+// depending on where it was set up; a pattern level has one set-up path and the test runs on its distinct block sets.
+bool repeat_eligible(int m, int diag) { return m == 2 && !diag; }
+
+bool same_bits(double a, double b) {
+    uint64_t x, y;
+    memcpy(&x, &a, 8);
+    memcpy(&y, &b, 8);
+    return x == y;
+}
+
+// Structure class of a level (layout.cuh) from `nb` uploaded off-diagonal block sets; repeat: ST_REPEAT may be
+// chosen (repeat_eligible).
+void detect_structure(const double* lo, const double* up, int64_t nb, int m, bool repeat, int* st, int* ilo,
+                      int* iup) {
     *st = AMG1D_ST_DENSE; *ilo = 0; *iup = 0;
     if (m < 2) return;
     const int mm = m * m;
     std::vector<char> lo_col(m, 0), lo_row(m, 0), up_col(m, 0), up_row(m, 0);
+    bool lo_rep = true, up_rep = true;     // every column of A_lo equals column 0, every row of A_up row 0
     for (int64_t e = 0; e < nb; ++e)
         for (int j = 0; j < m; ++j)
             for (int i = 0; i < m; ++i) {
                 if (lo[e * mm + j * m + i] != 0.0) { lo_col[j] = 1; lo_row[i] = 1; }
                 if (up[e * mm + j * m + i] != 0.0) { up_col[j] = 1; up_row[i] = 1; }
+                lo_rep = lo_rep && same_bits(lo[e * mm + j * m + i], lo[e * mm + i]);
+                up_rep = up_rep && same_bits(up[e * mm + j * m + i], up[e * mm + j * m]);
             }
     auto single = [m](const std::vector<char>& mask, int* idx) {
         int cnt = 0;
@@ -1820,6 +1840,7 @@ void detect_structure(const double* lo, const double* up, int64_t nb, int m, int
     int a, b;
     if (single(lo_col, &a) && single(up_row, &b)) { *st = AMG1D_ST_COLROW; *ilo = a; *iup = b; return; }
     if (single(lo_row, &a) && single(up_col, &b)) { *st = AMG1D_ST_ROWCOL; *ilo = a; *iup = b; return; }
+    if (lo_rep && up_rep && repeat) *st = AMG1D_ST_REPEAT;
 }
 
 // A level upload failed after alloc_level_common succeeded: give back what it took (operator tiles,
@@ -2188,7 +2209,7 @@ int amg1d_set_level(amg1d_t* h, int level, int64_t n_elem, int m, const double* 
         if (A_lo[q] != 0.0 || A_up[(size_t)(n_elem - 1) * mm + q] != 0.0)
             return fail(h, AMG1D_ERR_ARG, "A_lo[0] and A_up[n-1] must be zero blocks");
     int st = 0, ilo = 0, iup = 0;
-    if (h->opt_compress) detect_structure(A_lo, A_up, n_elem, m, &st, &ilo, &iup);
+    if (h->opt_compress) detect_structure(A_lo, A_up, n_elem, m, false, &st, &ilo, &iup);
     RET(alloc_level_common(h, level, n_elem, m, dinv_is_diagonal, perm, n_dof_host, st, ilo, iup));
     Level& lv = h->L[level];
     const int dsz = lv.diag ? m : mm;
@@ -2253,7 +2274,7 @@ int amg1d_set_level_pattern(amg1d_t* h, int level, int64_t n_elem, int m, int n_
     const int mm = m * m;
     const int nb = n_head + 1 + n_tail;
     int st = 0, ilo = 0, iup = 0;
-    if (h->opt_compress) detect_structure(A_lo, A_up, nb, m, &st, &ilo, &iup);
+    if (h->opt_compress) detect_structure(A_lo, A_up, nb, m, repeat_eligible(m, dinv_is_diagonal), &st, &ilo, &iup);
     RET(alloc_level_common(h, level, n_elem, m, dinv_is_diagonal, nullptr, n_elem * m, st, ilo, iup));
     Level& lv = h->L[level];
     const int dsz = lv.diag ? m : mm;
@@ -2325,7 +2346,7 @@ int amg1d_set_level_smoother(amg1d_t* h, int level, const double* S_lo, const do
     const int m = lv.m, mm = m * m;
     const int64_t n = lv.n;
     int st = 0, ilo = 0, iup = 0;
-    if (h->opt_compress) detect_structure(S_lo, S_up, n, m, &st, &ilo, &iup);
+    if (h->opt_compress) detect_structure(S_lo, S_up, n, m, false, &st, &ilo, &iup);
     lv.smd = amg1d_desc(m, 1, st, ilo, iup);            // the "Dinv" rows of this tile are unused (zeros)
     const int64_t bytes = (amg1d_tiles(n) + 1) * (int64_t)lv.smd.K * AMG1D_TILE * 8;
     RET(dev_alloc(h, (void**)&lv.smat_alloc, bytes));

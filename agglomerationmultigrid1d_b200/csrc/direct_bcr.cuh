@@ -48,6 +48,9 @@ __global__ void k_bcr_extract(const double* __restrict__ mat, MatDesc d, int64_t
     if (d.st == AMG1D_ST_DENSE) {
         vlo = T[q * AMG1D_TILE];
         vup = T[(d.o_up + q) * AMG1D_TILE];
+    } else if (d.st == AMG1D_ST_REPEAT) {
+        vlo = T[i * AMG1D_TILE];
+        vup = T[(d.o_up + j) * AMG1D_TILE];
     } else if (d.st == AMG1D_ST_COLROW) {
         vlo = (j == d.ilo) ? T[i * AMG1D_TILE] : 0.0;
         vup = (i == d.iup) ? T[(d.o_up + j) * AMG1D_TILE] : 0.0;

@@ -155,28 +155,33 @@ __device__ __forceinline__ void store_vec(double* __restrict__ p, const double (
 // register; any other row index stays with the generic tier (fast_tier_ok below).
 #define FUSED_COLROW_IUP 1
 
-// Tile rows of the level's operator part per structure class.
+// Tile rows of the level's operator part per structure class.  The classes that keep the dense FMA chains
+// (ST_DENSE, ST_REPEAT) read A_lo(i, j) / A_up(i, j) from the stored entry lo(i, j) / up(i, j).
 template <int M, int ST>
 struct OpShape {
     static constexpr int NO = ST ? M : M * M;           // stored entries of A_lo (and of A_up)
     static constexpr int O_DI = NO, O_UP = NO + M * M, O_DV = 2 * NO + M * M;
+    static constexpr bool DENSE_CHAINS = ST == AMG1D_ST_DENSE || ST == AMG1D_ST_REPEAT;
+    __host__ __device__ static constexpr int lo(int i, int j) { return ST == AMG1D_ST_REPEAT ? i : j * M + i; }
+    __host__ __device__ static constexpr int up(int i, int j) { return ST == AMG1D_ST_REPEAT ? j : j * M + i; }
 };
 
 // y = A_lo xl + A_di xc + A_up xr with the operator streamed from the tile (T points at
 // [tile][0][lane]).  Neighbour values: ST_COLROW needs only xl[ilo], passed as xl[0]; ST_ROWCOL needs
-// only xr[iup], passed as xr[0].  Same accumulation order as g_row_Ax.
+// only xr[iup], passed as xr[0]; ST_DENSE and ST_REPEAT need both blocks whole.  Same accumulation
+// order as g_row_Ax.
 template <int M, int ST>
 __device__ __forceinline__ void stream_Ax(const double* __restrict__ T, int ilo, int iup,
                                           const double (&xl)[M], const double (&xc)[M],
                                           const double (&xr)[M], double (&y)[M]) {
     using S = OpShape<M, ST>;
-    if constexpr (ST == AMG1D_ST_DENSE) {
+    if constexpr (S::DENSE_CHAINS) {
 #pragma unroll
         for (int i = 0; i < M; ++i) y[i] = 0.0;
 #pragma unroll
         for (int j = 0; j < M; ++j)
 #pragma unroll
-            for (int i = 0; i < M; ++i) y[i] = fma(T[(j * M + i) * AMG1D_TILE], xl[j], y[i]);
+            for (int i = 0; i < M; ++i) y[i] = fma(T[S::lo(i, j) * AMG1D_TILE], xl[j], y[i]);
     } else if constexpr (ST == AMG1D_ST_COLROW) {
 #pragma unroll
         for (int i = 0; i < M; ++i) y[i] = fma(T[i * AMG1D_TILE], xl[0], 0.0);
@@ -191,11 +196,11 @@ __device__ __forceinline__ void stream_Ax(const double* __restrict__ T, int ilo,
     for (int j = 0; j < M; ++j)
 #pragma unroll
         for (int i = 0; i < M; ++i) y[i] = fma(T[(S::O_DI + j * M + i) * AMG1D_TILE], xc[j], y[i]);
-    if constexpr (ST == AMG1D_ST_DENSE) {
+    if constexpr (S::DENSE_CHAINS) {
 #pragma unroll
         for (int j = 0; j < M; ++j)
 #pragma unroll
-            for (int i = 0; i < M; ++i) y[i] = fma(T[(S::O_UP + j * M + i) * AMG1D_TILE], xr[j], y[i]);
+            for (int i = 0; i < M; ++i) y[i] = fma(T[(S::O_UP + S::up(i, j)) * AMG1D_TILE], xr[j], y[i]);
     } else if constexpr (ST == AMG1D_ST_COLROW) {
         double yr = y[FUSED_COLROW_IUP];
 #pragma unroll
@@ -353,13 +358,14 @@ struct RegOpDv {
 template <int M, int ST, class OP>
 __device__ __forceinline__ void reg_Ax(const OP& A, int ilo, int iup, const double (&xl)[M],
                                        const double (&xc)[M], const double (&xr)[M], double (&y)[M]) {
-    if constexpr (ST == AMG1D_ST_DENSE) {
+    using S = OpShape<M, ST>;
+    if constexpr (S::DENSE_CHAINS) {
 #pragma unroll
         for (int i = 0; i < M; ++i) y[i] = 0.0;
 #pragma unroll
         for (int j = 0; j < M; ++j)
 #pragma unroll
-            for (int i = 0; i < M; ++i) y[i] = fma(A.lo[j * M + i], xl[j], y[i]);
+            for (int i = 0; i < M; ++i) y[i] = fma(A.lo[S::lo(i, j)], xl[j], y[i]);
     } else if constexpr (ST == AMG1D_ST_COLROW) {
 #pragma unroll
         for (int i = 0; i < M; ++i) y[i] = fma(A.lo[i], xl[0], 0.0);
@@ -374,11 +380,11 @@ __device__ __forceinline__ void reg_Ax(const OP& A, int ilo, int iup, const doub
     for (int j = 0; j < M; ++j)
 #pragma unroll
         for (int i = 0; i < M; ++i) y[i] = fma(A.di[j * M + i], xc[j], y[i]);
-    if constexpr (ST == AMG1D_ST_DENSE) {
+    if constexpr (S::DENSE_CHAINS) {
 #pragma unroll
         for (int j = 0; j < M; ++j)
 #pragma unroll
-            for (int i = 0; i < M; ++i) y[i] = fma(A.up[j * M + i], xr[j], y[i]);
+            for (int i = 0; i < M; ++i) y[i] = fma(A.up[S::up(i, j)], xr[j], y[i]);
     } else if constexpr (ST == AMG1D_ST_COLROW) {
         double yr = y[FUSED_COLROW_IUP];
 #pragma unroll
@@ -617,7 +623,7 @@ __device__ __forceinline__ void load_blocks(const double* __restrict__ mat, cons
 // 2x2 and 1x1 kernels are capped at 64 registers for 8 CTAs/SM.
 #ifndef FUSED_MINB_SMALL
 #define FUSED_MINB_SMALL 8   // m <= 2: <= 64 registers, no spills; measured best of 3 / 8 / 10 / 12 (T: -4 %)
-#endif
+#endif                       // ST_REPEAT 2x2 legs: 56 registers; 10 CTAs (48, spills) measured slower (DESIGN 6)
 constexpr int fused_min_blocks(int m, int st) {
     return m >= 5 ? (st != AMG1D_ST_DENSE ? 3 : 2)
          : m == 4 ? (st != AMG1D_ST_DENSE ? 5 : 3)
@@ -1431,7 +1437,7 @@ inline cudaError_t pipe_configure_all() {
     if (e == cudaSuccess) e = pipe_configure(f_down_pp<MM, MCC, FUSED_B, SS, 3, true>, sizeof(PipeDownSmem<MM, MCC, FUSED_B, SS>)); \
     if (e == cudaSuccess) e = pipe_configure(f_up_pp<MM, MCC, FUSED_B, SS, 0>, sizeof(PipeUpSmem<MM, MCC, FUSED_B, SS>)); \
     if (e == cudaSuccess) e = pipe_configure(f_up_pp<MM, MCC, FUSED_B, SS, 3>, sizeof(PipeUpSmem<MM, MCC, FUSED_B, SS>));
-    PP(4, 2, 1) PP(4, 3, 1) PP(2, 2, 0) PP(2, 2, 1)
+    PP(4, 2, 1) PP(4, 3, 1) PP(2, 2, 0) PP(2, 2, 1) PP(2, 2, 3)
 #undef PP
     return e;
 }
@@ -1561,7 +1567,8 @@ __device__ __forceinline__ void cp_async16(double* smem_dst, const double* gmem_
 }
 
 // Dense register copy of the element's operator whatever the level's structure class (entries that
-// the class does not store are exact zeros, so the dense chains give identical results).  T points at
+// the class does not store are exact zeros or, ST_REPEAT, copies of the stored column / row, so the
+// dense chains give identical results).  T points at
 // the element's lane of its (shared-memory) tile.
 template <int M>
 __device__ __forceinline__ void tail_load(const MatDesc& d, const double* T, bool active, RegOp<M, 0>& A) {
@@ -1571,6 +1578,14 @@ __device__ __forceinline__ void tail_load(const MatDesc& d, const double* T, boo
         if (d.st == AMG1D_ST_DENSE) {
 #pragma unroll
             for (int k = 0; k < M * M; ++k) { A.lo[k] = T[k * AMG1D_TILE]; A.up[k] = T[(d.o_up + k) * AMG1D_TILE]; }
+        } else if (d.st == AMG1D_ST_REPEAT) {
+#pragma unroll
+            for (int j = 0; j < M; ++j)
+#pragma unroll
+                for (int i = 0; i < M; ++i) {
+                    A.lo[j * M + i] = T[i * AMG1D_TILE];
+                    A.up[j * M + i] = T[(d.o_up + j) * AMG1D_TILE];
+                }
         } else {
 #pragma unroll
             for (int j = 0; j < M; ++j)
@@ -1737,7 +1752,8 @@ f_tail(const TailLevel* __restrict__ lv, int nl, const double* __restrict__ fac,
 // ---- host-side dispatch ---------------------------------------------------------------------------------
 #define FUSED_FOR_M(X) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9)
 
-// structure classes need m >= 2, and ST_COLROW the DG trace row (see FUSED_COLROW_IUP)
+// structure classes need m >= 2, and ST_COLROW the DG trace row (see FUSED_COLROW_IUP); ST_REPEAT is
+// instantiated for block-Jacobi 2 x 2 levels only, the only ones amg1d.cu gives that class
 inline bool fast_tier_ok(const MatDesc& d) {
     if (d.st == AMG1D_ST_DENSE) return true;
     if (d.m < 2) return false;
@@ -1754,7 +1770,7 @@ inline bool fused_sweep(const MatDesc& d, const double* mat, const double* b, co
         f_sweep<MM, DG != 0, SS><<<grid, 256, 0, st>>>(mat, d.ilo, d.iup, b, xin, xout, n, alpha, zero_guess); \
         return true;
 #define X(MM) Y(MM, 0, 0) Y(MM, 1, 0) Y(MM, 0, 1) Y(MM, 1, 1) Y(MM, 0, 2) Y(MM, 1, 2)
-        FUSED_FOR_M(X)
+        FUSED_FOR_M(X) Y(2, 0, 3)
 #undef X
 #undef Y
         default: return false;
@@ -1773,7 +1789,7 @@ inline bool fused_resnorm(const MatDesc& d, const double* mat, const double* b, 
         f_resnorm<MM, SS><<<(unsigned)grid, 256, 0, st>>>(mat, d.K, d.ilo, d.iup, b, x, n, partial);    \
         return true;
 #define X(MM) Y(MM, 0) Y(MM, 1) Y(MM, 2)
-        FUSED_FOR_M(X)
+        FUSED_FOR_M(X) Y(2, 3)
 #undef X
 #undef Y
         default: return false;
@@ -1791,7 +1807,7 @@ inline bool fused_matvec_dot(const MatDesc& d, const double* mat, const double* 
         f_matvec_dot<MM, SS><<<(unsigned)grid, 256, 0, st>>>(mat, d.K, d.ilo, d.iup, x, y, n, partial); \
         return true;
 #define X(MM) Y(MM, 0) Y(MM, 1) Y(MM, 2)
-        FUSED_FOR_M(X)
+        FUSED_FOR_M(X) Y(2, 3)
 #undef X
 #undef Y
         default: return false;
@@ -1799,13 +1815,14 @@ inline bool fused_matvec_dot(const MatDesc& d, const double* mat, const double* 
 }
 
 // (M, MC, ST, DIAG) combinations with a register-resident multi-sweep kernel:
-//   block Jacobi, dense and DG-assembled structure (DG / agglomerated levels);
+//   block Jacobi, dense, DG-assembled and repeated column / row structure (DG / agglomerated levels);
 //   point Jacobi on CG levels in group form (m = 1: CG p=1; m >= 2: ST_ROWCOL).
 #define FUSED_COMBOS(X)                                                                              \
     X(1, 1, 0, false) X(2, 1, 0, false) X(2, 2, 0, false) X(3, 1, 0, false) X(3, 2, 0, false)         \
     X(4, 2, 0, false) X(4, 3, 0, false) X(5, 3, 0, false)                                             \
     X(2, 1, 1, false) X(2, 2, 1, false) X(3, 1, 1, false) X(3, 2, 1, false)                           \
     X(4, 2, 1, false) X(4, 3, 1, false) X(5, 3, 1, false)                                             \
+    X(2, 1, 3, false) X(2, 2, 3, false)                                                               \
     X(1, 1, 0, true) X(1, 2, 0, true) X(2, 1, 2, true) X(3, 1, 2, true) X(4, 2, 2, true)
 
 inline int fused_key(int m, int mc, int st, int diag) { return ((m * 16 + mc) * 4 + st) * 2 + (diag ? 1 : 0); }
@@ -1863,7 +1880,7 @@ inline int fused_down(const MatDesc& d, int mc, const TransferMap& tm, int nswee
             fused_prev_persistent() = true;                                                               \
             return *err == cudaSuccess ? FUSED_OK : FUSED_ERR;                                            \
         }
-        PP(4, 2, 1) PP(4, 3, 1) PP(2, 2, 0) PP(2, 2, 1)
+        PP(4, 2, 1) PP(4, 3, 1) PP(2, 2, 0) PP(2, 2, 1) PP(2, 2, 3)
 #undef PP
     }
     if ((rec & 8) && (rec & 3) && !po.tab && fused_has_dv(d.m, mc, d.st, d.diag)) {   // inverse in registers
@@ -1873,7 +1890,7 @@ inline int fused_down(const MatDesc& d, int mc, const TransferMap& tm, int nswee
                                 xout, P0, P1, tm, rc, n, alpha, nsweep, zero ? 1 : 0, w, sl, rec, hl);     \
             return *err == cudaSuccess ? FUSED_OK : FUSED_ERR;                                            \
         }
-        DV(4, 2, 1) DV(4, 3, 1) DV(2, 2, 0) DV(2, 2, 1)
+        DV(4, 2, 1) DV(4, 3, 1) DV(2, 2, 0) DV(2, 2, 1) DV(2, 2, 3)
 #undef DV
     }
     switch (fused_key(d.m, mc, d.st, d.diag)) {
@@ -1918,7 +1935,7 @@ inline int fused_up(const MatDesc& d, int mc, const TransferMap& tm, int nsweep,
             fused_prev_persistent() = true;                                                               \
             return *err == cudaSuccess ? FUSED_OK : FUSED_ERR;                                            \
         }
-        PP(4, 2, 1) PP(4, 3, 1) PP(2, 2, 0) PP(2, 2, 1)
+        PP(4, 2, 1) PP(4, 3, 1) PP(2, 2, 0) PP(2, 2, 1) PP(2, 2, 3)
 #undef PP
     }
     if ((rec & 8) && (rec & 3) && !po.tab && fused_has_dv(d.m, mc, d.st, d.diag)) {
@@ -1928,7 +1945,7 @@ inline int fused_up(const MatDesc& d, int mc, const TransferMap& tm, int nsweep,
                                 xin, xout, P0, P1, tm, xcoarse, n, alpha, nsweep, w, partial, sl, rec, hl); \
             return *err == cudaSuccess ? FUSED_OK : FUSED_ERR;                                            \
         }
-        DV(4, 2, 1) DV(4, 3, 1) DV(2, 2, 0) DV(2, 2, 1)
+        DV(4, 2, 1) DV(4, 3, 1) DV(2, 2, 0) DV(2, 2, 1) DV(2, 2, 3)
 #undef DV
     }
     switch (fused_key(d.m, mc, d.st, d.diag)) {
@@ -1966,7 +1983,7 @@ inline bool fused_residual_restrict(const MatDesc& d, int mc, const TransferMap&
                                                                              tm, rc, n, out);           \
         return true;
 #define X(MM, MCC) Y(MM, MCC, 0) Y(MM, MCC, 1) Y(MM, MCC, 2)
-        FRR_PAIRS(X)
+        FRR_PAIRS(X) Y(2, 1, 3) Y(2, 2, 3)
 #undef X
 #undef Y
         default: return false;

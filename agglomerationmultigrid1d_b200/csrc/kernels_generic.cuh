@@ -41,13 +41,16 @@ struct TransferMap {
 
 // Row i of  A_lo x_l + A_di x_c + A_up x_r  for one element; T points at [tile][0][lane].  Terms are
 // accumulated in ascending column order, A_lo first, then A_di, then A_up (the order of a CSC SpMV over
-// the reference's DOF numbering); the compressed structure classes skip exact zeros only.
+// the reference's DOF numbering); the compressed structure classes skip exact zeros only (ST_REPEAT
+// skips nothing: it reads every A_lo(i, j) from c[i] and every A_up(i, j) from r[j]).
 __device__ __forceinline__ double g_row_Ax(const double* __restrict__ T, const MatDesc& d, int i,
                                            const double* xl, const double* xc, const double* xr) {
     const int m = d.m;
     double y = 0.0;
     if (d.st == AMG1D_ST_DENSE) {
         for (int j = 0; j < m; ++j) y = fma(T[(j * m + i) * AMG1D_TILE], xl[j], y);
+    } else if (d.st == AMG1D_ST_REPEAT) {
+        for (int j = 0; j < m; ++j) y = fma(T[i * AMG1D_TILE], xl[j], y);
     } else if (d.st == AMG1D_ST_COLROW) {
         y = fma(T[i * AMG1D_TILE], xl[d.ilo], y);
     } else if (i == d.ilo) {
@@ -58,6 +61,8 @@ __device__ __forceinline__ double g_row_Ax(const double* __restrict__ T, const M
     const double* U = T + (int64_t)d.o_up * AMG1D_TILE;
     if (d.st == AMG1D_ST_DENSE) {
         for (int j = 0; j < m; ++j) y = fma(U[(j * m + i) * AMG1D_TILE], xr[j], y);
+    } else if (d.st == AMG1D_ST_REPEAT) {
+        for (int j = 0; j < m; ++j) y = fma(U[j * AMG1D_TILE], xr[j], y);
     } else if (d.st == AMG1D_ST_ROWCOL) {
         y = fma(U[i * AMG1D_TILE], xr[d.iup], y);
     } else if (i == d.iup) {

@@ -180,7 +180,7 @@ inline int fused_down_multi(const MatDesc& d, int mc, const TransferMap& tm, int
                                 cols, k, P0, P1, tm, n, alpha, nsweep, zero ? 1 : 0, w, sl, rec);                    \
             return *err == cudaSuccess ? FUSED_OK : FUSED_ERR;                                                        \
         }
-        DV(4, 2, 1) DV(4, 3, 1) DV(2, 2, 0) DV(2, 2, 1)
+        DV(4, 2, 1) DV(4, 3, 1) DV(2, 2, 0) DV(2, 2, 1) DV(2, 2, 3)
 #undef DV
     }
     switch (fused_key(d.m, mc, d.st, d.diag)) {
@@ -213,7 +213,7 @@ inline int fused_up_multi(const MatDesc& d, int mc, const TransferMap& tm, int n
                                 d.iup, cols, k, P0, P1, tm, n, alpha, nsweep, w, sl, rec);                           \
             return *err == cudaSuccess ? FUSED_OK : FUSED_ERR;                                                        \
         }
-        DV(4, 2, 1) DV(4, 3, 1) DV(2, 2, 0) DV(2, 2, 1)
+        DV(4, 2, 1) DV(4, 3, 1) DV(2, 2, 0) DV(2, 2, 1) DV(2, 2, 3)
 #undef DV
     }
     switch (fused_key(d.m, mc, d.st, d.diag)) {
@@ -297,7 +297,7 @@ inline bool fused_matvec_dot_multi(const MatDesc& d, const double* mat, const Ma
         f_matvec_dot_multi<MM, SS><<<(unsigned)grid, 256, 0, st>>>(mat, d.K, d.ilo, d.iup, cols, k, n);             \
         return true;
 #define X(MM) Y(MM, 0) Y(MM, 1) Y(MM, 2)
-        FUSED_FOR_M(X)
+        FUSED_FOR_M(X) Y(2, 3)
 #undef X
 #undef Y
         default: return false;

@@ -336,14 +336,20 @@ void* amg1d_dev_ptr(amg1d_t* h, int level, int which);             /* raw device
  * which one is active; bit-identical results);
  * before the first level is
  * set: "compress" (1 = store only the structurally non-zero column / row of the off-diagonal blocks
- * where every element of the level has that structure, default 1), "shard_min" (elements per rank
+ * where every element of the level has that structure, or - block-Jacobi 2 x 2 levels given to
+ * amg1d_set_level_pattern - one column of A_lo and one row of A_up where all columns / rows are bitwise
+ * equal; default 1), "shard_min" (elements per rank
  * below which a level is gathered to rank 0, default 8192), "ghost_depth" (ghost elements per slab
  * edge, default 4 = max(nPre, nPost) + 1; CG levels with two-parent transfers need + ratio). */
 int amg1d_set_option(amg1d_t* h, const char* key, int64_t value);
 int64_t amg1d_get_info(amg1d_t* h, const char* key); /* "kernel_launches", "launches_per_cycle",
                                                         "device_bytes", "n_levels", "local_elements",
                                                         "local_dofs", "gather_level", "tail_start",
-                                                        "ghost_depth", "structure:<level>",
+                                                        "ghost_depth", "structure:<level>" (storage
+                                                        class of the level's off-diagonal blocks: 0 dense,
+                                                        1 one column of A_lo / one row of A_up non-zero,
+                                                        2 one row of A_lo / one column of A_up non-zero,
+                                                        3 all columns of A_lo / all rows of A_up equal),
                                                         "tile_rows:<level>", "dinv_recompute:<level>" (1 = the fused
                                                         legs of the level invert A_di in registers),
                                                         "leg_pipeline:<level>" (1 = they are the persistent
